@@ -7,7 +7,10 @@ residues per rank per step (k-NN graph + edge features once per frame, 100 x den
 de-normalise, VQ lookup, IC decoder, ic_to_xyz).  At N > 1 every rank samples its own protein (weak scaling,
 no collective on the data path; SURVEY.md section 8e).
 
-    python bench.py --gpus N --steps K --warmup W [--precision f16|fp32] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--precision f16|fp32] [--impl reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what rank 0's last timed step returned (sampler.Backmapper.sample: latent, idx, zq, ic_recon, xyz) as
+DIR/<name>.npy, so that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 
 prints ONE JSON line (rank 0):
   value         device-resident throughput (CUDA events, max over ranks, L2 flushed between timed steps)
@@ -34,6 +37,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (which may be read-only)
 
 import torch  # noqa: E402
 
@@ -56,6 +60,7 @@ C3_JOB = dict(proteins=256, lmin=300, lmax=700, compact=0.002, seed=7300)       
 # canonical algorithmic work per edge of the three per-edge kernels (SURVEY.md section 8d): GEMM flops only
 EDGE_FLOPS = {0: 2 * 2 * 128 * 128, 1: 2 * 3 * 128 * 128, 2: 2 * 2 * 128 * 128}
 FP32_NOMINAL_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12      # ALU-bound kernels have no measured peak: nominal FFMA rate, labelled as such
+DUMP_LIMIT = 64 << 20                                      # bytes written by --dump-outputs, all arrays together
 
 
 def _peaks():
@@ -110,6 +115,21 @@ class ClockSampler:
                     reasons.add(n)
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(out: dict, path: str):
+    """CUDA tensors -> path/<name>.npy: floating point as float32, integer indices as float64 (exact).  When the arrays
+    together would exceed DUMP_LIMIT, each keeps the same fixed, seeded sample of its rows (same shapes -> same rows)."""
+    import numpy as np
+    arrays = {k: v.detach().cpu().numpy().astype(np.float32 if v.is_floating_point() else np.float64)
+              for k, v in out.items() if v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT:
+            rows = np.random.default_rng(0).choice(a.shape[0], max(1, a.shape[0] * DUMP_LIMIT // total), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def _workload(rank: int, name: str = "c2", world: int = 1):
@@ -269,7 +289,7 @@ def run_metrics(args):
         metrics.bond_graph_stats(ref, xyz, z, num)
     torch.cuda.synchronize()
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(args.steps, 20)
+    reps = args.steps
     a.record()
     for _ in range(reps):
         counts, _ = metrics.bond_graph_stats(ref, xyz, z, num)
@@ -561,7 +581,12 @@ def main():
     ap.add_argument("--scale", default="all", choices=["all", "c3", "c4", "none"], help="scale_checks jobs run through the sharded driver")
     ap.add_argument("--scale-passes", type=int, default=2)
     ap.add_argument("--lean", action="store_true", help="only value / e2e / roofline (no roofline_all, scale_checks, drop-in, CPU legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of rank 0's last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("metrics", "c5")):
+        ap.error("--dump-outputs writes the outputs of the sampling path: --impl codlad_b200 with --workload c2, c3 or c4")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload in ("metrics", "c5"):
@@ -598,13 +623,17 @@ def main():
     l0 = plan.launches
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     for a, b in ev:
+        out = None                      # free the previous step's outputs before this step allocates, as if they were not kept
         flush.fill_(1)
         a.record()
-        bm.sample(plan, fs, generator=gen)
+        out = bm.sample(plan, fs, generator=gen)
         b.record()
     D.barrier()
     launches = plan.launches - l0
     ms_dev = D.max_over_ranks(sum(a.elapsed_time(b) for a, b in ev) / args.steps, dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)           # before the passes below overwrite the plan's buffers
+    del out
     residues = fs.NB * fs.L * world
     value = residues / (ms_dev * 1e-3)
 

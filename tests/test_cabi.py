@@ -36,7 +36,8 @@ def test_library_builds_loads_and_exports_all_symbols():
 def test_sass_contains_only_sm100a():
     import subprocess
     from codlad_b200 import build
-    out = subprocess.run(["cuobjdump", "-lelf", build.build()], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")      # the toolkit that built the library, whatever PATH says
+    out = subprocess.run([cuobjdump, "-lelf", build.build()], capture_output=True, text=True, check=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
