@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CB2_LIB") or os.path.join(_HERE, "libcodlad_b200.so")      # CB2_LIB: experiment builds
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 PRECISION = {"fp32": 0, "f32": 0, "f16": 1, "fp16": 1}
 
@@ -38,6 +38,7 @@ SIGNATURES = {
     "cb2_plan_forward": (_I, [_P, _P, _P, _P, _P]),
     "cb2_plan_forward_partial": (_I, [_P, _P, _P, _I, _P]),
     "cb2_plan_set_schedule": (_I, [_P, _P, _P, _I, _P]),
+    "cb2_plan_set_ddim_schedule": (_I, [_P, _P, _P, _I, _P]),
     "cb2_plan_sample": (_I, [_P, _P, _P, _I, _P]),
     "cb2_plan_set_topology": (_I, [_P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
     "cb2_plan_decode": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _P]),
@@ -47,6 +48,7 @@ SIGNATURES = {
     "cb2_knn_topk": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "cb2_vq_lookup": (_I, [_P, _P, _I, _I, _P, _P, _I, _P, _P, _P]),
     "cb2_p_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
+    "cb2_ddim_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
     "cb2_ic_to_xyz": (_I, [_P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
     "cb2_superposed_rmsd": (_I, [_P, _P, _P, _I, _P, _P]),
     "cb2_eval_bond_graphs": (_I, [_P, _P, _P, _P, _I, _I, _P, _I, C.c_float, _P, _P, _P]),

@@ -557,10 +557,9 @@ int cb2_plan_forward(cb2_plan* h, const float* x, const float* t, float* out, vo
     return 0;
 }
 
-int cb2_plan_set_schedule(cb2_plan* h, const float* t_of_step, const float* coef, int T, void* stream) {
+static int set_schedule(cb2_plan* h, const float* t_of_step, const float* coef, int T, int kind, cudaStream_t s) {
     if (!h || !t_of_step || !coef || T <= 0 || !h->p.model) { set_error("set_schedule: bad argument"); return 1; }
     Plan& p = h->p;
-    cudaStream_t s = (cudaStream_t)stream;
     if (T > p.mod_capacity) { set_error("set_schedule: T=%d exceeds capacity %d", T, p.mod_capacity); return 1; }
     CB2_CUDA(cudaMemcpyAsync(p.tvals, t_of_step, T * sizeof(float), cudaMemcpyHostToDevice, s));
     CB2_CUDA(cudaMemcpyAsync(p.coef, coef, (size_t)T * 8 * sizeof(float), cudaMemcpyHostToDevice, s));
@@ -568,8 +567,19 @@ int cb2_plan_set_schedule(cb2_plan* h, const float* t_of_step, const float* coef
     CB2_CUDA(cudaStreamSynchronize(s));     // host staging buffers may be freed by the caller on return
     p.launches += 2;
     p.coef_steps = T;
+    p.update_kind = kind;
+    p.coef_noisy = kind == UPDATE_DDPM;
+    for (int i = 0; i < T && !p.coef_noisy; ++i) p.coef_noisy = coef[(size_t)i * 8 + 4] != 0.0f;      // some DDIM sigma != 0
     if (p.graph) { cudaGraphExecDestroy(p.graph); p.graph = nullptr; }
     return 0;
+}
+
+int cb2_plan_set_schedule(cb2_plan* h, const float* t_of_step, const float* coef, int T, void* stream) {
+    return set_schedule(h, t_of_step, coef, T, UPDATE_DDPM, (cudaStream_t)stream);
+}
+
+int cb2_plan_set_ddim_schedule(cb2_plan* h, const float* t_of_step, const float* ddim_coef, int T, void* stream) {
+    return set_schedule(h, t_of_step, ddim_coef, T, UPDATE_DDIM, (cudaStream_t)stream);
 }
 
 static int enqueue_loop(cb2_plan* h, float* x, const float* noise, cudaStream_t s) {
@@ -579,7 +589,8 @@ static int enqueue_loop(cb2_plan* h, float* x, const float* noise, cudaStream_t 
     float *cur = h->xa, *nxt = h->xb;
     for (int step = p.coef_steps - 1; step >= 0; --step) {
         const float* mod_row = p.mod + (size_t)step * CB2_MOD_TOTAL;     // every member shares the step -> stride 0
-        if (int e = run_forward(p, cur, mod_row, 0, noise + (size_t)step * n3, nxt, p.coef + (size_t)step * 8, s)) {
+        const float* step_noise = noise != nullptr ? noise + (size_t)step * n3 : nullptr;
+        if (int e = run_forward(p, cur, mod_row, 0, step_noise, nxt, p.coef + (size_t)step * 8, s)) {
             char prev[1024];
             snprintf(prev, sizeof(prev), "%s", g_err);
             const unsigned int* tl = edge_tc_trap_log();
@@ -599,9 +610,10 @@ static int enqueue_loop(cb2_plan* h, float* x, const float* noise, cudaStream_t 
 }
 
 int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, void* stream) {
-    if (!h || !x || !noise) { set_error("sample: null argument"); return 1; }
+    if (!h || !x) { set_error("sample: null argument"); return 1; }
     Plan& p = h->p;
     if (!h->frames_ready || p.coef_steps <= 0) { set_error("sample: set_frames / set_schedule must be called first"); return 1; }
+    if (!noise && p.coef_noisy) { set_error("sample: noise may be NULL only on a DDIM schedule whose sigma are all zero (eta = 0)"); return 1; }
     cudaStream_t s = (cudaStream_t)stream;
     if (!use_graph) return enqueue_loop(h, x, noise, s);
     // (kernel variants are chosen at capture time from the geometry: a frame set with / without padded residues needs its own graph)
@@ -775,6 +787,12 @@ int cb2_p_sample(const float* x, const float* model_out, const float* noise, con
                  int rows_per_member, int rows, int C, float* x_next, void* stream) {
     if (!x || !model_out || !noise || !coef || !step_of_member || !x_next) { set_error("p_sample: null argument"); return 1; }
     return launch_p_sample(x, model_out, noise, coef, step_of_member, rows_per_member, rows, C, x_next, (cudaStream_t)stream);
+}
+
+int cb2_ddim_sample(const float* x, const float* model_out, const float* noise, const float* coef, const int* step_of_member,
+                    int rows_per_member, int rows, int C, float* x_next, void* stream) {
+    if (!x || !model_out || !coef || !step_of_member || !x_next) { set_error("ddim_sample: null argument"); return 1; }
+    return launch_ddim_sample(x, model_out, noise, coef, step_of_member, rows_per_member, rows, C, x_next, (cudaStream_t)stream);
 }
 
 int cb2_ic_to_xyz(const float* ca_full, const float* ic_recon, int NB, int L, const int* frame_of, const int* lengths,

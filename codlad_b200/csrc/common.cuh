@@ -48,6 +48,17 @@ __device__ __forceinline__ float warp_max(float v) {
     return v;
 }
 
+// One DDIM step of one latent coordinate (IDDPM gaussian_diffusion.py ddim_sample, clip_denoised=False) from the step's row
+// c = {sqrt(1/a), sqrt(1/a - 1), sqrt(a_prev), sqrt(max(0, 1 - a_prev - sigma^2)), sigma * [step != 0], 0, 0, 0}.  eps is
+// re-derived from x0 as IDDPM's _predict_eps_from_xstart does.  `noise` is read only when it is given and sigma != 0.
+__device__ __forceinline__ float ddim_update(float x, float eps, const float* c, const float* noise) {
+    const float x0 = c[0] * x - c[1] * eps;
+    const float eps2 = (c[0] * x - x0) / c[1];
+    float out = c[2] * x0 + c[3] * eps2;
+    if (noise != nullptr && c[4] != 0.0f) out += c[4] * *noise;
+    return out;
+}
+
 // LayerNorm statistics of one 128-wide row held as 4 values per lane of one warp.
 // Matches torch.layer_norm: biased variance, rstd = 1/sqrt(var + eps).
 __device__ __forceinline__ void warp_ln_stats(const float v[4], float eps, float& mean, float& rstd) {

@@ -50,6 +50,7 @@ struct DenoiserModel {
 };
 
 enum Precision { PREC_F32 = 0, PREC_F16 = 1 };
+enum UpdateKind { UPDATE_DDPM = 0, UPDATE_DDIM = 1 };
 
 // One plan = one geometry: F frames of padded length L, NB members (member b uses frame
 // frame_of[b]), K neighbours.  Owns every intermediate buffer of the denoiser.
@@ -84,8 +85,10 @@ struct Plan {
     int* mod_row = nullptr;         // [NB] row of `mod` used by each member (forward() path)
     float* tvals = nullptr;         // [mod_capacity] timestep values staging
     // sampling-loop state
-    float* coef = nullptr;          // [T, 8] per-step p_sample scalars (fp32)
+    float* coef = nullptr;          // [T, 8] per-step update scalars (fp32): p_sample or DDIM rows, as update_kind says
     int coef_steps = 0;
+    int update_kind = 0;            // UPDATE_DDPM | UPDATE_DDIM, uniform over the schedule (the fused update selects on it)
+    bool coef_noisy = true;         // the update reads its noise (DDPM always; DDIM when some sigma != 0)
     cudaGraphExec_t graph = nullptr;
     const void* graph_key[4] = {nullptr, nullptr, nullptr, nullptr};
     int graph_steps = 0;
@@ -104,6 +107,8 @@ int launch_edge_raw_features(const float* X, const int* idx, const float* D, int
 int launch_timestep_mod(const DenoiserModel& m, const float* tvals, int n, float* scratch_silu_c, float* mod, __half* mod16, cudaStream_t s);
 int launch_p_sample(const float* x, const float* out6, const float* noise, const float* coef_rows, const int* step_of_row,
                     int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
+int launch_ddim_sample(const float* x, const float* out6, const float* noise, const float* coef_rows, const int* step_of_row,
+                       int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
 float* plan_P(Plan& p, int which);
 
 struct NodeArgs;   // node.cu

@@ -11,7 +11,8 @@
 //    mask; then the per-node halves of the NEXT edge MLP's first layer
 //    (W1 [h_V_i | h_E | h_V_j] = W1a h_V_i + W1b h_E + W1c h_V_j: the a/c products are per node),
 //    and for the last decoder layer FinalLayer (latent_model.py:21-35) fused with the DDPM
-//    p_sample update (diffusion_and_flow/gaussian_diffusion.py:303-318,345-351,440-446).
+//    p_sample update (diffusion_and_flow/gaussian_diffusion.py:303-318,345-351,440-446) or, on a
+//    DDIM schedule, IDDPM's ddim_sample update (ddim_update, common.cuh).
 //
 // fp32 SIMT: 16 rows per CTA, 128 threads, thread = output column (see tile_gemm.cuh).
 #include "model.h"
@@ -91,8 +92,9 @@ struct NodeParams {
     int do_final;
     const float *fin_mod, *fin_w_t, *fin_b;   // fin_mod row b at fin_mod + b*mod_stride
     float* out6;             // [N,6]
-    const float *x_t, *noise, *coef;          // p_sample inputs (nullable -> forward() only)
+    const float *x_t, *noise, *coef;          // p_sample inputs (nullable -> forward() only); DDIM: noise may be null
     float* x_next;
+    int ddim;                // the fused update is DDIM (coef = a DDIM row) instead of p_sample
 };
 
 constexpr int NR = 16;
@@ -288,7 +290,10 @@ __global__ void __launch_bounds__(128) node_update_kernel(NodeParams p) {
 #pragma unroll
             for (int u = 0; u < 6; ++u) o[u] = warp_sum(o[u]) + p.fin_b[u];
             if (lane < 6) p.out6[(size_t)n * 6 + lane] = o[lane];
-            if (p.x_next != nullptr && lane < 3) {
+            if (p.x_next != nullptr && lane < 3 && p.ddim) {
+                const float* nz = p.noise != nullptr ? p.noise + (size_t)n * 3 + lane : nullptr;
+                p.x_next[(size_t)n * 3 + lane] = ddim_update(p.x_t[(size_t)n * 3 + lane], o[lane], p.coef, nz);
+            } else if (p.x_next != nullptr && lane < 3) {
                 // learned-range variance + epsilon parameterisation (gaussian_diffusion.py:303-318,345-351,440-446)
                 const float eps = o[lane], vv = o[3 + lane];
                 const float min_log = p.coef[0], max_log = p.coef[1];
@@ -320,6 +325,17 @@ __global__ void p_sample_kernel(const float* __restrict__ x, const float* __rest
     x_next[t] = mean_ + cf[6] * expf(0.5f * logvar) * noise[t];
 }
 
+__global__ void ddim_sample_kernel(const float* __restrict__ x, const float* __restrict__ out6, const float* __restrict__ noise,
+                                   const float* __restrict__ coef_rows, const int* __restrict__ step_of_row, int rows_per_b,
+                                   int n_rows, int C, float* __restrict__ x_next) {
+    // Stand-alone DDIM update for callers that run their own denoiser (generic ddim_sample path); noise may be null.
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_rows * C) return;
+    const int row = t / C, d = t - row * C;
+    const float* cf = coef_rows + (size_t)step_of_row[row / rows_per_b] * 8;
+    x_next[t] = ddim_update(x[t], out6[(size_t)row * 2 * C + d], cf, noise != nullptr ? noise + t : nullptr);
+}
+
 }  // namespace
 
 int launch_timestep_mod(const DenoiserModel& m, const float* tvals, int n, float* scratch_silu_c, float* mod, __half* mod16, cudaStream_t s) {
@@ -338,6 +354,14 @@ int launch_p_sample(const float* x, const float* out6, const float* noise, const
                     int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s) {
     const int total = n_rows * C;
     p_sample_kernel<<<(total + 255) / 256, 256, 0, s>>>(x, out6, noise, coef_rows, step_of_row, rows_per_b, n_rows, C, x_next);
+    CB2_LAUNCH_CHECK();
+    return 0;
+}
+
+int launch_ddim_sample(const float* x, const float* out6, const float* noise, const float* coef_rows, const int* step_of_row,
+                       int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s) {
+    const int total = n_rows * C;
+    ddim_sample_kernel<<<(total + 255) / 256, 256, 0, s>>>(x, out6, noise, coef_rows, step_of_row, rows_per_b, n_rows, C, x_next);
     CB2_LAUNCH_CHECK();
     return 0;
 }
@@ -415,6 +439,7 @@ int launch_node_update(Plan& p, int phase, const float* mod_base, int mod_stride
             np.fin_w_t = m.fin_w_t; np.fin_b = m.fin_b;
             np.out6 = p.out6;
             np.x_t = x_t; np.noise = noise; np.x_next = x_next; np.coef = coef_row;
+            np.ddim = p.update_kind == UPDATE_DDIM;
         }
     }
     return node_launch(p, np, s);

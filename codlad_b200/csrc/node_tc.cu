@@ -134,6 +134,7 @@ void node_tc_update_params(Plan& p, int phase, const float* mod_base, int mod_st
             np.fin_w_t = m.fin_w_t; np.fin_b = m.fin_b;
             np.out6 = p.out6;
             np.x_t = x_t; np.noise = noise; np.x_next = x_next; np.coef = coef_row;
+            np.ddim = p.update_kind == UPDATE_DDIM;
         }
     }
 }

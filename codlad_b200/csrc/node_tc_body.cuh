@@ -34,6 +34,7 @@ struct NodeTcParams {
     float* out6;
     const float *x_t, *noise, *coef;
     float* x_next;
+    int ddim;                    // the fused update is DDIM (coef = a DDIM row; noise may be null) instead of p_sample
     unsigned long long* trace;   // debug timeline of CTA 0 (nullptr = off)
     int trace_slot;              // debug: launch window slot (trace_window)
 };
@@ -418,7 +419,7 @@ __device__ __forceinline__ void node_block(unsigned char* smem, const uint32_t t
             }
         }
         if (p.do_final) {
-            // ---- FinalLayer (adaLN modulate + Linear 128 -> 6) fused with the DDPM p_sample update.  The fp32 rows are parked in
+            // ---- FinalLayer (adaLN modulate + Linear 128 -> 6) fused with the DDPM p_sample (or DDIM) update.  The fp32 rows are parked in
             //      shared memory (the FFN hidden tiles are dead); each warp then owns two nodes, lanes across features ----
             float* sH = reinterpret_cast<float*>(act_tile(2));
 #pragma unroll
@@ -458,7 +459,11 @@ __device__ __forceinline__ void node_block(unsigned char* smem, const uint32_t t
                     for (int u = 1; u < 6; ++u) mine = lane == u ? o[u] : mine;
                     p.out6[(size_t)n * 6 + lane] = mine;
                 }
-                if (p.x_next != nullptr && lane < 3) {
+                if (p.x_next != nullptr && lane < 3 && p.ddim) {
+                    const float eps = lane == 0 ? o[0] : (lane == 1 ? o[1] : o[2]);
+                    const float* nz = p.noise != nullptr ? p.noise + (size_t)n * 3 + lane : nullptr;
+                    p.x_next[(size_t)n * 3 + lane] = ddim_update(p.x_t[(size_t)n * 3 + lane], eps, p.coef, nz);
+                } else if (p.x_next != nullptr && lane < 3) {
                     const float eps = lane == 0 ? o[0] : (lane == 1 ? o[1] : o[2]);
                     const float vv = lane == 0 ? o[3] : (lane == 1 ? o[4] : o[5]);
                     const float x = p.x_t[(size_t)n * 3 + lane];

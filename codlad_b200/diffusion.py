@@ -6,6 +6,8 @@ computed once).  The step loop itself is CUDA:
   * when the model is a `codlad_b200.latent_model` denoiser, `p_sample_loop` hands the whole loop
     (T denoiser forwards + T fused p_sample updates) to `cb2_plan_sample` as one CUDA graph;
   * any other callable goes through a generic loop whose update is the `cb2_p_sample` kernel.
+`ddim_sample_loop` (IDDPM's DDIM sampler, which the reference does not ship) takes the same two routes with the DDIM
+update (`cb2_plan_set_ddim_schedule` / `cb2_ddim_sample`).
 `training_losses` (config 5, "next" row f-1 of SURVEY.md section 8) is not implemented yet.
 """
 from __future__ import annotations
@@ -108,10 +110,27 @@ class SpacedDiffusion:
         c[:, 6] = (np.arange(T) != 0).astype(np.float32)
         return c
 
-    def _coef_on(self, device):
-        key = str(device)
+    def ddim_coef_table(self, eta: float = 0.0) -> np.ndarray:
+        """[T, 8] fp32 rows consumed by cb2_plan_set_ddim_schedule / cb2_ddim_sample, computed in float64 and rounded once:
+        {sqrt(1/acp), sqrt(1/acp - 1), sqrt(acp_prev), sqrt(max(0, 1 - acp_prev - sigma^2)), sigma * (step != 0), 0, 0, 0} with
+        sigma = eta sqrt((1 - acp_prev) / (1 - acp)) sqrt(1 - acp / acp_prev) (IDDPM gaussian_diffusion.py ddim_sample).  The max
+        keeps rounding near eta = 1 from turning a tiny argument into a NaN."""
+        ac, ac_prev = self.alphas_cumprod, self.alphas_cumprod_prev
+        sigma = eta * np.sqrt((1.0 - ac_prev) / (1.0 - ac)) * np.sqrt(1.0 - ac / ac_prev)
+        c = np.zeros((self.num_timesteps, 8), dtype=np.float32)
+        c[:, 0] = self.sqrt_recip_alphas_cumprod
+        c[:, 1] = self.sqrt_recipm1_alphas_cumprod
+        c[:, 2] = np.sqrt(ac_prev)
+        c[:, 3] = np.sqrt(np.maximum(0.0, 1.0 - ac_prev - sigma ** 2))
+        c[:, 4] = sigma * (np.arange(self.num_timesteps) != 0)
+        return c
+
+    def _coef_on(self, device, eta=None):
+        """coef_table (eta None) or ddim_coef_table(eta) on `device`, uploaded once."""
+        key = str(device) if eta is None else ("ddim", float(eta), str(device))
         if key not in self._coef_dev:
-            self._coef_dev[key] = torch.from_numpy(self.coef_table()).to(device)
+            table = self.coef_table() if eta is None else self.ddim_coef_table(eta)
+            self._coef_dev[key] = torch.from_numpy(table).to(device)
         return self._coef_dev[key]
 
     # -- sampling ----------------------------------------------------------------------------------
@@ -161,6 +180,65 @@ class SpacedDiffusion:
         eps = out[..., :C_]
         c = self._coef_on(x.device)[t].view(-1, *([1] * (x.dim() - 1)), 8)
         return {"sample": nxt, "pred_xstart": c[..., 2] * x - c[..., 3] * eps}
+
+    # -- DDIM (IDDPM / DiT gaussian_diffusion.py ddim_sample*; the reference has no DDIM sampler) ---------------------
+    @staticmethod
+    def _check_ddim_args(clip_denoised, denoised_fn, cond_fn):
+        if cond_fn is not None or denoised_fn is not None or clip_denoised:
+            raise NotImplementedError("DDIM sampling supports clip_denoised=False without cond_fn / denoised_fn")
+
+    def ddim_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, cond_fn=None, model_kwargs=None,
+                         device=None, progress=False, eta=0.0, step_noise=None):
+        """IDDPM ddim_sample_loop.  With eta = 0 the loop is deterministic and draws no per-step noise; otherwise
+        `step_noise` [T, *shape] (extension, as in p_sample_loop) injects the N(0,1) draws, default one torch.randn call.
+        A codlad_b200 denoiser runs the whole loop as one CUDA graph with the update fused into its last kernel."""
+        self._check_ddim_args(clip_denoised, denoised_fn, cond_fn)
+        from .latent_model import fused_sampler_for
+        fused = fused_sampler_for(model)
+        if fused is not None:
+            return fused.sample_loop(self, shape, noise, model_kwargs or {}, device, step_noise, update="ddim", eta=eta)
+        final = None
+        for final in self.ddim_sample_loop_progressive(model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
+                                                       device, progress, eta, step_noise):
+            pass
+        return final["sample"]
+
+    def ddim_sample_loop_progressive(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, cond_fn=None,
+                                     model_kwargs=None, device=None, progress=False, eta=0.0, step_noise=None):
+        """IDDPM ddim_sample_loop_progressive (generic callable model; update on the GPU via cb2_ddim_sample)."""
+        self._check_ddim_args(clip_denoised, denoised_fn, cond_fn)
+        N.require_cuda()
+        device = torch.device(device if device is not None else "cuda")
+        img = noise if noise is not None else torch.randn(*shape, device=device)
+        img = img.to(device, torch.float32).contiguous()
+        for i in list(range(self.num_timesteps))[::-1]:
+            t = torch.tensor([i] * shape[0], device=device)
+            n = None
+            if eta != 0:
+                n = step_noise[i].to(device, torch.float32).contiguous() if step_noise is not None else torch.randn_like(img)
+            out = self.ddim_sample(model, img, t, clip_denoised=False, model_kwargs=model_kwargs, eta=eta, _noise=n)
+            yield out
+            img = out["sample"]
+
+    def ddim_sample(self, model, x, t, clip_denoised=True, denoised_fn=None, cond_fn=None, model_kwargs=None, eta=0.0, _noise=None):
+        """IDDPM ddim_sample: one DDIM step; model(x, timestep_map[t], **kwargs) -> [B,...,2C] (the variance half is unused).
+        Returns dict(sample, pred_xstart).  With eta = 0 no noise is drawn or read."""
+        self._check_ddim_args(clip_denoised, denoised_fn, cond_fn)
+        model_kwargs = model_kwargs or {}
+        map_t = torch.tensor(self.timestep_map, device=t.device, dtype=t.dtype)[t]     # respace.py:124-125
+        out = model(x, map_t, **model_kwargs).to(torch.float32).contiguous()
+        C_ = x.shape[-1]
+        rows = x.numel() // C_
+        noise = None
+        if eta != 0:
+            noise = (_noise if _noise is not None else torch.randn_like(x)).contiguous()
+        coef = self._coef_on(x.device, eta)
+        nxt = torch.empty_like(x)
+        N.check(N.lib().cb2_ddim_sample(N.dptr(x.contiguous(), torch.float32), N.dptr(out), N.dptr(noise, torch.float32), N.dptr(coef),
+                                        N.dptr(t.to(torch.int32).contiguous()), rows // x.shape[0], rows, C_, N.dptr(nxt), N.stream_ptr()),
+                "ddim_sample")
+        c = coef[t].view(-1, *([1] * (x.dim() - 1)), 8)
+        return {"sample": nxt, "pred_xstart": c[..., 0] * x - c[..., 1] * out[..., :C_]}
 
     def p_mean_variance(self, model, x, t, clip_denoised=True, denoised_fn=None, model_kwargs=None, x_self_cond=None):
         """gaussian_diffusion.py:262-360 for the shipped configuration (epsilon prediction, learned-range variance):

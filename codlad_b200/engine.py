@@ -146,9 +146,19 @@ class Plan:
         N.check(N.lib().cb2_plan_set_schedule(self.handle, t.data_ptr(), c.data_ptr(), int(t.numel()), N.stream_ptr()), "set_schedule")
         self.T = int(t.numel())
 
-    def sample(self, x, noise, use_graph: bool = True):
-        """In-place reverse diffusion of x [NB,L,3] with noise [T,NB,L,3] (both CUDA fp32 contiguous)."""
-        assert x.shape == (self.NB, self.L, 3) and noise.shape == (self.T, self.NB, self.L, 3)
+    def set_ddim_schedule(self, timestep_map, coef):
+        """DDIM schedule: coef = SpacedDiffusion.ddim_coef_table(eta); sample() then applies DDIM updates."""
+        t = torch.as_tensor(np.asarray(timestep_map), dtype=torch.float32).contiguous()
+        c = torch.as_tensor(np.asarray(coef), dtype=torch.float32).contiguous()
+        assert c.shape == (t.numel(), 8)
+        N.check(N.lib().cb2_plan_set_ddim_schedule(self.handle, t.data_ptr(), c.data_ptr(), int(t.numel()), N.stream_ptr()),
+                "set_ddim_schedule")
+        self.T = int(t.numel())
+
+    def sample(self, x, noise=None, use_graph: bool = True):
+        """In-place reverse diffusion of x [NB,L,3] with noise [T,NB,L,3] (both CUDA fp32 contiguous).  noise may be None
+        on a DDIM schedule with eta = 0 (the C side refuses it otherwise)."""
+        assert x.shape == (self.NB, self.L, 3) and (noise is None or noise.shape == (self.T, self.NB, self.L, 3))
         N.check(N.lib().cb2_plan_sample(self.handle, N.dptr(x, torch.float32), N.dptr(noise, torch.float32), int(use_graph), N.stream_ptr()),
                 "sample")
         return x

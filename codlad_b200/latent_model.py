@@ -153,29 +153,38 @@ class _FusedSampler:
     def __init__(self, model: ProteinMPNN_diffusion_new):
         self.model = model
 
-    def sample_loop(self, diffusion, shape, noise, model_kwargs, device, step_noise):
+    def sample_loop(self, diffusion, shape, noise, model_kwargs, device, step_noise, update="ddpm", eta=0.0):
+        """update "ddpm" (p_sample_loop) or "ddim" with `eta` (ddim_sample_loop; eta = 0 draws no step noise)."""
         batch = model_kwargs.get("batch")
         model = self.model
         plan = model.plan_for(batch, shape[0])
         ent = model._entry_of(plan)
         T = diffusion.num_timesteps
-        sched_key = (T, tuple(int(v) for v in diffusion.timestep_map))
+        ddim = update == "ddim"
+        sched_key = (update, float(eta) if ddim else None, T, tuple(int(v) for v in diffusion.timestep_map))
         if ent["schedule"] != sched_key:                 # (re-)tabulate the adaLN rows only when the schedule changes: it drops the graph
-            plan.set_schedule(diffusion.timestep_map, diffusion.coef_table())
+            if ddim:
+                plan.set_ddim_schedule(diffusion.timestep_map, diffusion.ddim_coef_table(eta))
+            else:
+                plan.set_schedule(diffusion.timestep_map, diffusion.coef_table())
             ent["schedule"] = sched_key
+        noisy = not ddim or eta != 0
         dev = plan.device
         bufs = ent["bufs"]
-        if bufs is None or bufs[1].shape[0] != T:         # persistent x / noise buffers: the CUDA graph of the loop is keyed on them
-            bufs = ent["bufs"] = (torch.empty(*shape, device=dev, dtype=torch.float32), torch.empty(T, *shape, device=dev, dtype=torch.float32))
-        x, eps = bufs
+        if bufs is None or (noisy and (bufs[1] is None or bufs[1].shape[0] != T)):
+            # persistent x / noise buffers: the CUDA graph of the loop is keyed on them
+            x = bufs[0] if bufs is not None else torch.empty(*shape, device=dev, dtype=torch.float32)
+            bufs = ent["bufs"] = (x, torch.empty(T, *shape, device=dev, dtype=torch.float32) if noisy else None)
+        x, eps = bufs[0], bufs[1] if noisy else None
         if noise is not None:
             x.copy_(noise, non_blocking=True)
         else:
             torch.randn(*shape, device=dev, out=x)
-        if step_noise is not None:
-            eps.copy_(step_noise, non_blocking=True)
-        else:
-            torch.randn(T, *shape, device=dev, out=eps)
+        if eps is not None:
+            if step_noise is not None:
+                eps.copy_(step_noise, non_blocking=True)
+            else:
+                torch.randn(T, *shape, device=dev, out=eps)
         plan.sample(x, eps, use_graph=True)
         return x.clone()                                 # the caller owns its result; the buffer is reused by the next call
 

@@ -112,10 +112,18 @@ def frames_from_batch(batch: dict, infos, num_ensemble: int = 1, frame_of=None) 
 
 
 class Backmapper:
-    """CG trace -> all-atom ensemble: 100-step latent diffusion + VQ-VAE decode + IC reconstruction."""
+    """CG trace -> all-atom ensemble: 100-step latent diffusion + VQ-VAE decode + IC reconstruction.
+    sampler="ddpm" is the reference's ancestral sampler; sampler="ddim" uses IDDPM's DDIM update with `eta` on the same
+    respacing (eta = 0: deterministic, no per-step noise is drawn or stored)."""
 
     def __init__(self, denoiser_state: dict, vae_state: dict, vae_type: str = "N6", k_neighbors: int = 64,
-                 num_sampling_steps: int = 100, precision: str = "f16", latent_stats=None, max_plans: int = 4):
+                 num_sampling_steps: int = 100, precision: str = "f16", latent_stats=None, max_plans: int = 4,
+                 sampler: str = "ddpm", eta: float = 0.0):
+        if sampler not in ("ddpm", "ddim"):
+            raise ValueError(f"sampler must be 'ddpm' or 'ddim', got {sampler!r}")
+        if sampler == "ddpm" and eta != 0:
+            raise ValueError("eta applies to sampler='ddim' only")
+        self.sampler, self.eta = sampler, float(eta)
         self.precision = precision
         self.k_neighbors = int(k_neighbors)
         self.max_plans = int(max_plans)
@@ -137,7 +145,10 @@ class Backmapper:
                 self._bufs.pop(id(old), None)
                 old.close()
             plan = Plan(self.denoiser, fs.F, fs.NB, fs.L, self.precision, keep_debug)
-            plan.set_schedule(self.diffusion.timestep_map, self.diffusion.coef_table())
+            if self.sampler == "ddim":
+                plan.set_ddim_schedule(self.diffusion.timestep_map, self.diffusion.ddim_coef_table(self.eta))
+            else:
+                plan.set_schedule(self.diffusion.timestep_map, self.diffusion.coef_table())
         else:
             self._plans.pop(key)                                   # re-insert: most recently used last
         self._plans[key] = plan
@@ -153,22 +164,25 @@ class Backmapper:
     def sample(self, plan: Plan, fs: FrameSet, z: torch.Tensor = None, step_noise: torch.Tensor = None,
                use_graph: bool = True, generator: torch.Generator = None):
         """Device-resident path: returns dict(latent, idx, ic_recon, xyz) of CUDA tensors.
-        z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted."""
+        z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted.  DDIM with eta = 0 uses no
+        step noise: `step_noise` is ignored."""
         dev = plan.device
         shape = (fs.NB, fs.L, 3)
+        noisy = self.sampler == "ddpm" or self.eta != 0
         bufs = self._bufs.get(id(plan))
         if bufs is None:      # persistent buffers: the CUDA graph of the step loop is keyed on these pointers
-            bufs = (torch.empty(*shape, device=dev), torch.empty(self.T, *shape, device=dev))
+            bufs = (torch.empty(*shape, device=dev), torch.empty(self.T, *shape, device=dev) if noisy else None)
             self._bufs[id(plan)] = bufs
         x, noise = bufs
         if z is not None:
             x.copy_(z, non_blocking=True)
         else:
             torch.randn(*shape, device=dev, generator=generator, out=x)
-        if step_noise is not None:
-            noise.copy_(step_noise, non_blocking=True)
-        else:
-            torch.randn(self.T, *shape, device=dev, generator=generator, out=noise)
+        if noise is not None:
+            if step_noise is not None:
+                noise.copy_(step_noise, non_blocking=True)
+            else:
+                torch.randn(self.T, *shape, device=dev, generator=generator, out=noise)
         plan.sample(x, noise, use_graph)
         idx, zq, ic, xyz = plan.decode(self.vae, x, denorm=True, num_atoms_total=fs.total_atoms)
         return {"latent": x, "idx": idx, "zq": zq, "ic_recon": ic, "xyz": xyz}

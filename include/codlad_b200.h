@@ -24,7 +24,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 1
+#define CB2_ABI_VERSION 2
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -88,9 +88,17 @@ CB2_API int cb2_plan_forward_partial(cb2_plan* p, const float* x, const float* t
  * posterior_mean_coef1, posterior_mean_coef2, (step != 0), 0} as fp32.  Builds the [T, 6016] adaLN table. */
 CB2_API int cb2_plan_set_schedule(cb2_plan* p, const float* t_of_step, const float* coef, int T, void* stream);
 
+/* DDIM counterpart of cb2_plan_set_schedule (IDDPM gaussian_diffusion.py ddim_sample, clip_denoised=False; the reference
+ * itself has no DDIM sampler).  HOST arrays: t_of_step [T] = timestep_map, ddim_coef [T][8] = {sqrt(1/acp), sqrt(1/acp - 1),
+ * sqrt(acp_prev), sqrt(max(0, 1 - acp_prev - sigma^2)), sigma * (step != 0), 0, 0, 0} as fp32, with
+ * sigma = eta sqrt((1 - acp_prev) / (1 - acp)) sqrt(1 - acp / acp_prev).  Builds the adaLN table; cb2_plan_sample then applies
+ * the DDIM update until the next cb2_plan_set_schedule. */
+CB2_API int cb2_plan_set_ddim_schedule(cb2_plan* p, const float* t_of_step, const float* ddim_coef, int T, void* stream);
+
 /* Replaces: GaussianDiffusion.p_sample_loop (gaussian_diffusion.py:451-547): T denoiser forwards + p_sample
  * updates, steps T-1 .. 0.  x [NB,L,3] in/out; noise [T,NB,L,3] (noise[s] is used at step s; the reference
- * draws it with randn_like at :440).  use_graph != 0 captures the whole loop in one CUDA graph and replays it. */
+ * draws it with randn_like at :440).  use_graph != 0 captures the whole loop in one CUDA graph and replays it.
+ * After cb2_plan_set_ddim_schedule the updates are DDIM steps; noise may then be NULL when every sigma is zero (eta = 0). */
 CB2_API int cb2_plan_sample(cb2_plan* p, float* x, const float* noise, int use_graph, void* stream);
 
 /* Decode-side geometry.  ca_full [F,L+2,3] device (untrimmed trace); HOST OR DEVICE (copied with
@@ -140,6 +148,11 @@ CB2_API int cb2_vq_lookup(const cb2_vae* v, const float* x, int NB, int L, const
  * x, noise, x_next [rows,C]; model_out [rows,2C]; coef [T,8] device; step_of_member [NB] int32 device;
  * rows = NB*rows_per_member. */
 CB2_API int cb2_p_sample(const float* x, const float* model_out, const float* noise, const float* coef,
+                 const int* step_of_member, int rows_per_member, int rows, int C, float* x_next, void* stream);
+
+/* One DDIM update (IDDPM ddim_sample, clip_denoised=False) on a model output the caller produced; same conventions as
+ * cb2_p_sample with coef = the [T,8] rows of cb2_plan_set_ddim_schedule.  noise may be NULL (no noise term). */
+CB2_API int cb2_ddim_sample(const float* x, const float* model_out, const float* noise, const float* coef,
                  const int* step_of_member, int rows_per_member, int rows, int C, float* x_next, void* stream);
 
 /* Replaces: ic_to_xyz (utils_ic.py:242-268) alone; same conventions as cb2_plan_set_topology but all DEVICE. */
