@@ -499,22 +499,23 @@ int edge_dispatch(Plan& p, int mode, int layer, const float* mod_base, int mod_s
                                     : launch_edge_f32(p, mode, layer, mod_base, mod_stride, s);
 }
 
-// One denoiser forward; when x_next != nullptr the last kernel also applies the p_sample update.
+// One denoiser forward; when x_next != nullptr the last kernel also applies the p_sample (or DDIM) update, then, when
+// inpaint_row != nullptr, the inpainting overwrite of the kept rows.
 int run_forward(Plan& p, const float* x, const float* mod_base, int mod_stride, const float* noise, float* x_next,
-                const float* coef_row, cudaStream_t s, int stop_after = -1) {
+                const float* coef_row, const float* inpaint_row, cudaStream_t s, int stop_after = -1) {
     int n = 0;
     auto done = [&]() { return stop_after >= 0 && ++n >= stop_after; };     // debug: stop after `stop_after` kernels
     const bool tc = p.precision == PREC_F16 && p.node_tc != nullptr;
-    auto node_update = [&](int phase, const float* xt, const float* nz, float* xn, const float* cf) {
-        return tc ? launch_node_update_tc(p, phase, mod_base, mod_stride, xt, nz, xn, cf, s)
-                  : launch_node_update(p, phase, mod_base, mod_stride, xt, nz, xn, cf, s);
+    auto node_update = [&](int phase, const float* xt, const float* nz, float* xn, const float* cf, const float* iq) {
+        return tc ? launch_node_update_tc(p, phase, mod_base, mod_stride, xt, nz, xn, cf, iq, s)
+                  : launch_node_update(p, phase, mod_base, mod_stride, xt, nz, xn, cf, iq, s);
     };
     if (int e = tc ? launch_node_init_tc(p, x, s) : launch_node_init(p, x, mod_base, mod_stride, s)) return e;
     if (done()) return 0;
     for (int l = 0; l < 3; ++l) {
         if (int e = edge_dispatch(p, EDGE_ENC_NODE, l, mod_base, mod_stride, s)) return e;
         if (done()) return 0;
-        if (int e = node_update(l, nullptr, nullptr, nullptr, nullptr)) return e;
+        if (int e = node_update(l, nullptr, nullptr, nullptr, nullptr, nullptr)) return e;
         if (done()) return 0;
         if (int e = edge_dispatch(p, EDGE_ENC_EDGE, l, mod_base, mod_stride, s)) return e;
         if (done()) return 0;
@@ -523,7 +524,8 @@ int run_forward(Plan& p, const float* x, const float* mod_base, int mod_stride, 
         if (int e = edge_dispatch(p, EDGE_DEC, l, mod_base, mod_stride, s)) return e;
         if (done()) return 0;
         const bool last = l == 2;
-        if (int e = node_update(3 + l, last ? x : nullptr, last ? noise : nullptr, last ? x_next : nullptr, last ? coef_row : nullptr)) return e;
+        if (int e = node_update(3 + l, last ? x : nullptr, last ? noise : nullptr, last ? x_next : nullptr, last ? coef_row : nullptr,
+                                last ? inpaint_row : nullptr)) return e;
         if (done()) return 0;
     }
     return 0;
@@ -540,7 +542,7 @@ int cb2_plan_forward_partial(cb2_plan* h, const float* x, const float* t, int st
     cudaStream_t s = (cudaStream_t)stream;
     if (int e = launch_timestep_mod(*p.model, t, p.NB, p.silu_c, p.mod, p.mod16, s)) return e;
     p.coef_steps = 0;
-    return run_forward(p, x, p.mod, CB2_MOD_TOTAL, nullptr, nullptr, nullptr, s, stop_after);
+    return run_forward(p, x, p.mod, CB2_MOD_TOTAL, nullptr, nullptr, nullptr, nullptr, s, stop_after);
 }
 
 int cb2_plan_forward(cb2_plan* h, const float* x, const float* t, float* out, void* stream) {
@@ -552,7 +554,7 @@ int cb2_plan_forward(cb2_plan* h, const float* x, const float* t, float* out, vo
     if (int e = launch_timestep_mod(*p.model, t, p.NB, p.silu_c, p.mod, p.mod16, s)) return e;
     p.launches += 2;
     p.coef_steps = 0;   // the table no longer holds a sampling schedule
-    if (int e = run_forward(p, x, p.mod, CB2_MOD_TOTAL, nullptr, nullptr, nullptr, s)) return e;
+    if (int e = run_forward(p, x, p.mod, CB2_MOD_TOTAL, nullptr, nullptr, nullptr, nullptr, s)) return e;
     CB2_CUDA(cudaMemcpyAsync(out, p.out6, (size_t)p.NB * p.L * 6 * sizeof(float), cudaMemcpyDeviceToDevice, s));
     return 0;
 }
@@ -582,15 +584,52 @@ int cb2_plan_set_ddim_schedule(cb2_plan* h, const float* t_of_step, const float*
     return set_schedule(h, t_of_step, ddim_coef, T, UPDATE_DDIM, (cudaStream_t)stream);
 }
 
+int cb2_plan_set_inpaint(cb2_plan* h, const unsigned char* keep, const float* x0, const float* q_coef, int T, void* stream) {
+    if (!h || !h->p.model) { set_error("set_inpaint: bad argument"); return 1; }
+    Plan& p = h->p;
+    if (!keep) { p.inpaint = false; return 0; }
+    if (!x0 || !q_coef || T <= 0) { set_error("set_inpaint: x0, q_coef and T > 0 are required with a keep mask"); return 1; }
+    if (T > p.mod_capacity) { set_error("set_inpaint: T=%d exceeds capacity %d", T, p.mod_capacity); return 1; }
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t N = (size_t)p.NB * p.L;
+    if (!p.inp_keep) {     // allocated once: the captured loop reads these addresses, so new contents need no recapture
+        unsigned char* keep_buf = nullptr;
+        float *x0_buf = nullptr, *eps_buf = nullptr, *coef_buf = nullptr;
+        int e = 0;
+        e |= dev_alloc(p.allocs, &keep_buf, N);
+        e |= dev_alloc(p.allocs, &x0_buf, N * 3);
+        e |= dev_alloc(p.allocs, &eps_buf, N * 3);
+        e |= dev_alloc(p.allocs, &coef_buf, (size_t)(p.mod_capacity + 1) * 2);
+        if (e) return e;    // the plan keeps none of them (those that were allocated are freed with it)
+        p.inp_keep = keep_buf; p.inp_x0 = x0_buf; p.inp_eps = eps_buf; p.inp_coef = coef_buf;
+    }
+    CB2_CUDA(cudaMemcpyAsync(p.inp_keep, keep, N, cudaMemcpyDeviceToDevice, s));
+    CB2_CUDA(cudaMemcpyAsync(p.inp_x0, x0, N * 3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    const size_t nq = (size_t)(T + 1) * 2;
+    if (p.inp_coef_host.size() != nq || memcmp(p.inp_coef_host.data(), q_coef, nq * sizeof(float)) != 0) {
+        p.inp_coef_host.assign(q_coef, q_coef + nq);
+        CB2_CUDA(cudaMemcpyAsync(p.inp_coef, q_coef, nq * sizeof(float), cudaMemcpyHostToDevice, s));
+        CB2_CUDA(cudaStreamSynchronize(s));     // the caller may free q_coef on return
+    }
+    p.inpaint_steps = T;
+    p.inpaint = true;
+    return 0;
+}
+
 static int enqueue_loop(cb2_plan* h, float* x, const float* noise, cudaStream_t s) {
     Plan& p = h->p;
     const size_t n3 = (size_t)p.NB * p.L * 3;
     CB2_CUDA(cudaMemcpyAsync(h->xa, x, n3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (p.inpaint) {
+        if (int e = launch_inpaint_init(p.inp_keep, p.inp_x0, p.inp_coef + (size_t)p.coef_steps * 2, p.NB * p.L, h->xa, p.inp_eps, s)) return e;
+        p.launches++;
+    }
     float *cur = h->xa, *nxt = h->xb;
     for (int step = p.coef_steps - 1; step >= 0; --step) {
         const float* mod_row = p.mod + (size_t)step * CB2_MOD_TOTAL;     // every member shares the step -> stride 0
         const float* step_noise = noise != nullptr ? noise + (size_t)step * n3 : nullptr;
-        if (int e = run_forward(p, cur, mod_row, 0, step_noise, nxt, p.coef + (size_t)step * 8, s)) {
+        const float* inpaint_row = p.inpaint ? p.inp_coef + (size_t)step * 2 : nullptr;
+        if (int e = run_forward(p, cur, mod_row, 0, step_noise, nxt, p.coef + (size_t)step * 8, inpaint_row, s)) {
             char prev[1024];
             snprintf(prev, sizeof(prev), "%s", g_err);
             const unsigned int* tl = edge_tc_trap_log();
@@ -614,10 +653,15 @@ int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, vo
     Plan& p = h->p;
     if (!h->frames_ready || p.coef_steps <= 0) { set_error("sample: set_frames / set_schedule must be called first"); return 1; }
     if (!noise && p.coef_noisy) { set_error("sample: noise may be NULL only on a DDIM schedule whose sigma are all zero (eta = 0)"); return 1; }
+    if (p.inpaint && p.inpaint_steps != p.coef_steps) {
+        set_error("sample: the inpainting table has T=%d, the schedule T=%d", p.inpaint_steps, p.coef_steps);
+        return 1;
+    }
     cudaStream_t s = (cudaStream_t)stream;
     if (!use_graph) return enqueue_loop(h, x, noise, s);
     // (kernel variants are chosen at capture time from the geometry: a frame set with / without padded residues needs its own graph)
-    if (!p.graph || p.graph_key[0] != x || p.graph_key[1] != noise || p.graph_steps != p.coef_steps || p.graph_all_full != p.all_full) {
+    if (!p.graph || p.graph_key[0] != x || p.graph_key[1] != noise || p.graph_steps != p.coef_steps || p.graph_all_full != p.all_full ||
+        p.graph_inpaint != p.inpaint) {
         if (p.graph) { cudaGraphExecDestroy(p.graph); p.graph = nullptr; }
         cudaStream_t cs;
         CB2_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
@@ -638,9 +682,10 @@ int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, vo
         cudaStreamDestroy(cs);
         if (ce != cudaSuccess) { set_error("graph instantiate failed: %s", cudaGetErrorString(ce)); p.graph = nullptr; return (int)ce; }
         p.graph_key[0] = x; p.graph_key[1] = noise; p.graph_steps = p.coef_steps; p.graph_all_full = p.all_full;
+        p.graph_inpaint = p.inpaint;
     }
     CB2_CUDA(cudaGraphLaunch(p.graph, s));
-    p.launches += 16LL * p.coef_steps;
+    p.launches += 16LL * p.coef_steps + (p.inpaint ? 1 : 0);
     return 0;
 }
 
@@ -758,7 +803,8 @@ int cb2_plan_run_stage(cb2_plan* h, const cb2_vae* v, int stage, int layer, floa
             const bool last = layer == 5, tc = p.precision == PREC_F16 && p.node_tc != nullptr;
             const float *xt = last ? h->xa : nullptr, *nz = last ? h->xa : nullptr, *cf = last ? p.coef : nullptr;
             float* xn = last ? h->xb : nullptr;
-            return tc ? launch_node_update_tc(p, layer, p.mod, 0, xt, nz, xn, cf, s) : launch_node_update(p, layer, p.mod, 0, xt, nz, xn, cf, s);
+            return tc ? launch_node_update_tc(p, layer, p.mod, 0, xt, nz, xn, cf, nullptr, s)
+                      : launch_node_update(p, layer, p.mod, 0, xt, nz, xn, cf, nullptr, s);
         }
         case 4: return launch_knn(p.X, p.lengths, p.F, p.L, p.K, p.nbr_dist, p.nbr_idx, s);
         case 5: return launch_edge_features(*p.model, p.X, p.lengths, p.nbr_idx, p.nbr_dist, p.F, p.L, p.K, p.E_dbg, p.hE0, p.precision, s);

@@ -89,10 +89,19 @@ struct Plan {
     int coef_steps = 0;
     int update_kind = 0;            // UPDATE_DDPM | UPDATE_DDIM, uniform over the schedule (the fused update selects on it)
     bool coef_noisy = true;         // the update reads its noise (DDPM always; DDIM when some sigma != 0)
+    // latent inpainting (cb2_plan_set_inpaint): plan-owned copies, allocated on first use; their addresses never change
+    bool inpaint = false;           // kept rows are overwritten after every update (uniform per launch, like update_kind)
+    int inpaint_steps = 0;          // T of the uploaded inpainting table (must equal coef_steps to sample)
+    unsigned char* inp_keep = nullptr;   // [NB*L] 1 = keep this row's latent
+    float* inp_x0 = nullptr;        // [NB*L, 3] normalised latent to keep
+    float* inp_eps = nullptr;       // [NB*L, 3] the fixed draw of the kept rows (saved from the initial noise)
+    float* inp_coef = nullptr;      // [mod_capacity + 1, 2] rows s: {sqrt(acp_prev[s]), sqrt(1 - acp_prev[s])}, row T: head
+    std::vector<float> inp_coef_host;    // what inp_coef holds (re-uploaded only when it changes)
     cudaGraphExec_t graph = nullptr;
     const void* graph_key[4] = {nullptr, nullptr, nullptr, nullptr};
     int graph_steps = 0;
     bool graph_all_full = false;    // the captured launches chose the masked / unmasked message kernels from all_full
+    bool graph_inpaint = false;     // the captured loop applies the inpainting overwrite
     std::vector<void*> allocs;
     void* tmaps = nullptr;          // host-side CUtensorMap storage of the tcgen05 edge kernels
     void* node_tc = nullptr;        // ... and of the tcgen05 node kernels
@@ -109,12 +118,17 @@ int launch_p_sample(const float* x, const float* out6, const float* noise, const
                     int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
 int launch_ddim_sample(const float* x, const float* out6, const float* noise, const float* coef_rows, const int* step_of_row,
                        int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
+// in place on the loop's initial latent x: eps = x and x = q_head[0] x0 + q_head[1] eps on the kept rows
+int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, float* x, float* eps, cudaStream_t s);
 float* plan_P(Plan& p, int which);
 
+// The fused update's kept-row overwrite reads the plan's inpainting buffers with `inpaint_row` = the step's
+// {sqrt(acp_prev), sqrt(1 - acp_prev)}; nullptr = no inpainting.
 struct NodeArgs;   // node.cu
 int launch_node_init(Plan& p, const float* x, const float* mod_base, int mod_stride_b, cudaStream_t s);
 int launch_node_update(Plan& p, int phase /*0..2 enc, 3..5 dec*/, const float* mod_base, int mod_stride_b,
-                       const float* x_t, const float* noise, float* x_next, const float* coef_row, cudaStream_t s);
+                       const float* x_t, const float* noise, float* x_next, const float* coef_row, const float* inpaint_row,
+                       cudaStream_t s);
 int launch_edge_f32(Plan& p, int mode, int layer, const float* mod_base, int mod_stride_b, cudaStream_t s);
 int launch_edge_tc(Plan& p, int mode, int layer, const float* mod_base, int mod_stride_b, cudaStream_t s);
 int edge_tc_prepare(Plan& p);
@@ -122,7 +136,7 @@ int node_tc_prepare(Plan& p);
 void node_tc_release(Plan& p);
 int launch_node_init_tc(Plan& p, const float* x, cudaStream_t s);
 int launch_node_update_tc(Plan& p, int phase, const float* mod_base, int mod_stride_b, const float* x_t, const float* noise,
-                          float* x_next, const float* coef_row, cudaStream_t s);
+                          float* x_next, const float* coef_row, const float* inpaint_row, cudaStream_t s);
 void edge_tc_release(Plan& p);
 const unsigned int* edge_tc_trap_log();      // debug (CB2_TRAP_DEBUG): record of a timed-out barrier wait, or nullptr
 

@@ -12,7 +12,10 @@
 //    (W1 [h_V_i | h_E | h_V_j] = W1a h_V_i + W1b h_E + W1c h_V_j: the a/c products are per node),
 //    and for the last decoder layer FinalLayer (latent_model.py:21-35) fused with the DDPM
 //    p_sample update (diffusion_and_flow/gaussian_diffusion.py:303-318,345-351,440-446) or, on a
-//    DDIM schedule, IDDPM's ddim_sample update (ddim_update, common.cuh).
+//    DDIM schedule, IDDPM's ddim_sample update (ddim_update, common.cuh).  With latent inpainting on,
+//    the kept rows are then overwritten with the forward marginal of their latent (inpaint_level).
+//  * inpaint_init:  before the first step, saves the kept rows' initial noise as their fixed draw and
+//    puts them at the head level of the schedule.
 //
 // fp32 SIMT: 16 rows per CTA, 128 threads, thread = output column (see tile_gemm.cuh).
 #include "model.h"
@@ -111,7 +114,10 @@ __device__ __forceinline__ void rows_ln(float* sB, float* sStat, int tid) {
     }
 }
 
-__global__ void __launch_bounds__(128) node_update_kernel(NodeParams p) {
+// INPAINT: the final update is followed by the inpainting overwrite of the rows `ir` keeps (the last node launch of a step with
+// latent inpainting on); otherwise `ir` is unused.
+template <bool INPAINT>
+__global__ void __launch_bounds__(128) node_update_kernel(NodeParams p, InpaintRows ir) {
     extern __shared__ __align__(16) float smem[];
     float* sA = smem;                  // [16][128] current h
     float* sMid = sA + NR * 128;       // [16][512] S rows, then FFN hidden
@@ -304,6 +310,12 @@ __global__ void __launch_bounds__(128) node_update_kernel(NodeParams p) {
                 const float mean_ = p.coef[4] * x0 + p.coef[5] * x;
                 p.x_next[(size_t)n * 3 + lane] = mean_ + p.coef[6] * expf(0.5f * logvar) * p.noise[(size_t)n * 3 + lane];
             }
+            if constexpr (INPAINT) {
+                if (lane < 3 && ir.keep[n]) {
+                    const size_t k = (size_t)n * 3 + lane;
+                    p.x_next[k] = inpaint_level(ir.level, ir.x0[k], ir.eps[k]);
+                }
+            }
         }
     }
 }
@@ -336,6 +348,15 @@ __global__ void ddim_sample_kernel(const float* __restrict__ x, const float* __r
     x_next[t] = ddim_update(x[t], out6[(size_t)row * 2 * C + d], cf, noise != nullptr ? noise + t : nullptr);
 }
 
+__global__ void inpaint_init_kernel(const unsigned char* __restrict__ keep, const float* __restrict__ x0, const float* __restrict__ q_head,
+                                    int n_rows, float* __restrict__ x, float* __restrict__ eps) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_rows * 3 || !keep[t / 3]) return;
+    const float e = x[t];
+    eps[t] = e;
+    x[t] = inpaint_level(q_head, x0[t], e);
+}
+
 }  // namespace
 
 int launch_timestep_mod(const DenoiserModel& m, const float* tvals, int n, float* scratch_silu_c, float* mod, __half* mod16, cudaStream_t s) {
@@ -366,14 +387,23 @@ int launch_ddim_sample(const float* x, const float* out6, const float* noise, co
     return 0;
 }
 
-static int node_launch(Plan& p, NodeParams& np, cudaStream_t s) {
+int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, float* x, float* eps, cudaStream_t s) {
+    const int total = n_rows * 3;
+    inpaint_init_kernel<<<(total + 255) / 256, 256, 0, s>>>(keep, x0, q_head, n_rows, x, eps);
+    CB2_LAUNCH_CHECK();
+    return 0;
+}
+
+static int node_launch(Plan& p, NodeParams& np, cudaStream_t s, const InpaintRows* ir = nullptr) {
     const size_t smem = (size_t)(NR * 128 + NR * 512 + NR * 128) * 4;
     static bool attr = false;
     if (!attr) {
-        CB2_CUDA(cudaFuncSetAttribute(node_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CB2_CUDA(cudaFuncSetAttribute(node_update_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CB2_CUDA(cudaFuncSetAttribute(node_update_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr = true;
     }
-    node_update_kernel<<<(np.N + NR - 1) / NR, 128, smem, s>>>(np);
+    if (ir != nullptr) node_update_kernel<true><<<(np.N + NR - 1) / NR, 128, smem, s>>>(np, *ir);
+    else node_update_kernel<false><<<(np.N + NR - 1) / NR, 128, smem, s>>>(np, InpaintRows{});
     CB2_LAUNCH_CHECK();
     p.launches++;
     return 0;
@@ -401,7 +431,7 @@ int launch_node_init(Plan& p, const float* x, const float* mod_base, int mod_str
 }
 
 int launch_node_update(Plan& p, int phase, const float* mod_base, int mod_stride_b, const float* x_t, const float* noise,
-                       float* x_next, const float* coef_row, cudaStream_t s) {
+                       float* x_next, const float* coef_row, const float* inpaint_row, cudaStream_t s) {
     const DenoiserModel& m = *p.model;
     NodeParams np;
     base_params(p, np);
@@ -440,6 +470,10 @@ int launch_node_update(Plan& p, int phase, const float* mod_base, int mod_stride
             np.out6 = p.out6;
             np.x_t = x_t; np.noise = noise; np.x_next = x_next; np.coef = coef_row;
             np.ddim = p.update_kind == UPDATE_DDIM;
+            if (inpaint_row != nullptr) {
+                const InpaintRows ir{p.inp_keep, p.inp_x0, p.inp_eps, inpaint_row};
+                return node_launch(p, np, s, &ir);
+            }
         }
     }
     return node_launch(p, np, s);

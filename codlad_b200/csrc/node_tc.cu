@@ -13,7 +13,8 @@
 //
 //   P1  acc = W3 . S^T                          EA  h1 = gate1 * mod(LN(h_V + (acc + cnt b3)/30))
 //   P2  4 x acc_c = Win[c] . h1^T               EG  mid_c = 2 GELU(acc_c + b_in)
-//   P3  acc = sum_c (Wout[:, c]/2) . mid_c^T    EB  h2 = mask * gate2 * mod(LN(h1 + acc + b_out))   (+ FinalLayer, p_sample)
+//   P3  acc = sum_c (Wout[:, c]/2) . mid_c^T    EB  h2 = mask * gate2 * mod(LN(h1 + acc + b_out))   (+ FinalLayer, p_sample / DDIM,
+//                                                                                                       inpainting overwrite)
 //   P4  own / gathered halves of the next edge MLPs' first layer        EP  -> P16 (fp16 [own + bias | gathered (+ table)])
 //
 // State h_V stays fp32 in HBM; only MMA operands are fp16 (fp32 accumulation in TMEM).
@@ -25,7 +26,8 @@ using namespace tc;
 
 namespace {
 
-__global__ void __launch_bounds__(NODE_CTA_THREADS, 1) node_tc_kernel(const __grid_constant__ CUtensorMap wmap, const NodeTcParams p) {
+template <bool INPAINT>
+__device__ __forceinline__ void node_tc_run(const CUtensorMap& wmap, const NodeTcParams& p, const InpaintRows& ir) {
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5;
@@ -40,17 +42,29 @@ __global__ void __launch_bounds__(NODE_CTA_THREADS, 1) node_tc_kernel(const __gr
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = s_tmem;
-    node_block(smem, tmem_base, &wmap, p, blockIdx.x * NT, p.N, true);
+    node_block<INPAINT>(smem, tmem_base, &wmap, p, blockIdx.x * NT, p.N, true, ir);
     if (tid == 0) trace_window(p.trace, p.trace_slot, true);
     if (warp == 16) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+}
+
+__global__ void __launch_bounds__(NODE_CTA_THREADS, 1) node_tc_kernel(const __grid_constant__ CUtensorMap wmap, const NodeTcParams p) {
+    node_tc_run<false>(wmap, p, InpaintRows{});
+}
+
+// the last node launch of a step with latent inpainting on
+__global__ void __launch_bounds__(NODE_CTA_THREADS, 1) node_tc_inpaint_kernel(const __grid_constant__ CUtensorMap wmap, const NodeTcParams p,
+                                                                             const __grid_constant__ InpaintRows ir) {
+    node_tc_run<true>(wmap, p, ir);
 }
 
 
 struct NodeTcState { CUtensorMap wmap; };
 
-int node_tc_launch(Plan& p, NodeTcParams& np, cudaStream_t s) {
+int node_tc_launch(Plan& p, NodeTcParams& np, cudaStream_t s, const InpaintRows* ir = nullptr) {
     const NodeTcState& st = *reinterpret_cast<const NodeTcState*>(p.node_tc);
-    CB2_CUDA(launch_pdl(node_tc_kernel, dim3((np.N + NT - 1) / NT), dim3(NODE_CTA_THREADS), NODE_TC_SMEM, s, st.wmap, np));
+    const dim3 grid((np.N + NT - 1) / NT), block(NODE_CTA_THREADS);
+    if (ir != nullptr) CB2_CUDA(launch_pdl(node_tc_inpaint_kernel, grid, block, NODE_TC_SMEM, s, st.wmap, np, *ir));
+    else CB2_CUDA(launch_pdl(node_tc_kernel, grid, block, NODE_TC_SMEM, s, st.wmap, np));
     CB2_LAUNCH_CHECK();
     p.launches++;
     return 0;
@@ -73,6 +87,7 @@ int node_tc_prepare(Plan& p) {
     p.node_tc = st;
     if (encode_rows_map(fn, &st->wmap, p.model->dev_f16, (size_t)p.model->n_f16_blocks * 128, 128)) return 1;
     CB2_CUDA(cudaFuncSetAttribute(node_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NODE_TC_SMEM));
+    CB2_CUDA(cudaFuncSetAttribute(node_tc_inpaint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NODE_TC_SMEM));
     return 0;
 }
 
@@ -140,9 +155,13 @@ void node_tc_update_params(Plan& p, int phase, const float* mod_base, int mod_st
 }
 
 int launch_node_update_tc(Plan& p, int phase, const float* mod_base, int mod_stride_b, const float* x_t, const float* noise,
-                          float* x_next, const float* coef_row, cudaStream_t s) {
+                          float* x_next, const float* coef_row, const float* inpaint_row, cudaStream_t s) {
     NodeTcParams np;
     node_tc_update_params(p, phase, mod_base, mod_stride_b, x_t, noise, x_next, coef_row, np);
+    if (inpaint_row != nullptr && np.do_final) {
+        const InpaintRows ir{p.inp_keep, p.inp_x0, p.inp_eps, inpaint_row};
+        return node_tc_launch(p, np, s, &ir);
+    }
     return node_tc_launch(p, np, s);
 }
 

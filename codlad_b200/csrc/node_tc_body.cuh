@@ -78,9 +78,11 @@ constexpr size_t NODE_TC_SMEM = (size_t)N_SLOT * TILE_BYTES + (size_t)N_ACT * AC
 // One block of NT nodes [node0, min(node0 + NT, n_end)) through the whole node update.  Called by every thread of a 576-thread CTA
 // (16 epilogue warps, MMA warp 16, TMA warp 17) with `smem` = the CTA's dynamic shared memory (NODE_TC_SMEM bytes, 1024-aligned,
 // free of live mbarriers) and an allocated 512-column TMEM region.  `dep_wait`: the epilogue warps execute griddepcontrol.wait
-// before their first read of activations (stand-alone kernel); the fused caller has already waited.
+// before their first read of activations (stand-alone kernel); the fused caller has already waited.  INPAINT: the final update
+// is followed by the inpainting overwrite of the rows `ir` keeps.
+template <bool INPAINT>
 __device__ __forceinline__ void node_block(unsigned char* smem, const uint32_t tmem_base, const CUtensorMap* wmap_p, const NodeTcParams& p,
-                                           const int node0, const int n_end, const bool dep_wait) {
+                                           const int node0, const int n_end, const bool dep_wait, const InpaintRows& ir) {
     unsigned char* sW = smem;                                          // N_SLOT weight slots (A operands)
     unsigned char* sAct = sW + N_SLOT * TILE_BYTES;                    // N_ACT activation tiles (B operands)
     float* sRed = reinterpret_cast<float*>(sAct + N_ACT * ACT_BYTES);  // [2 uses][4 node groups][4 feature quarters][16] LayerNorm partials
@@ -419,8 +421,9 @@ __device__ __forceinline__ void node_block(unsigned char* smem, const uint32_t t
             }
         }
         if (p.do_final) {
-            // ---- FinalLayer (adaLN modulate + Linear 128 -> 6) fused with the DDPM p_sample (or DDIM) update.  The fp32 rows are parked in
-            //      shared memory (the FFN hidden tiles are dead); each warp then owns two nodes, lanes across features ----
+            // ---- FinalLayer (adaLN modulate + Linear 128 -> 6) fused with the DDPM p_sample (or DDIM) update and the inpainting
+            //      overwrite of kept rows.  The fp32 rows are parked in shared memory (the FFN hidden tiles are dead); each warp
+            //      then owns two nodes, lanes across features ----
             float* sH = reinterpret_cast<float*>(act_tile(2));
 #pragma unroll
             for (int i = 0; i < NPTH; ++i) sH[(nl0 + i) * 128 + fl] = v[i];
@@ -472,6 +475,12 @@ __device__ __forceinline__ void node_block(unsigned char* smem, const uint32_t t
                     const float x0 = p.coef[2] * x - p.coef[3] * eps;
                     const float mean_ = p.coef[4] * x0 + p.coef[5] * x;
                     p.x_next[(size_t)n * 3 + lane] = mean_ + p.coef[6] * expf(0.5f * logvar) * p.noise[(size_t)n * 3 + lane];
+                }
+                if constexpr (INPAINT) {
+                    if (lane < 3 && ir.keep[n]) {
+                        const size_t k = (size_t)n * 3 + lane;
+                        p.x_next[k] = inpaint_level(ir.level, ir.x0[k], ir.eps[k]);
+                    }
                 }
             }
         }

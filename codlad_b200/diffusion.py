@@ -7,7 +7,8 @@ computed once).  The step loop itself is CUDA:
     (T denoiser forwards + T fused p_sample updates) to `cb2_plan_sample` as one CUDA graph;
   * any other callable goes through a generic loop whose update is the `cb2_p_sample` kernel.
 `ddim_sample_loop` (IDDPM's DDIM sampler, which the reference does not ship) takes the same two routes with the DDIM
-update (`cb2_plan_set_ddim_schedule` / `cb2_ddim_sample`).
+update (`cb2_plan_set_ddim_schedule` / `cb2_ddim_sample`).  `inpaint_coef_table` feeds latent inpainting on a plan
+(`cb2_plan_set_inpaint`, `sampler.Backmapper.resample`).
 `training_losses` (config 5, "next" row f-1 of SURVEY.md section 8) is not implemented yet.
 """
 from __future__ import annotations
@@ -124,6 +125,14 @@ class SpacedDiffusion:
         c[:, 3] = np.sqrt(np.maximum(0.0, 1.0 - ac_prev - sigma ** 2))
         c[:, 4] = sigma * (np.arange(self.num_timesteps) != 0)
         return c
+
+    def inpaint_coef_table(self) -> np.ndarray:
+        """[T+1, 2] fp32 rows consumed by cb2_plan_set_inpaint, computed in float64 and rounded once.  Row s < T is
+        {sqrt(acp_prev[s]), sqrt(1 - acp_prev[s])}, the level a kept row takes after step s; row T is {sqrt(acp[T-1]),
+        sqrt(1 - acp[T-1])}, its level before the first step.  Row 0 is exactly (1, 0), so kept rows end at their latent.
+        The same table serves DDPM and DDIM on this respacing."""
+        level = np.append(self.alphas_cumprod_prev, self.alphas_cumprod[-1])
+        return np.stack([np.sqrt(level), np.sqrt(1.0 - level)], axis=1).astype(np.float32)
 
     def _coef_on(self, device, eta=None):
         """coef_table (eta None) or ddim_coef_table(eta) on `device`, uploaded once."""

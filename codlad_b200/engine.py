@@ -163,6 +163,27 @@ class Plan:
                 "sample")
         return x
 
+    def set_inpaint(self, keep, x0, q_coef):
+        """Latent inpainting for the following sample() calls: the rows where keep [NB,L] (CUDA bool) is True follow the
+        normalised latent x0 [NB,L,3] (CUDA fp32), the others are regenerated.  q_coef = SpacedDiffusion.inpaint_coef_table()
+        of the plan's schedule.  keep and x0 are copied into plan-owned buffers, so x0 may be the tensor later passed to
+        sample(); changing them does not recapture the graph."""
+        if not torch.is_tensor(keep) or keep.dtype != torch.bool or tuple(keep.shape) != (self.NB, self.L):
+            raise ValueError(f"keep must be a bool tensor of shape {(self.NB, self.L)}")
+        if not torch.is_tensor(x0) or x0.dtype != torch.float32 or tuple(x0.shape) != (self.NB, self.L, 3):
+            raise ValueError(f"x0 must be a float32 tensor of shape {(self.NB, self.L, 3)}")
+        if keep.device != self.device or x0.device != self.device:
+            raise ValueError(f"keep and x0 must be on {self.device}")
+        q = torch.as_tensor(np.asarray(q_coef), dtype=torch.float32).contiguous()
+        if q.dim() != 2 or q.shape[0] < 2 or q.shape[1] != 2:
+            raise ValueError("q_coef must be a [T+1, 2] table (SpacedDiffusion.inpaint_coef_table)")
+        N.check(N.lib().cb2_plan_set_inpaint(self.handle, N.dptr(keep.to(torch.uint8).contiguous()), N.dptr(x0.contiguous()),
+                                             q.data_ptr(), int(q.shape[0]) - 1, N.stream_ptr()), "set_inpaint")
+
+    def clear_inpaint(self):
+        """Turn latent inpainting off: sample() regenerates every row again."""
+        N.check(N.lib().cb2_plan_set_inpaint(self.handle, None, None, None, 0, N.stream_ptr()), "set_inpaint")
+
     def run_edge_kernel(self, mode: int, layer: int):
         """Measurement hook: one per-edge kernel on the current state (0 enc node msg, 1 enc edge update, 2 dec msg)."""
         N.check(N.lib().cb2_plan_run_edge_kernel(self.handle, int(mode), int(layer), N.stream_ptr()), "run_edge_kernel")

@@ -165,7 +165,28 @@ class Backmapper:
                use_graph: bool = True, generator: torch.Generator = None):
         """Device-resident path: returns dict(latent, idx, ic_recon, xyz) of CUDA tensors.
         z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted.  DDIM with eta = 0 uses no
-        step noise: `step_noise` is ignored."""
+        step noise: `step_noise` is ignored.  Every residue is sampled anew, also after resample() on the same plan."""
+        plan.clear_inpaint()
+        return self._sample(plan, fs, z, step_noise, use_graph, generator)
+
+    def resample(self, plan: Plan, fs: FrameSet, latent: torch.Tensor, keep: torch.Tensor, z: torch.Tensor = None,
+                 step_noise: torch.Tensor = None, generator: torch.Generator = None):
+        """Latent inpainting: keep the residues of an earlier pass where keep [NB,L] (bool) is True and sample the others
+        anew, conditioned on the kept ones through the denoiser.  latent [NB,L,3] is that pass's normalised latent
+        (`sample(...)["latent"]`, which may be passed as is).  Kept rows follow the forward marginal of their latent with the
+        fixed draw z and end at it exactly, so they keep their VQ index.  z and step_noise as in sample().  Returns the same
+        dict as sample()."""
+        shape = (fs.NB, fs.L, 3)
+        if not torch.is_tensor(latent) or latent.dtype != torch.float32 or tuple(latent.shape) != shape:
+            raise ValueError(f"latent must be a float32 tensor of shape {shape}")
+        if not torch.is_tensor(keep) or keep.dtype != torch.bool or tuple(keep.shape) != shape[:2]:
+            raise ValueError(f"keep must be a bool tensor of shape {shape[:2]}")
+        if latent.device != plan.device or keep.device != plan.device:
+            raise ValueError(f"latent and keep must be on {plan.device}")
+        plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())      # copies latent before z overwrites its buffer
+        return self._sample(plan, fs, z, step_noise, True, generator)
+
+    def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator):
         dev = plan.device
         shape = (fs.NB, fs.L, 3)
         noisy = self.sampler == "ddpm" or self.eta != 0

@@ -24,7 +24,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 2
+#define CB2_ABI_VERSION 3
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -98,8 +98,21 @@ CB2_API int cb2_plan_set_ddim_schedule(cb2_plan* p, const float* t_of_step, cons
 /* Replaces: GaussianDiffusion.p_sample_loop (gaussian_diffusion.py:451-547): T denoiser forwards + p_sample
  * updates, steps T-1 .. 0.  x [NB,L,3] in/out; noise [T,NB,L,3] (noise[s] is used at step s; the reference
  * draws it with randn_like at :440).  use_graph != 0 captures the whole loop in one CUDA graph and replays it.
- * After cb2_plan_set_ddim_schedule the updates are DDIM steps; noise may then be NULL when every sigma is zero (eta = 0). */
+ * After cb2_plan_set_ddim_schedule the updates are DDIM steps; noise may then be NULL when every sigma is zero (eta = 0).
+ * With inpainting on (cb2_plan_set_inpaint) the kept rows follow their latent and T must equal the inpainting table's. */
 CB2_API int cb2_plan_sample(cb2_plan* p, float* x, const float* noise, int use_graph, void* stream);
+
+/* Latent inpainting for the following cb2_plan_sample calls (the replacement method; the reference has no such sampler):
+ * the rows marked in keep [NB*L] (u8, non-zero = keep) follow their normalised latent x0 [NB,L,3], every other row is
+ * regenerated, conditioned on the kept ones through the denoiser.  With eps = the kept rows of the initial noise x, a kept
+ * row starts at q_coef[T] and after the update of step s is overwritten with q_coef[s], where a row {a, b} means
+ * a * x0 + b * eps (fp32, two rounded products and one rounded sum).  q_coef [T+1][2] is a HOST array:
+ * rows 0..T-1 = {sqrt(acp_prev), sqrt(1 - acp_prev)} of each step, row T = {sqrt(acp[T-1]), sqrt(1 - acp[T-1])}, so that
+ * kept rows end at x0 exactly.  It serves DDPM and DDIM schedules alike.  keep and x0 are copied into plan-owned buffers
+ * (x0 may therefore be the x later passed to cb2_plan_sample); new contents need no graph recapture.  keep == NULL turns
+ * inpainting off (x0 and q_coef are then ignored).  Each sample call with inpainting on launches one more kernel. */
+CB2_API int cb2_plan_set_inpaint(cb2_plan* p, const unsigned char* keep, const float* x0, const float* q_coef, int T,
+                         void* stream);
 
 /* Decode-side geometry.  ca_full [F,L+2,3] device (untrimmed trace); HOST OR DEVICE (copied with
  * cudaMemcpyDefault): csr_row_ptr [F*L+1] / csr_col [E]
