@@ -1,4 +1,5 @@
 // C ABI (include/codlad_b200.h): model packing, plan management and the step-loop driver.
+#include <math.h>
 #include <stdarg.h>
 #include <string.h>
 
@@ -9,6 +10,7 @@
 #include "../../include/codlad_b200.h"
 #include "decode.h"
 #include "model.h"
+#include "repair.h"
 
 namespace cb2 {
 
@@ -107,6 +109,7 @@ struct cb2_plan {
     float *edge_w = nullptr, *S40 = nullptr, *phi = nullptr, *ic = nullptr, *zq = nullptr;
     int* vq_idx = nullptr;
     float *xa = nullptr, *xb = nullptr;     // ping-pong latents of the sampling loop
+    float4* clash_bounds = nullptr;         // [NB*L] residue centre + radius of cb2_plan_residue_clashes
     int keep_debug = 0;
     bool frames_ready = false, topo_ready = false;
 };
@@ -749,6 +752,20 @@ int cb2_plan_decode(cb2_plan* h, const cb2_vae* v, const float* latent, int deno
                                      nullptr, s)) return e;
         p.launches += 1;
     }
+    return 0;
+}
+
+int cb2_plan_residue_clashes(cb2_plan* h, const float* xyz, float threshold, int grow, int* counts, unsigned char* keep, void* stream) {
+    if (!h || !xyz || !counts) { set_error("residue_clashes: null argument"); return 1; }
+    if (!h->topo_ready) { set_error("residue_clashes: cb2_plan_set_topology has not been called"); return 1; }
+    Plan& p = h->p;
+    if (!(threshold > 0.0f) || !isfinite(threshold)) { set_error("residue_clashes: threshold must be finite and positive"); return 1; }
+    if (grow < 0 || (grow > 0 && grow >= p.K)) { set_error("residue_clashes: grow=%d outside [0, K=%d)", grow, p.K); return 1; }
+    if (!h->clash_bounds)
+        if (int e = dev_alloc(p.allocs, &h->clash_bounds, (size_t)p.NB * p.L)) return e;
+    if (int e = launch_residue_clashes(xyz, h->slot_atom, h->out_off, p.lengths, p.frame_of, p.nbr_idx, p.NB, p.L, p.K, threshold, grow,
+                                       h->clash_bounds, counts, keep, (cudaStream_t)stream)) return e;
+    p.launches += keep ? 3 : 2;
     return 0;
 }
 

@@ -9,6 +9,7 @@
 // full symmetric matrix, like `(bonds != ref_bonds).sum()` does.
 #include "../../include/codlad_b200.h"
 #include "common.cuh"
+#include "pair_dist.cuh"
 
 namespace cb2 {
 
@@ -162,23 +163,17 @@ __global__ void __launch_bounds__(256) superposed_rmsd_kernel(const float* __res
 // fp32 distances in the reference's operation order; the three sums are accumulated in double, per CTA and then over CTAs in a
 // fixed order (deterministic).
 constexpr int PL_THREADS = 256, PL_MAX_BLOCKS = 592;
-constexpr float PL_EPS = 1e-7f;                          // test.py:27
 
 __device__ __forceinline__ float pair_dist(const float* __restrict__ x, const long long* __restrict__ row, int width) {
+    if (width == 2) return atom_pair_dist(x + row[0] * 3, x + row[1] * 3);      // pair_dist.cuh, shared with the clash counts
     float d2 = 0.f;
-    if (width == 2) {
-        const float *a = x + row[0] * 3, *b = x + row[1] * 3;
+    const float *a = x + row[0] * 3, *b = x + row[1] * 3, *c = x + row[2] * 3, *e = x + row[3] * 3;
 #pragma unroll
-        for (int k = 0; k < 3; ++k) { const float d = __fsub_rn(a[k], b[k]); d2 = __fadd_rn(d2, __fmul_rn(d, d)); }
-    } else {
-        const float *a = x + row[0] * 3, *b = x + row[1] * 3, *c = x + row[2] * 3, *e = x + row[3] * 3;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            const float d = __fsub_rn(__fdiv_rn(__fadd_rn(a[k], b[k]), 2.f), __fdiv_rn(__fadd_rn(c[k], e[k]), 2.f));
-            d2 = __fadd_rn(d2, __fmul_rn(d, d));
-        }
+    for (int k = 0; k < 3; ++k) {
+        const float d = __fsub_rn(__fdiv_rn(__fadd_rn(a[k], b[k]), 2.f), __fdiv_rn(__fadd_rn(c[k], e[k]), 2.f));
+        d2 = __fadd_rn(d2, __fmul_rn(d, d));
     }
-    return __fsqrt_rn(__fadd_rn(d2, PL_EPS));
+    return __fsqrt_rn(__fadd_rn(d2, PAIR_EPS));
 }
 
 __global__ void __launch_bounds__(PL_THREADS) pair_losses_kernel(const float* __restrict__ xyz, const float* __restrict__ xyz_data,

@@ -6,6 +6,8 @@ host<->device copies only.
 from __future__ import annotations
 
 import ctypes as C
+import math
+import numbers
 
 import numpy as np
 import torch
@@ -19,6 +21,15 @@ def sinusoid_freqs() -> torch.Tensor:
     import math
     half = 128
     return torch.exp(-math.log(10000) * torch.arange(start=0, end=half, dtype=torch.float32) / half)
+
+
+def check_clash_args(threshold, grow, K: int):
+    """Arguments of the per-residue clash criterion: a finite positive threshold (Angstrom) and 0 <= grow < K (grow = 0 also on a
+    decode-only plan, K = 0).  Raises ValueError; touches no device."""
+    if isinstance(threshold, bool) or not isinstance(threshold, numbers.Real) or not math.isfinite(threshold) or threshold <= 0:
+        raise ValueError(f"threshold must be a finite positive number, got {threshold!r}")
+    if isinstance(grow, bool) or not isinstance(grow, numbers.Integral) or grow < 0 or (grow > 0 and grow >= K):
+        raise ValueError(f"grow must be an integer in [0, {K}), got {grow!r}")
 
 
 class DenoiserEngine:
@@ -204,6 +215,22 @@ class Plan:
                                         N.dptr(ic) if ic is not None else None, N.dptr(xyz) if xyz is not None else None,
                                         N.stream_ptr()), "decode")
         return idx, zq, ic, xyz
+
+    def residue_clashes(self, xyz, threshold: float = 1.2, grow: int = 0):
+        """Per-residue clash counts of a decoded sample and the keep mask that resamples the clashing residues
+        (cb2_plan_residue_clashes; needs set_topology).  xyz [total atoms, 3] CUDA fp32 as decode() writes it.  Returns
+        (counts [NB, L] int32, keep [NB, L] bool): counts[b, i] = atom pairs of residue i with other residues of member b closer
+        than `threshold` (peptide bond left out), keep False where residue i or one of its `grow` nearest other residues clashes."""
+        if not torch.is_tensor(xyz) or xyz.dtype != torch.float32 or xyz.dim() != 2 or xyz.shape[1] != 3:
+            raise ValueError("xyz must be a float32 tensor of shape [total atoms, 3]")
+        if xyz.device != self.device:
+            raise ValueError(f"xyz must be on {self.device}")
+        check_clash_args(threshold, grow, self.K)
+        counts = torch.empty(self.NB, self.L, device=self.device, dtype=torch.int32)
+        keep = torch.empty(self.NB, self.L, device=self.device, dtype=torch.uint8)
+        N.check(N.lib().cb2_plan_residue_clashes(self.handle, N.dptr(xyz.contiguous()), C.c_float(threshold), int(grow), N.dptr(counts),
+                                                 N.dptr(keep), N.stream_ptr()), "residue_clashes")
+        return counts, keep.view(torch.bool)
 
     # -- debug -------------------------------------------------------------------------------------
     def buffer(self, name: str) -> torch.Tensor:

@@ -18,9 +18,19 @@ import torch
 
 from . import batching, distributed, topology, weights
 from .diffusion import create_diffusion
-from .engine import DenoiserEngine, Plan, VaeEngine
+from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args
 
 VAE_DATA = {"N6": "PED", "K3": "PDB", "K4": "Atlas"}
+
+
+def clash_pair_totals(counts: torch.Tensor) -> torch.Tensor:
+    """Clashing atom pairs per member (int64 [NB]) from per-residue counts [NB, L], where every pair counts for both residues."""
+    return counts.sum(1, dtype=torch.int64) // 2
+
+
+def repair_accept(prev_pairs: torch.Tensor, new_pairs: torch.Tensor) -> torch.Tensor:
+    """The acceptance rule of Backmapper.repair, per member: take the resampled latent only if it has fewer clashing pairs."""
+    return new_pairs < prev_pairs
 
 
 @dataclass
@@ -185,6 +195,64 @@ class Backmapper:
             raise ValueError(f"latent and keep must be on {plan.device}")
         plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())      # copies latent before z overwrites its buffer
         return self._sample(plan, fs, z, step_noise, True, generator)
+
+    def residue_clashes(self, plan: Plan, fs: FrameSet, xyz: torch.Tensor, threshold: float = 1.2, grow: int = 0):
+        """Per-residue clashes of a decoded sample, on the device (cb2_plan_residue_clashes): clash_result's criterion
+        (test.py:118-139) per residue, with no reference structure.  xyz [fs.total_atoms, 3] as sample() returns it.  Returns
+        (counts int32 [NB, L], keep bool [NB, L]): counts[b, i] = atom pairs of residue i with other residues of member b closer
+        than `threshold` Angstrom, the peptide bond C(i)-N(i+1) left out (each pair counts for both residues); keep is False
+        where residue i or one of its `grow` nearest other residues (the plan's k-NN graph) clashes -- the mask resample() takes."""
+        shape = (fs.total_atoms, 3)
+        if not torch.is_tensor(xyz) or xyz.dtype != torch.float32 or tuple(xyz.shape) != shape:
+            raise ValueError(f"xyz must be a float32 tensor of shape {shape}")
+        if xyz.device != plan.device:
+            raise ValueError(f"xyz must be on {plan.device}")
+        return plan.residue_clashes(xyz, threshold, grow)
+
+    def repair(self, plan: Plan, fs: FrameSet, out: dict, max_rounds: int = 3, grow: int = 0, threshold: float = 1.2,
+               generator: torch.Generator = None):
+        """Clash-driven repair of a backmapped sample `out` (the dict of sample() / resample()): each round flags the clashing
+        residues (residue_clashes), stops when no member has a clash, and otherwise resamples the flagged residues of every
+        member with latent inpainting, fresh noise from `generator`.  Per member the new latent is accepted only when its number
+        of clashing pairs went down; otherwise the member keeps its previous latent.  The accepted latents are decoded once at the
+        end.  Kept residues keep their latent and VQ index; their coordinates can still move where the IC decoder's radius graph
+        reaches a regenerated neighbour.  A round costs one resample pass (one sampling pass plus decode).
+        Returns the dict of sample() plus `clashes` (int32 [NB, L], the counts of the returned structure) and `clash_pairs`
+        (int64 [rounds run + 1, NB], clashing pairs per member; row 0 is the input's).  The plan is left for plain sample()."""
+        if not isinstance(out, dict) or not all(k in out for k in ("latent", "idx", "zq", "ic_recon", "xyz")):
+            raise ValueError("out must be the dict returned by sample() or resample()")
+        if isinstance(max_rounds, bool) or not isinstance(max_rounds, int) or max_rounds < 0:
+            raise ValueError(f"max_rounds must be a non-negative integer, got {max_rounds!r}")
+        check_clash_args(threshold, grow, plan.K)
+        shape = (fs.NB, fs.L, 3)
+        latent = out["latent"]
+        if not torch.is_tensor(latent) or latent.dtype != torch.float32 or tuple(latent.shape) != shape or latent.device != plan.device:
+            raise ValueError(f"out['latent'] must be a float32 tensor of shape {shape} on {plan.device}")
+        counts, keep = self.residue_clashes(plan, fs, out["xyz"], threshold, grow)
+        pairs = clash_pair_totals(counts)
+        rows = [pairs]
+        latent = latent.clone()                  # resample() writes the plan's latent buffer, which out["latent"] may be
+        for _ in range(max_rounds):
+            if not bool((pairs > 0).any()):
+                break
+            new = self.resample(plan, fs, latent, keep, generator=generator)
+            new_counts, new_keep = self.residue_clashes(plan, fs, new["xyz"], threshold, grow)
+            new_pairs = clash_pair_totals(new_counts)
+            acc = repair_accept(pairs, new_pairs)
+            latent = torch.where(acc[:, None, None], new["latent"], latent)
+            keep = torch.where(acc[:, None], new_keep, keep)
+            pairs = torch.where(acc, new_pairs, pairs)
+            rows.append(pairs)
+        plan.clear_inpaint()
+        if len(rows) == 1:                       # nothing resampled: the input as it is
+            res = dict(out)
+        else:
+            idx, zq, ic, xyz = plan.decode(self.vae, latent, denorm=True, num_atoms_total=fs.total_atoms)
+            res = {"latent": latent, "idx": idx, "zq": zq, "ic_recon": ic, "xyz": xyz}
+            counts, _ = self.residue_clashes(plan, fs, xyz, threshold, grow)
+        res["clashes"] = counts
+        res["clash_pairs"] = torch.stack(rows, 0)
+        return res
 
     def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator):
         dev = plan.device

@@ -24,7 +24,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 3
+#define CB2_ABI_VERSION 4
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -129,6 +129,19 @@ CB2_API int cb2_plan_set_topology(cb2_plan* p, const cb2_vae* v, const float* ca
  * padded positions), zq [NB,L,3], ic_recon [NB,L,13,3], xyz [sum Na,3]. */
 CB2_API int cb2_plan_decode(cb2_plan* p, const cb2_vae* v, const float* latent, int denorm, int* idx, float* zq,
                     float* ic_recon, float* xyz, void* stream);
+
+/* Not in the reference: per-residue form of clash_result's criterion (test.py:118-139) on a decoded sample, with no reference
+ * structure and no dataset pair lists.  xyz [sum Na,3] is laid out as cb2_plan_decode writes it (slot_atom / out_offset of
+ * cb2_plan_set_topology, which must have been called).  counts [NB*L] int32: counts[b*L+i] = number of atom pairs (a in residue
+ * i, c in another residue j of member b) with d(a, c) < threshold, where d = sqrt(|a - c|^2 + 1e-7) in fp32 exactly as
+ * cb2_pair_losses forms it, leaving out the peptide pair C(i)-N(i+1) (slots 2 and 1); a pair counts once for each of its two
+ * residues; padded rows get 0.  Every pair is tested (bounding-sphere pruning that never drops one), so the counts equal a
+ * brute-force pass.  keep [NB*L] u8 or NULL: 0 where residue i or one of its `grow` nearest other residues (the plan's k-NN
+ * rows, distance order) has a clash, 1 elsewhere and on padded rows -- the keep mask of cb2_plan_set_inpaint that resamples the
+ * clashing residues.  threshold must be finite and positive (the reference uses 1.2 A), 0 <= grow < K (grow = 0 on a decode-only
+ * plan).  Deterministic; two launches, three with keep. */
+CB2_API int cb2_plan_residue_clashes(cb2_plan* p, const float* xyz, float threshold, int grow, int* counts, unsigned char* keep,
+                             void* stream);
 
 /* Debug / parity access to plan-owned buffers: "nbr_idx" "nbr_dist" "E" "hE0" "hE" "hV" "S" "out6" "mod".
  * Copies the first dst_bytes of the buffer into the caller's device memory (error if it is smaller). */
