@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CB2_LIB") or os.path.join(_HERE, "libcodlad_b200.so")      # CB2_LIB: experiment builds
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 PRECISION = {"fp32": 0, "f32": 0, "f16": 1, "fp16": 1}
 
@@ -41,6 +41,7 @@ SIGNATURES = {
     "cb2_plan_set_ddim_schedule": (_I, [_P, _P, _P, _I, _P]),
     "cb2_plan_sample": (_I, [_P, _P, _P, _I, _P]),
     "cb2_plan_set_inpaint": (_I, [_P, _P, _P, _P, _I, _P]),
+    "cb2_plan_set_start": (_I, [_P, _I, _P]),
     "cb2_plan_set_topology": (_I, [_P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
     "cb2_plan_decode": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "cb2_plan_residue_clashes": (_I, [_P, _P, C.c_float, _I, _P, _P, _P]),

@@ -619,16 +619,26 @@ int cb2_plan_set_inpaint(cb2_plan* h, const unsigned char* keep, const float* x0
     return 0;
 }
 
+int cb2_plan_set_start(cb2_plan* h, int steps, void* stream) {
+    (void)stream;       // host-side state only
+    if (!h || !h->p.model) { set_error("set_start: bad argument"); return 1; }
+    if (steps < 0) { set_error("set_start: steps must be >= 0, got %d", steps); return 1; }
+    h->p.start_steps = steps;
+    return 0;
+}
+
 static int enqueue_loop(cb2_plan* h, float* x, const float* noise, cudaStream_t s) {
     Plan& p = h->p;
     const size_t n3 = (size_t)p.NB * p.L * 3;
     CB2_CUDA(cudaMemcpyAsync(h->xa, x, n3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    const bool refine = p.start_steps > 0;
+    const int steps = refine ? p.start_steps : p.coef_steps;
     if (p.inpaint) {
-        if (int e = launch_inpaint_init(p.inp_keep, p.inp_x0, p.inp_coef + (size_t)p.coef_steps * 2, p.NB * p.L, h->xa, p.inp_eps, s)) return e;
+        if (int e = launch_inpaint_init(p.inp_keep, p.inp_x0, p.inp_coef + (size_t)steps * 2, p.NB * p.L, refine, h->xa, p.inp_eps, s)) return e;
         p.launches++;
     }
     float *cur = h->xa, *nxt = h->xb;
-    for (int step = p.coef_steps - 1; step >= 0; --step) {
+    for (int step = steps - 1; step >= 0; --step) {
         const float* mod_row = p.mod + (size_t)step * CB2_MOD_TOTAL;     // every member shares the step -> stride 0
         const float* step_noise = noise != nullptr ? noise + (size_t)step * n3 : nullptr;
         const float* inpaint_row = p.inpaint ? p.inp_coef + (size_t)step * 2 : nullptr;
@@ -660,11 +670,19 @@ int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, vo
         set_error("sample: the inpainting table has T=%d, the schedule T=%d", p.inpaint_steps, p.coef_steps);
         return 1;
     }
+    if (p.start_steps > p.coef_steps) {
+        set_error("sample: the start (%d steps) exceeds the schedule's T=%d", p.start_steps, p.coef_steps);
+        return 1;
+    }
+    if (p.start_steps > 0 && !p.inpaint) {
+        set_error("sample: a start of %d steps refines the inpainting latent x0: cb2_plan_set_inpaint must be called first", p.start_steps);
+        return 1;
+    }
     cudaStream_t s = (cudaStream_t)stream;
     if (!use_graph) return enqueue_loop(h, x, noise, s);
     // (kernel variants are chosen at capture time from the geometry: a frame set with / without padded residues needs its own graph)
     if (!p.graph || p.graph_key[0] != x || p.graph_key[1] != noise || p.graph_steps != p.coef_steps || p.graph_all_full != p.all_full ||
-        p.graph_inpaint != p.inpaint) {
+        p.graph_inpaint != p.inpaint || p.graph_start != p.start_steps) {
         if (p.graph) { cudaGraphExecDestroy(p.graph); p.graph = nullptr; }
         cudaStream_t cs;
         CB2_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
@@ -685,10 +703,10 @@ int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, vo
         cudaStreamDestroy(cs);
         if (ce != cudaSuccess) { set_error("graph instantiate failed: %s", cudaGetErrorString(ce)); p.graph = nullptr; return (int)ce; }
         p.graph_key[0] = x; p.graph_key[1] = noise; p.graph_steps = p.coef_steps; p.graph_all_full = p.all_full;
-        p.graph_inpaint = p.inpaint;
+        p.graph_inpaint = p.inpaint; p.graph_start = p.start_steps;
     }
     CB2_CUDA(cudaGraphLaunch(p.graph, s));
-    p.launches += 16LL * p.coef_steps + (p.inpaint ? 1 : 0);
+    p.launches += 16LL * (p.start_steps > 0 ? p.start_steps : p.coef_steps) + (p.inpaint ? 1 : 0);
     return 0;
 }
 

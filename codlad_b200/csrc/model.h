@@ -97,9 +97,11 @@ struct Plan {
     float* inp_eps = nullptr;       // [NB*L, 3] the fixed draw of the kept rows (saved from the initial noise)
     float* inp_coef = nullptr;      // [mod_capacity + 1, 2] rows s: {sqrt(acp_prev[s]), sqrt(1 - acp_prev[s])}, row T: head
     std::vector<float> inp_coef_host;    // what inp_coef holds (re-uploaded only when it changes)
+    int start_steps = 0;            // cb2_plan_set_start: > 0 = partial-noise refinement over steps start_steps-1 .. 0
     cudaGraphExec_t graph = nullptr;
     const void* graph_key[4] = {nullptr, nullptr, nullptr, nullptr};
     int graph_steps = 0;
+    int graph_start = 0;            // start_steps of the captured loop
     bool graph_all_full = false;    // the captured launches chose the masked / unmasked message kernels from all_full
     bool graph_inpaint = false;     // the captured loop applies the inpainting overwrite
     std::vector<void*> allocs;
@@ -118,8 +120,10 @@ int launch_p_sample(const float* x, const float* out6, const float* noise, const
                     int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
 int launch_ddim_sample(const float* x, const float* out6, const float* noise, const float* coef_rows, const int* step_of_row,
                        int rows_per_b, int n_rows, int C, float* x_next, cudaStream_t s);
-// in place on the loop's initial latent x: eps = x and x = q_head[0] x0 + q_head[1] eps on the kept rows
-int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, float* x, float* eps, cudaStream_t s);
+// in place on the loop's initial latent x: eps = x on the kept rows, and x = q_head[0] x0 + q_head[1] x on the kept rows, or on
+// every row when all_rows (partial-noise refinement)
+int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, bool all_rows, float* x, float* eps,
+                        cudaStream_t s);
 float* plan_P(Plan& p, int which);
 
 // The fused update's kept-row overwrite reads the plan's inpainting buffers with `inpaint_row` = the step's

@@ -15,7 +15,8 @@
 //    DDIM schedule, IDDPM's ddim_sample update (ddim_update, common.cuh).  With latent inpainting on,
 //    the kept rows are then overwritten with the forward marginal of their latent (inpaint_level).
 //  * inpaint_init:  before the first step, saves the kept rows' initial noise as their fixed draw and
-//    puts them at the head level of the schedule.
+//    puts them at the head level of the schedule; for partial-noise refinement (all_rows) every row
+//    starts at the level of its own x0 there.
 //
 // fp32 SIMT: 16 rows per CTA, 128 threads, thread = output column (see tile_gemm.cuh).
 #include "model.h"
@@ -348,12 +349,15 @@ __global__ void ddim_sample_kernel(const float* __restrict__ x, const float* __r
     x_next[t] = ddim_update(x[t], out6[(size_t)row * 2 * C + d], cf, noise != nullptr ? noise + t : nullptr);
 }
 
+// all_rows is uniform per launch; eps is saved for kept rows only, as the overwrite reads it for them alone.
 __global__ void inpaint_init_kernel(const unsigned char* __restrict__ keep, const float* __restrict__ x0, const float* __restrict__ q_head,
-                                    int n_rows, float* __restrict__ x, float* __restrict__ eps) {
+                                    int n_rows, int all_rows, float* __restrict__ x, float* __restrict__ eps) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_rows * 3 || !keep[t / 3]) return;
+    if (t >= n_rows * 3) return;
+    const bool kept = keep[t / 3] != 0;
+    if (!kept && !all_rows) return;
     const float e = x[t];
-    eps[t] = e;
+    if (kept) eps[t] = e;
     x[t] = inpaint_level(q_head, x0[t], e);
 }
 
@@ -387,9 +391,10 @@ int launch_ddim_sample(const float* x, const float* out6, const float* noise, co
     return 0;
 }
 
-int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, float* x, float* eps, cudaStream_t s) {
+int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, bool all_rows, float* x, float* eps,
+                        cudaStream_t s) {
     const int total = n_rows * 3;
-    inpaint_init_kernel<<<(total + 255) / 256, 256, 0, s>>>(keep, x0, q_head, n_rows, x, eps);
+    inpaint_init_kernel<<<(total + 255) / 256, 256, 0, s>>>(keep, x0, q_head, n_rows, all_rows ? 1 : 0, x, eps);
     CB2_LAUNCH_CHECK();
     return 0;
 }

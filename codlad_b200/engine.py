@@ -32,6 +32,12 @@ def check_clash_args(threshold, grow, K: int):
         raise ValueError(f"grow must be an integer in [0, {K}), got {grow!r}")
 
 
+def check_start_steps(steps):
+    """Argument of Plan.set_start: a non-negative integer (0 = the whole schedule).  Raises ValueError; touches no device."""
+    if isinstance(steps, bool) or not isinstance(steps, numbers.Integral) or steps < 0:
+        raise ValueError(f"steps must be a non-negative integer, got {steps!r}")
+
+
 class DenoiserEngine:
     """Packed device copy of an `mpnn_diffusion` state_dict (models/latent_model.py:78-165)."""
 
@@ -190,6 +196,14 @@ class Plan:
             raise ValueError("q_coef must be a [T+1, 2] table (SpacedDiffusion.inpaint_coef_table)")
         N.check(N.lib().cb2_plan_set_inpaint(self.handle, N.dptr(keep.to(torch.uint8).contiguous()), N.dptr(x0.contiguous()),
                                              q.data_ptr(), int(q.shape[0]) - 1, N.stream_ptr()), "set_inpaint")
+
+    def set_start(self, steps: int):
+        """Partial-noise refinement for the following sample() calls (cb2_plan_set_start): steps = 0 runs the whole schedule;
+        1 <= steps <= T runs only respaced steps steps-1 .. 0 and refines the inpainting latent x0 of set_inpaint, which must be
+        on.  Every row then starts at the forward marginal of its x0 at that level, with the x passed to sample() as the noise;
+        kept rows still end at x0.  noise slices [0, steps) are read.  sample() refuses steps > T or steps without inpainting."""
+        check_start_steps(steps)
+        N.check(N.lib().cb2_plan_set_start(self.handle, int(steps), N.stream_ptr()), "set_start")
 
     def clear_inpaint(self):
         """Turn latent inpainting off: sample() regenerates every row again."""

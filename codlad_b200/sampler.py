@@ -12,13 +12,15 @@ Host work here is input-format conversion only (padding, CSR of the given CG_nbr
 """
 from __future__ import annotations
 
+import math
+import numbers
 from dataclasses import dataclass, field
 
 import torch
 
-from . import batching, distributed, topology, weights
+from . import batching, distributed, metrics, topology, weights
 from .diffusion import create_diffusion
-from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args
+from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args, check_start_steps
 
 VAE_DATA = {"N6": "PED", "K3": "PDB", "K4": "Atlas"}
 
@@ -31,6 +33,37 @@ def clash_pair_totals(counts: torch.Tensor) -> torch.Tensor:
 def repair_accept(prev_pairs: torch.Tensor, new_pairs: torch.Tensor) -> torch.Tensor:
     """The acceptance rule of Backmapper.repair, per member: take the resampled latent only if it has fewer clashing pairs."""
     return new_pairs < prev_pairs
+
+
+def trajectory_chunks(n_frames: int, chunks: int):
+    """Split n_frames consecutive frames into `chunks` contiguous runs whose lengths differ by at most one, longer runs first.
+    Returns [(first frame, length)]."""
+    if isinstance(chunks, bool) or not isinstance(chunks, numbers.Integral) or chunks < 1:
+        raise ValueError(f"chunks must be a positive integer, got {chunks!r}")
+    if chunks > n_frames:
+        raise ValueError(f"chunks ({chunks}) exceeds the number of frames ({n_frames})")
+    q, r = divmod(int(n_frames), int(chunks))
+    runs, start = [], 0
+    for c in range(chunks):
+        n = q + (1 if c < r else 0)
+        runs.append((start, n))
+        start += n
+    return runs
+
+
+def residue_atom_ranges(fs: "FrameSet"):
+    """The atoms of every real residue of every member of `fs`, gathered through slot_atom into contiguous ranges.  Returns
+    (atoms int64 [A], counts int64 [R], rows int64 [R]): residue r = row rows[r] of the flattened [NB, L] grid owns
+    atoms[sum(counts[:r]) : sum(counts[:r + 1])], rows of the output xyz laid out as decode writes it, in slot order.  Padded rows
+    and residues without atoms are left out, so no range is empty."""
+    fo = fs.frame_of.long().cpu()
+    slots = fs.slot_atom.cpu().view(fs.F, fs.L, topology.SLOTS_PER_RESIDUE)[fo]                  # [NB, L, 14]
+    valid = torch.arange(fs.L)[None] < fs.lengths.cpu().long()[fo][:, None]                      # [NB, L]
+    present = (slots >= 0) & valid[..., None]
+    counts = present.sum(-1).flatten()
+    rows = torch.nonzero(counts > 0).squeeze(1)
+    atoms = (slots.long() + fs.out_off.cpu().long()[:, None, None])[present]      # row-major: each residue's atoms in one run
+    return atoms, counts[rows], rows
 
 
 @dataclass
@@ -177,6 +210,7 @@ class Backmapper:
         z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted.  DDIM with eta = 0 uses no
         step noise: `step_noise` is ignored.  Every residue is sampled anew, also after resample() on the same plan."""
         plan.clear_inpaint()
+        plan.set_start(0)
         return self._sample(plan, fs, z, step_noise, use_graph, generator)
 
     def resample(self, plan: Plan, fs: FrameSet, latent: torch.Tensor, keep: torch.Tensor, z: torch.Tensor = None,
@@ -186,6 +220,31 @@ class Backmapper:
         (`sample(...)["latent"]`, which may be passed as is).  Kept rows follow the forward marginal of their latent with the
         fixed draw z and end at it exactly, so they keep their VQ index.  z and step_noise as in sample().  Returns the same
         dict as sample()."""
+        self._check_latent_keep(plan, fs, latent, keep)
+        plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())      # copies latent before z overwrites its buffer
+        plan.set_start(0)
+        return self._sample(plan, fs, z, step_noise, True, generator)
+
+    def refine(self, plan: Plan, fs: FrameSet, latent: torch.Tensor, steps: int, keep: torch.Tensor = None, z: torch.Tensor = None,
+               step_noise: torch.Tensor = None, generator: torch.Generator = None):
+        """Partial-noise refinement (SDEdit): noise the normalised latent [NB,L,3] to the level of respaced step `steps` with the
+        draw z, x = sqrt(acp[steps-1]) latent + sqrt(1 - acp[steps-1]) z, and run only the last `steps` of the T steps,
+        conditioned on the frames of `fs` as uploaded now.  The strength is steps / T, with 1 <= steps <= T.  latent may be
+        `sample(...)["latent"]` as it is.  keep [NB,L] (bool) keeps those residues exactly, as resample() does; None refines every
+        residue.  z [NB,L,3] and step_noise [T,NB,L,3] (slices [0, steps) are read) are drawn when omitted; DDIM with eta = 0 uses
+        no step noise.  Returns the same dict as sample(); a later sample() or resample() is a full pass again."""
+        check_start_steps(steps)
+        if not 1 <= steps <= self.T:
+            raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
+        if keep is None:
+            keep = torch.zeros(fs.NB, fs.L, dtype=torch.bool, device=plan.device)
+        self._check_latent_keep(plan, fs, latent, keep)
+        plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())
+        plan.set_start(steps)
+        return self._sample(plan, fs, z, step_noise, True, generator, steps)
+
+    @staticmethod
+    def _check_latent_keep(plan: Plan, fs: FrameSet, latent, keep):
         shape = (fs.NB, fs.L, 3)
         if not torch.is_tensor(latent) or latent.dtype != torch.float32 or tuple(latent.shape) != shape:
             raise ValueError(f"latent must be a float32 tensor of shape {shape}")
@@ -193,8 +252,6 @@ class Backmapper:
             raise ValueError(f"keep must be a bool tensor of shape {shape[:2]}")
         if latent.device != plan.device or keep.device != plan.device:
             raise ValueError(f"latent and keep must be on {plan.device}")
-        plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())      # copies latent before z overwrites its buffer
-        return self._sample(plan, fs, z, step_noise, True, generator)
 
     def residue_clashes(self, plan: Plan, fs: FrameSet, xyz: torch.Tensor, threshold: float = 1.2, grow: int = 0):
         """Per-residue clashes of a decoded sample, on the device (cb2_plan_residue_clashes): clash_result's criterion
@@ -254,7 +311,61 @@ class Backmapper:
         res["clash_pairs"] = torch.stack(rows, 0)
         return res
 
-    def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator):
+    def residue_motion(self, fs: FrameSet, xyz_a: torch.Tensor, xyz_b: torch.Tensor) -> torch.Tensor:
+        """Per-residue RMSD between two decoded structures of the same frame set (xyz [fs.total_atoms, 3] CUDA float32, as
+        sample() returns them), each residue's atoms superposed on their own (cb2_superposed_rmsd over the residue_atom_ranges).
+        Returns float64 [NB, L] on the device, NaN on padded rows.  Between consecutive frames of a trajectory it measures
+        side-chain flicker; between a sample and its refine() or repair() it shows what the pass changed."""
+        shape = (fs.total_atoms, 3)
+        for name, t in (("xyz_a", xyz_a), ("xyz_b", xyz_b)):
+            if not torch.is_tensor(t) or t.dtype != torch.float32 or tuple(t.shape) != shape or not t.is_cuda:
+                raise ValueError(f"{name} must be a CUDA float32 tensor of shape {shape}")
+        if xyz_a.device != xyz_b.device:
+            raise ValueError("xyz_a and xyz_b must be on the same device")
+        atoms, counts, rows = residue_atom_ranges(fs)
+        out = torch.full((fs.NB * fs.L,), math.nan, dtype=torch.float64, device=xyz_a.device)
+        if rows.numel():
+            atoms = atoms.to(xyz_a.device)
+            out[rows.to(xyz_a.device)] = metrics.superposed_rmsd(xyz_a[atoms], xyz_b[atoms], counts)
+        return out.view(fs.NB, fs.L)
+
+    def backmap_trajectory(self, batches, info, num_ensemble: int = 1, steps: int = None, chunks: int = 1,
+                           generator: torch.Generator = None) -> torch.Tensor:
+        """Backmap consecutive frames of one protein with warm starts.  batches: one reference-schema batch dict per frame (one
+        frame each, all of the same length), info: the shared topology tuple.  The frames are split into `chunks` contiguous runs
+        (trajectory_chunks) that go through one plan together, each run with `num_ensemble` members.  The first frame of every run
+        is sampled from noise (sample()); every later frame refines each member's latent of the previous frame (refine(), `steps`
+        of the T steps, default T // 4), so members stay coherent along a run and cost steps / T of the loop per frame.  More chunks
+        put more frames into one pass and break coherence chunks - 1 times.  A run that has ended repeats its last frame, and that
+        result is dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        batches = list(batches)
+        if isinstance(num_ensemble, bool) or not isinstance(num_ensemble, numbers.Integral) or num_ensemble < 1:
+            raise ValueError(f"num_ensemble must be a positive integer, got {num_ensemble!r}")
+        steps = max(1, self.T // 4) if steps is None else steps
+        check_start_steps(steps)
+        if not 1 <= steps <= self.T:
+            raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
+        runs = trajectory_chunks(len(batches), chunks)
+        if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
+            raise ValueError("backmap_trajectory: every batch must hold one frame, all of the same length")
+        out = None
+        res = None
+        for p in range(runs[0][1]):                  # runs[0] is the longest
+            frames = [start + min(p, n - 1) for start, n in runs]
+            fs = frames_from_batch(batching.merge_batches([batches[f] for f in frames]), info, num_ensemble)
+            plan = self.upload(fs)
+            if p == 0:
+                res = self.sample(plan, fs, generator=generator)
+                Na = int(fs.num_atoms[0])
+                out = torch.empty(len(batches), num_ensemble, Na, 3, dtype=torch.float32, device=plan.device)
+            else:
+                res = self.refine(plan, fs, res["latent"], steps, generator=generator)
+            live = [c for c, (_, n) in enumerate(runs) if p < n]
+            xyz = res["xyz"].view(num_ensemble, len(runs), Na, 3)                 # members are ensemble-major: b = e * chunks + c
+            out[[runs[c][0] + p for c in live]] = xyz[:, live].transpose(0, 1)
+        return out.cpu()
+
+    def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator, steps: int = None):
         dev = plan.device
         shape = (fs.NB, fs.L, 3)
         noisy = self.sampler == "ddpm" or self.eta != 0
@@ -271,7 +382,8 @@ class Backmapper:
             if step_noise is not None:
                 noise.copy_(step_noise, non_blocking=True)
             else:
-                torch.randn(self.T, *shape, device=dev, generator=generator, out=noise)
+                n = self.T if steps is None else steps                 # the loop reads slices [0, steps) only
+                torch.randn(n, *shape, device=dev, generator=generator, out=noise[:n])
         plan.sample(x, noise, use_graph)
         idx, zq, ic, xyz = plan.decode(self.vae, x, denorm=True, num_atoms_total=fs.total_atoms)
         return {"latent": x, "idx": idx, "zq": zq, "ic_recon": ic, "xyz": xyz}

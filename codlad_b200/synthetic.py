@@ -75,6 +75,16 @@ def make_protein(L: int, num_frames: int, seed: int, compact: float = 0.0) -> Sy
     return SyntheticProtein(restype, X, topology.build_info(restype[1:-1]))
 
 
+def trajectory(L: int, num_frames: int, seed: int, step: float = 0.05, compact: float = 0.0) -> SyntheticProtein:
+    """One protein whose C-alpha trace moves from frame to frame by a Gaussian step of RMS length `step` Angstrom per residue
+    (a random walk from make_protein's first frame), like consecutive frames of an MD trajectory."""
+    prot = make_protein(L, 1, seed, compact)
+    g = torch.Generator().manual_seed(seed + 104729)
+    moves = torch.randn(num_frames - 1, L + 2, 3, generator=g) * (step / 3 ** 0.5)
+    ca = prot.ca_full[0] + torch.cat([torch.zeros(1, L + 2, 3), torch.cumsum(moves, 0)])
+    return SyntheticProtein(prot.restype_full, ca, prot.info)
+
+
 def collate(protein: SyntheticProtein, frames=None, prot_idx: int = 0) -> dict:
     """Batch dict for `frames` of one protein, exactly the keys/shapes the reference hot path
     indexes (models/latent_model.py:168-173, models/vae_model.py:708-726, test.py:567-569)."""

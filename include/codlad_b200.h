@@ -24,7 +24,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 4
+#define CB2_ABI_VERSION 5
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -113,6 +113,15 @@ CB2_API int cb2_plan_sample(cb2_plan* p, float* x, const float* noise, int use_g
  * inpainting off (x0 and q_coef are then ignored).  Each sample call with inpainting on launches one more kernel. */
 CB2_API int cb2_plan_set_inpaint(cb2_plan* p, const unsigned char* keep, const float* x0, const float* q_coef, int T,
                          void* stream);
+
+/* Partial-noise refinement (SDEdit; the reference has none) for the following cb2_plan_sample calls.  steps = 0 (the default) runs
+ * the whole schedule.  1 <= steps <= T runs only respaced steps steps-1 .. 0 of the loaded schedule (DDPM or DDIM), with the adaLN
+ * and coefficient rows a full pass uses for them, and refines the inpainting latent x0 of cb2_plan_set_inpaint, which must be on (an
+ * all-zero keep mask refines every row).  Before the first step EVERY row is set to q_coef[steps] applied to (x0, eps = that row of
+ * the initial x), so the initial x is the noise of the intermediate level; kept rows then follow x0 as without a start and still end
+ * at it exactly.  noise is read for slices [0, steps) only.  cb2_plan_sample refuses steps > T and steps > 0 without inpainting;
+ * a pass launches 16 * steps + 1 kernels.  steps < 0 is refused.  Host-side state only: no work is enqueued on `stream`. */
+CB2_API int cb2_plan_set_start(cb2_plan* p, int steps, void* stream);
 
 /* Decode-side geometry.  ca_full [F,L+2,3] device (untrimmed trace); HOST OR DEVICE (copied with
  * cudaMemcpyDefault): csr_row_ptr [F*L+1] / csr_col [E]
