@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CB2_LIB") or os.path.join(_HERE, "libcodlad_b200.so")      # CB2_LIB: experiment builds
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 PRECISION = {"fp32": 0, "f32": 0, "f16": 1, "fp16": 1}
 
@@ -43,12 +43,15 @@ SIGNATURES = {
     "cb2_plan_set_inpaint": (_I, [_P, _P, _P, _P, _I, _P]),
     "cb2_plan_set_start": (_I, [_P, _I, _P]),
     "cb2_plan_set_topology": (_I, [_P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
+    "cb2_plan_set_coords": (_I, [_P, _P, _P, _P]),
     "cb2_plan_decode": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "cb2_plan_residue_clashes": (_I, [_P, _P, C.c_float, _I, _P, _P, _P]),
     "cb2_plan_buffer": (_I, [_P, C.c_char_p, _P, _LL, _P]),
     "cb2_plan_run_edge_kernel": (_I, [_P, _I, _I, _P]),
     "cb2_plan_run_stage": (_I, [_P, _P, _I, _I, _P, _P]),
     "cb2_knn_topk": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
+    "cb2_radius_graph_rows": (_I, [_P, _P, _I, _I, C.c_float, _P, _P]),
+    "cb2_radius_graph_fill": (_I, [_P, _P, _I, _I, C.c_float, _P, _P, _P]),
     "cb2_vq_lookup": (_I, [_P, _P, _I, _I, _P, _P, _I, _P, _P, _P]),
     "cb2_p_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
     "cb2_ddim_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),

@@ -3,6 +3,7 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <algorithm>
 #include <map>
 #include <string>
 #include <vector>
@@ -102,7 +103,8 @@ struct cb2_plan {
     // decode-side buffers
     float* ca_full = nullptr;
     int *csr_row = nullptr, *csr_col = nullptr;
-    int E = 0;
+    int E = 0;              // edges of the current radius graph
+    int E_cap = 0;          // edges csr_col / edge_w hold; both are owned here (not in p.allocs) and replaced when they grow
     signed char* orders = nullptr;
     int* slot_atom = nullptr;
     long long* out_off = nullptr;
@@ -463,6 +465,8 @@ void cb2_plan_destroy(cb2_plan* h) {
     edge_tc_release(h->p);
     node_tc_release(h->p);
     for (void* q : h->p.allocs) cudaFree(q);
+    cudaFree(h->csr_col);
+    cudaFree(h->edge_w);
     delete h;
 }
 
@@ -710,6 +714,26 @@ int cb2_plan_sample(cb2_plan* h, float* x, const float* noise, int use_graph, vo
     return 0;
 }
 
+// Room for n_edges in csr_col / edge_w.  They grow geometrically and the replaced buffers are freed, so a long run of updates whose
+// edge count fluctuates holds at most about 1.5x its largest graph.  Only the eagerly launched decode and the IC filters read these
+// buffers (the captured step loop does not), so replacing them needs no graph recapture; the stream is synchronised first because
+// earlier decode launches may still be reading the old ones.
+static int reserve_edges(cb2_plan* h, int n_edges, cudaStream_t s) {
+    if (h->csr_col && n_edges <= h->E_cap) return 0;
+    const long long want = h->csr_col ? std::max<long long>(n_edges, (long long)h->E_cap + h->E_cap / 2) : n_edges;
+    const int cap = (int)std::min<long long>(want, 0x7fffffff);
+    if (h->csr_col) {
+        CB2_CUDA(cudaStreamSynchronize(s));
+        cudaFree(h->csr_col); cudaFree(h->edge_w);
+        h->csr_col = nullptr; h->edge_w = nullptr; h->E_cap = 0;
+    }
+    const size_t n = cap > 0 ? (size_t)cap : 1;
+    CB2_CUDA(cudaMalloc(&h->csr_col, n * sizeof(int)));
+    CB2_CUDA(cudaMalloc(&h->edge_w, n * 4 * 40 * sizeof(float)));
+    h->E_cap = cap;
+    return 0;
+}
+
 int cb2_plan_set_topology(cb2_plan* h, const cb2_vae* v, const float* ca_full, const int* csr_row_ptr, const int* csr_col,
                           int n_edges, const signed char* atom_orders, const int* slot_atom, const long long* out_offset,
                           void* stream) {
@@ -731,11 +755,7 @@ int cb2_plan_set_topology(cb2_plan* h, const cb2_vae* v, const float* ca_full, c
         e |= dev_alloc(p.allocs, &h->vq_idx, N);
         if (e) return e;
     }
-    if (n_edges > h->E || !h->csr_col) {
-        int e = dev_alloc(p.allocs, &h->csr_col, (size_t)n_edges);
-        e |= dev_alloc(p.allocs, &h->edge_w, (size_t)4 * n_edges * 40);
-        if (e) return e;
-    }
+    if (int e = reserve_edges(h, n_edges, s)) { h->topo_ready = false; return e; }     // no graph buffers: decode refuses
     h->E = n_edges;
     CB2_CUDA(cudaMemcpyAsync(h->ca_full, ca_full, (size_t)p.F * (p.L + 2) * 3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
     CB2_CUDA(cudaMemcpyAsync(h->csr_row, csr_row_ptr, (FL + 1) * sizeof(int), cudaMemcpyDefault, s));
@@ -748,6 +768,33 @@ int cb2_plan_set_topology(cb2_plan* h, const cb2_vae* v, const float* ca_full, c
     p.launches += 1;
     CB2_CUDA(cudaStreamSynchronize(s));
     h->topo_ready = true;
+    return 0;
+}
+
+int cb2_plan_set_coords(cb2_plan* h, const cb2_vae* v, const float* ca_full, void* stream) {
+    if (!h || !v || !ca_full) { set_error("set_coords: null argument"); return 1; }
+    if (!h->topo_ready) { set_error("set_coords: cb2_plan_set_topology has not been called (set_coords keeps its lengths, types and topology)"); return 1; }
+    Plan& p = h->p;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int FL = p.F * p.L;
+    CB2_CUDA(cudaMemcpyAsync(h->ca_full, ca_full, (size_t)p.F * (p.L + 2) * 3 * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (int e = launch_trim_coords(h->ca_full, p.lengths, p.F, p.L, p.X, s)) return e;
+    p.launches += 1;
+    if (p.model) {
+        if (int e = launch_knn(p.X, p.lengths, p.F, p.L, p.K, p.nbr_dist, p.nbr_idx, s)) return e;
+        if (int e = launch_edge_features(*p.model, p.X, p.lengths, p.nbr_idx, p.nbr_dist, p.F, p.L, p.K, p.E_dbg, p.hE0, p.precision, s)) return e;
+        p.launches += 2;
+    }
+    if (int e = launch_radius_rows(p.X, p.lengths, p.F, p.L, v->v.cutoff, h->csr_row, s)) return e;
+    p.launches += 2;
+    int n_edges = 0;
+    CB2_CUDA(cudaMemcpyAsync(&n_edges, h->csr_row + FL, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CB2_CUDA(cudaStreamSynchronize(s));     // the edge count sizes csr_col / edge_w and the filter launch
+    if (int e = reserve_edges(h, n_edges, s)) { h->topo_ready = false; return e; }     // no graph buffers: decode refuses
+    h->E = n_edges;
+    if (int e = launch_radius_fill(p.X, p.lengths, p.F, p.L, v->v.cutoff, h->csr_row, h->csr_col, s)) return e;
+    if (int e = launch_ic_edge_filters(v->v, p.X, p.F, p.L, h->csr_row, h->csr_col, n_edges, h->edge_w, s)) return e;
+    p.launches += 2;
     return 0;
 }
 
@@ -856,6 +903,16 @@ int cb2_plan_run_stage(cb2_plan* h, const cb2_vae* v, int stage, int layer, floa
 int cb2_knn_topk(const float* X, const int* lengths, int F, int L, int K, float* D, int* idx, void* stream) {
     if (!X || !D || !idx) { set_error("knn_topk: null argument"); return 1; }
     return launch_knn(X, lengths, F, L, K, D, idx, (cudaStream_t)stream);
+}
+
+int cb2_radius_graph_rows(const float* X, const int* lengths, int F, int L, float cutoff, int* row_ptr, void* stream) {
+    if (!X || !lengths || !row_ptr) { set_error("radius_graph_rows: null argument"); return 1; }
+    return launch_radius_rows(X, lengths, F, L, cutoff, row_ptr, (cudaStream_t)stream);
+}
+
+int cb2_radius_graph_fill(const float* X, const int* lengths, int F, int L, float cutoff, const int* row_ptr, int* col, void* stream) {
+    if (!X || !lengths || !row_ptr || !col) { set_error("radius_graph_fill: null argument"); return 1; }
+    return launch_radius_fill(X, lengths, F, L, cutoff, row_ptr, col, (cudaStream_t)stream);
 }
 
 int cb2_vq_lookup(const cb2_vae* v, const float* x, int NB, int L, const int* lengths, const int* frame_of, int denorm,

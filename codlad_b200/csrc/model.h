@@ -125,6 +125,11 @@ int launch_ddim_sample(const float* x, const float* out6, const float* noise, co
 int launch_inpaint_init(const unsigned char* keep, const float* x0, const float* q_head, int n_rows, bool all_rows, float* x, float* eps,
                         cudaStream_t s);
 float* plan_P(Plan& p, int which);
+// radius.cu: directed radius graph over the F*L padded rows (rows: counts + scan into row_ptr[F*L+1]; fill: the columns), and
+// X [F,L,3] from the untrimmed trace ca_full [F,L+2,3]
+int launch_radius_rows(const float* X, const int* lengths, int F, int L, float cutoff, int* row_ptr, cudaStream_t s);
+int launch_radius_fill(const float* X, const int* lengths, int F, int L, float cutoff, const int* row_ptr, int* col, cudaStream_t s);
+int launch_trim_coords(const float* ca_full, const int* lengths, int F, int L, float* X, cudaStream_t s);
 
 // The fused update's kept-row overwrite reads the plan's inpainting buffers with `inpaint_row` = the step's
 // {sqrt(acp_prev), sqrt(1 - acp_prev)}; nullptr = no inpainting.

@@ -141,6 +141,18 @@ class Plan:
                                               int(csr_col.numel()), orders.data_ptr(), slot_atom.data_ptr(), out_off.data_ptr(),
                                               N.stream_ptr()), "set_topology")
 
+    def set_coords(self, vae: VaeEngine, ca_full):
+        """Move the frames already on the plan to new coordinates, all on the device (cb2_plan_set_coords): ca_full [F, L+2, 3] CUDA
+        float32 on the plan's device, the untrimmed traces.  X, the k-NN graph, edge features and h_E0, the radius graph at the VAE's
+        cutoff and the IC filters are recomputed from it; lengths, residue types, members and topology stay.  Needs set_topology.
+        The step loop's captured graph stays valid."""
+        shape = (self.F, self.L + 2, 3)
+        if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or tuple(ca_full.shape) != shape:
+            raise ValueError(f"ca_full must be a float32 tensor of shape {shape}")
+        if ca_full.device != self.device:
+            raise ValueError(f"ca_full must be on {self.device}")
+        N.check(N.lib().cb2_plan_set_coords(self.handle, vae.handle, N.dptr(ca_full.contiguous()), N.stream_ptr()), "set_coords")
+
     # -- denoiser --------------------------------------------------------------------------------
     def forward(self, x, t):
         x = x.to(self.device, torch.float32).contiguous()
@@ -275,3 +287,31 @@ def knn_topk(X: torch.Tensor, lengths, K: int):
     lp = N.dptr(lengths.to(X.device, torch.int32).contiguous()) if lengths is not None else None
     N.check(N.lib().cb2_knn_topk(N.dptr(X, torch.float32), lp, F, L, int(K), N.dptr(D), N.dptr(idx), N.stream_ptr()), "knn_topk")
     return D, idx
+
+
+def radius_graph(X: torch.Tensor, lengths, cutoff: float = 21.0):
+    """Directed radius graph of every frame on the device (cb2_radius_graph_rows / _fill): X [F,L,3] CUDA fp32, lengths [F] (None =
+    all L) -> (row_ptr [F*L+1], col [E]) CUDA int32, the layout of batching.batch_csr(synthetic.radius_graph(...)): a CSR over the
+    padded rows with frame-local columns ascending, an edge i -> j when i != j, both are below the frame's length and
+    sqrt((dx*dx + dy*dy) + dz*dz) <= cutoff in correctly rounded fp32."""
+    N.require_cuda()
+    if not torch.is_tensor(X) or X.dtype != torch.float32 or X.dim() != 3 or X.shape[2] != 3 or X.shape[0] < 1 or X.shape[1] < 1:
+        raise ValueError("X must be a float32 tensor of shape [F, L, 3] with F, L >= 1")
+    if isinstance(cutoff, bool) or not isinstance(cutoff, numbers.Real) or not math.isfinite(cutoff) or cutoff < 0:
+        raise ValueError(f"cutoff must be a finite non-negative number, got {cutoff!r}")
+    X = X.contiguous()
+    F, L, _ = X.shape
+    if lengths is None:
+        lengths = torch.full((F,), L, dtype=torch.int32, device=X.device)
+    lengths = torch.as_tensor(lengths).to(X.device, torch.int32).contiguous()
+    if lengths.shape != (F,):
+        raise ValueError(f"lengths must have shape {(F,)}")
+    row_ptr = torch.empty(F * L + 1, device=X.device, dtype=torch.int32)
+    N.check(N.lib().cb2_radius_graph_rows(N.dptr(X), N.dptr(lengths), F, L, C.c_float(cutoff), N.dptr(row_ptr), N.stream_ptr()),
+            "radius_graph_rows")
+    col = torch.empty(int(row_ptr[-1]), device=X.device, dtype=torch.int32)
+    if col.numel() == 0:
+        return row_ptr, col
+    N.check(N.lib().cb2_radius_graph_fill(N.dptr(X), N.dptr(lengths), F, L, C.c_float(cutoff), N.dptr(row_ptr), N.dptr(col),
+                                          N.stream_ptr()), "radius_graph_fill")
+    return row_ptr, col

@@ -130,6 +130,18 @@ def frames_from_batch(batch: dict, infos, num_ensemble: int = 1, frame_of=None) 
         raise ValueError(f"frames_from_batch: {len(infos)} topology tuples for {F} frames")
     X, cg_z = batching.pad_frames(cg, num, L)
     ca_full = batching.pad_frames(og, num + 2, L + 2)[0]
+    orders, slot_atom, num_atoms = _topology_tables(infos, shared, num, L)
+    csr_row, csr_col = batching.batch_csr(batch["CG_nbr_list"], num, L)
+    if frame_of is None:
+        frame_of = torch.arange(F, dtype=torch.int32).repeat(num_ensemble)
+    frame_of = torch.as_tensor(frame_of, dtype=torch.int32)
+    return FrameSet(X, ca_full, cg_z, num.to(torch.int32), csr_row, csr_col, orders, slot_atom, num_atoms, frame_of)
+
+
+def _topology_tables(infos, shared: bool, num: torch.Tensor, L: int):
+    """Decoder topology of F frames of lengths num [F] padded to L: (orders [F,L,10,3] int8, slot_atom [F,L*14] int32,
+    num_atoms [F] int64), from one shared info tuple or one per frame."""
+    F = num.numel()
     orders = torch.zeros(F, L, 10, 3, dtype=torch.int8)
     orders[..., 1], orders[..., 2] = 1, 2
     slot_atom = torch.full((F, L * 14), -1, dtype=torch.int32)
@@ -147,11 +159,22 @@ def frames_from_batch(batch: dict, infos, num_ensemble: int = 1, frame_of=None) 
             orders[f, :n] = atom_orders.permute(1, 0, 2).to(torch.int8)
             slot_atom[f, :n * 14] = topology.slot_to_atom_map(per_frame[f], n)
             num_atoms[f] = permute.numel()
-    csr_row, csr_col = batching.batch_csr(batch["CG_nbr_list"], num, L)
-    if frame_of is None:
-        frame_of = torch.arange(F, dtype=torch.int32).repeat(num_ensemble)
-    frame_of = torch.as_tensor(frame_of, dtype=torch.int32)
-    return FrameSet(X, ca_full, cg_z, num.to(torch.int32), csr_row, csr_col, orders, slot_atom, num_atoms, frame_of)
+    return orders, slot_atom, num_atoms
+
+
+def frames_from_coords(ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int = 1) -> FrameSet:
+    """FrameSet of F frames of one protein given as coordinates: ca_full [F, L+2, 3] (the coordinate columns of OG_CG_nxyz per
+    frame, termini included), restype [L+2] (its residue ids), info the shared topology tuple; `num_ensemble` members per frame as in
+    frames_from_batch, which it equals on every field except the radius graph: csr_row is all zero and csr_col empty, because the
+    graph is meant to be built on the device (Backmapper.update_coords).  Host tensors."""
+    ca_full = ca_full.detach().cpu().to(torch.float32).contiguous()
+    F, L = ca_full.shape[0], ca_full.shape[1] - 2
+    num = torch.full((F,), L, dtype=torch.int64)
+    cg_z = restype.detach().cpu()[1:-1].to(torch.int32)[None].expand(F, L).contiguous()
+    orders, slot_atom, num_atoms = _topology_tables(info, True, num, L)
+    frame_of = torch.arange(F, dtype=torch.int32).repeat(num_ensemble)
+    return FrameSet(ca_full[:, 1:-1].contiguous(), ca_full, cg_z, num.to(torch.int32), torch.zeros(F * L + 1, dtype=torch.int32),
+                    torch.zeros(0, dtype=torch.int32), orders, slot_atom, num_atoms, frame_of)
 
 
 class Backmapper:
@@ -339,25 +362,85 @@ class Backmapper:
         put more frames into one pass and break coherence chunks - 1 times.  A run that has ended repeats its last frame, and that
         result is dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
         batches = list(batches)
+        steps, runs = self._trajectory_args(len(batches), num_ensemble, steps, chunks)
+        if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
+            raise ValueError("backmap_trajectory: every batch must hold one frame, all of the same length")
+
+        def frame_set(p, frames):
+            fs = frames_from_batch(batching.merge_batches([batches[f] for f in frames]), info, num_ensemble)
+            return self.upload(fs), fs
+
+        return self._trajectory_passes(len(batches), num_ensemble, steps, runs, frame_set, generator)
+
+    def update_coords(self, plan: Plan, fs: FrameSet, ca_full: torch.Tensor):
+        """Move a plan uploaded from `fs` (upload()) to new coordinates of the same frames, with no host work: ca_full [fs.F, fs.L+2, 3]
+        CUDA float32 on the plan's device, the untrimmed traces (cb2_plan_set_coords).  X, the k-NN graph and h_E0, the 21 A radius
+        graph and the IC filters are rebuilt on the device; lengths, residue types, members and topology stay.  Afterwards the host
+        fields X, ca_full, csr_row and csr_col of `fs` no longer describe the plan; its slot_atom, frame_of, out_off and num_atoms,
+        which decode and residue_motion use, stay valid."""
+        if (plan.F, plan.NB, plan.L) != (fs.F, fs.NB, fs.L):
+            raise ValueError("the plan was not uploaded from this frame set")
+        shape = (fs.F, fs.L + 2, 3)
+        if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or tuple(ca_full.shape) != shape:
+            raise ValueError(f"ca_full must be a float32 tensor of shape {shape}")
+        if ca_full.device != plan.device:
+            raise ValueError(f"ca_full must be on {plan.device}")
+        plan.set_coords(self.vae, ca_full)
+
+    def backmap_coords(self, ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int = 1, steps: int = None,
+                       chunks: int = 1, generator: torch.Generator = None) -> torch.Tensor:
+        """backmap_trajectory for a trajectory given as a coordinate array: ca_full float32 [n_frames, L+2, 3], host or CUDA, the
+        coordinate columns of OG_CG_nxyz of every frame (termini included); restype [L+2] integer, its residue ids
+        (OG_CG_nxyz[:, 0]); info the topology tuple.  The topology tables are built on the host once; ca_full is uploaded once,
+        whole, and every pass, the first included, moves the plan to its frames with update_coords, so the radius graph, X and
+        k-NN graph of every frame are built on the device and no batch dict or host graph is needed.  Same passes, arguments and
+        result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to backmap_trajectory on batches of the
+        same frames wherever the caller's graph follows the same 21 A rule (it can differ only for a pair at the cutoff)."""
+        if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or ca_full.dim() != 3 or ca_full.shape[2] != 3 \
+                or ca_full.shape[0] < 1 or ca_full.shape[1] < 3:
+            raise ValueError("ca_full must be a float32 tensor of shape [n_frames, L+2, 3] with n_frames >= 1 and L >= 1")
+        if ca_full.device.type not in ("cpu", "cuda") or (ca_full.is_cuda and ca_full.device.index not in (None, torch.cuda.current_device())):
+            raise ValueError("ca_full must be a host tensor or on the current CUDA device")
+        L = ca_full.shape[1] - 2
+        if not torch.is_tensor(restype) or restype.dtype.is_floating_point or restype.dtype.is_complex or restype.dtype == torch.bool \
+                or tuple(restype.shape) != (L + 2,):
+            raise ValueError(f"restype must be an integer tensor of shape {(L + 2,)}")
+        steps, runs = self._trajectory_args(ca_full.shape[0], num_ensemble, steps, chunks)
+        fs = frames_from_coords(ca_full[[start for start, _ in runs]], restype, info, num_ensemble)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        ca_dev = ca_full.to(dev).contiguous()
+        starts = torch.tensor([start for start, _ in runs], device=dev)
+        last = torch.tensor([n - 1 for _, n in runs], device=dev)
+
+        def frame_set(p, frames):                   # frames = starts + min(p, last), gathered on the device
+            plan = self.upload(fs) if p == 0 else self.plan_for(fs)
+            self.update_coords(plan, fs, ca_dev[starts + torch.clamp(last, max=p)])
+            return plan, fs
+
+        return self._trajectory_passes(ca_full.shape[0], num_ensemble, steps, runs, frame_set, generator)
+
+    def _trajectory_args(self, n_frames: int, num_ensemble, steps, chunks):
+        """Checks of the trajectory methods; returns (steps, runs) with the default steps = T // 4 and runs = trajectory_chunks."""
         if isinstance(num_ensemble, bool) or not isinstance(num_ensemble, numbers.Integral) or num_ensemble < 1:
             raise ValueError(f"num_ensemble must be a positive integer, got {num_ensemble!r}")
         steps = max(1, self.T // 4) if steps is None else steps
         check_start_steps(steps)
         if not 1 <= steps <= self.T:
             raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
-        runs = trajectory_chunks(len(batches), chunks)
-        if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
-            raise ValueError("backmap_trajectory: every batch must hold one frame, all of the same length")
+        return steps, trajectory_chunks(n_frames, chunks)
+
+    def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator) -> torch.Tensor:
+        """The pass loop of the trajectory methods.  Pass p puts frame start + min(p, n - 1) of every run (start, n) on one plan through
+        frame_set(p, frames) -> (plan, fs); pass 0 samples, every later pass refines each member from its own latent of the pass
+        before.  Results of runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
         out = None
         res = None
         for p in range(runs[0][1]):                  # runs[0] is the longest
-            frames = [start + min(p, n - 1) for start, n in runs]
-            fs = frames_from_batch(batching.merge_batches([batches[f] for f in frames]), info, num_ensemble)
-            plan = self.upload(fs)
+            plan, fs = frame_set(p, [start + min(p, n - 1) for start, n in runs])
             if p == 0:
                 res = self.sample(plan, fs, generator=generator)
                 Na = int(fs.num_atoms[0])
-                out = torch.empty(len(batches), num_ensemble, Na, 3, dtype=torch.float32, device=plan.device)
+                out = torch.empty(n_frames, num_ensemble, Na, 3, dtype=torch.float32, device=plan.device)
             else:
                 res = self.refine(plan, fs, res["latent"], steps, generator=generator)
             live = [c for c, (_, n) in enumerate(runs) if p < n]

@@ -24,7 +24,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 5
+#define CB2_ABI_VERSION 6
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -132,6 +132,16 @@ CB2_API int cb2_plan_set_topology(cb2_plan* p, const cb2_vae* v, const float* ca
                           const int* csr_col, int n_edges, const signed char* atom_orders, const int* slot_atom,
                           const long long* out_offset, void* stream);
 
+/* Not in the reference: moves a plan to new coordinates of the frames already on it, with no host work and no host graph.  ca_full
+ * [F,L+2,3] device (untrimmed traces, as for cb2_plan_set_topology).  Lengths, residue types, members and topology stay as they are;
+ * cb2_plan_set_topology must have been called.  In order, on `stream`: copies ca_full; writes X[f,i] = ca_full[f,1+i] for i below
+ * the frame's length and 0 beyond; on a plan with a denoiser, the k-NN graph, edge features and h_E0 of cb2_plan_set_frames; the
+ * directed radius graph at the VAE's own cutoff (21 A; the rule of cb2_radius_graph_rows); the IC distance filters.  The edge count
+ * is read back (4 bytes, one stream synchronisation) to size the graph; its buffers grow geometrically and the replaced ones are
+ * freed.  The captured step loop reads none of these buffers, so its graph stays valid.  The results equal cb2_plan_set_frames +
+ * cb2_plan_set_topology with the same X, ca_full and that radius graph, bit for bit. */
+CB2_API int cb2_plan_set_coords(cb2_plan* p, const cb2_vae* v, const float* ca_full, void* stream);
+
 /* Replaces: get_norm_feature(norm_in=False) + VAE.latent_decode + ic_to_xyz (test.py:548-582;
  * utils/dataset_module.py:230-256; models/vae_model.py:830-839; utils/utils_ic.py:242-268).
  * latent [NB,L,3]; denorm != 0 applies x*std+mean first.  Outputs (any may be NULL): idx [NB,L] int32 (-1 at
@@ -174,6 +184,15 @@ CB2_API int cb2_plan_run_stage(cb2_plan* p, const cb2_vae* v, int stage, int lay
 /* Replaces: CA_ProteinFeatures._dist (protein_mpnn_utils.py:447-459).  D [F,L,K] fp32, idx [F,L,K] int32,
  * sorted ascending by (distance, index).  lengths may be NULL (all L valid). */
 CB2_API int cb2_knn_topk(const float* X, const int* lengths, int F, int L, int K, float* D, int* idx, void* stream);
+
+/* Replaces: the 21 A radius graph the data pipeline builds on the host (utils/protein_module.py:567-584) and its CSR form
+ * (make_directed, models/gcn_nn.py:54-64).  X [F,L,3] fp32, lengths [F] int32.  Edge i -> j of frame f when i != j, both are below
+ * lengths[f] and sqrt((dx*dx + dy*dy) + dz*dz) <= cutoff with dx = x_j - x_i, every operation correctly rounded (no FMA).  Two
+ * calls: _rows writes row_ptr [F*L+1] (int32, CSR over the padded rows; row_ptr[F*L] = the edge count, which the caller reads to
+ * size col); _fill writes col [row_ptr[F*L]] int32, frame-local columns in ascending order.  Deterministic, no atomics. */
+CB2_API int cb2_radius_graph_rows(const float* X, const int* lengths, int F, int L, float cutoff, int* row_ptr, void* stream);
+CB2_API int cb2_radius_graph_fill(const float* X, const int* lengths, int F, int L, float cutoff, const int* row_ptr, int* col,
+                          void* stream);
 
 /* Replaces: VectorQuantize.forward eval (vae_model.py:835) for N = NB*L rows with per-frame lengths. */
 CB2_API int cb2_vq_lookup(const cb2_vae* v, const float* x, int NB, int L, const int* lengths, const int* frame_of,
