@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CB2_LIB") or os.path.join(_HERE, "libcodlad_b200.so")      # CB2_LIB: experiment builds
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 PRECISION = {"fp32": 0, "f32": 0, "f16": 1, "fp16": 1}
 
@@ -52,6 +52,7 @@ SIGNATURES = {
     "cb2_knn_topk": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "cb2_radius_graph_rows": (_I, [_P, _P, _I, _I, C.c_float, _P, _P]),
     "cb2_radius_graph_fill": (_I, [_P, _P, _I, _I, C.c_float, _P, _P, _P]),
+    "cb2_keyed_normal": (_I, [C.c_uint64, _P, _I, _I, C.c_uint32, _I, _I, _P, _P]),
     "cb2_vq_lookup": (_I, [_P, _P, _I, _I, _P, _P, _I, _P, _P, _P]),
     "cb2_p_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
     "cb2_ddim_sample": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),

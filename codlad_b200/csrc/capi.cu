@@ -915,6 +915,17 @@ int cb2_radius_graph_fill(const float* X, const int* lengths, int F, int L, floa
     return launch_radius_fill(X, lengths, F, L, cutoff, row_ptr, col, (cudaStream_t)stream);
 }
 
+int cb2_keyed_normal(uint64_t seed, const int64_t* keys, int NB, int L, uint32_t draw, int first_slice, int n_slices, float* out,
+                     void* stream) {
+    if (!keys || !out) { set_error("keyed_normal: null argument"); return 1; }
+    if (NB < 1 || L < 1 || L >= (1 << 21)) { set_error("keyed_normal: NB=%d must be >= 1 and L=%d in [1, 2^21)", NB, L); return 1; }
+    if (first_slice < 0 || n_slices < 1 || first_slice + (long long)n_slices > 2048) {
+        set_error("keyed_normal: slices [%d, %lld) must lie in [0, 2048) and hold at least one", first_slice, first_slice + (long long)n_slices);
+        return 1;
+    }
+    return launch_keyed_normal(seed, (const long long*)keys, NB, L, draw, first_slice, n_slices, out, (cudaStream_t)stream);
+}
+
 int cb2_vq_lookup(const cb2_vae* v, const float* x, int NB, int L, const int* lengths, const int* frame_of, int denorm,
                   int* idx, float* zq, void* stream) {
     if (!v || !x || !lengths || !frame_of || !idx || !zq) { set_error("vq_lookup: null argument"); return 1; }

@@ -130,6 +130,9 @@ float* plan_P(Plan& p, int which);
 int launch_radius_rows(const float* X, const int* lengths, int F, int L, float cutoff, int* row_ptr, cudaStream_t s);
 int launch_radius_fill(const float* X, const int* lengths, int F, int L, float cutoff, const int* row_ptr, int* col, cudaStream_t s);
 int launch_trim_coords(const float* ca_full, const int* lengths, int F, int L, float* X, cudaStream_t s);
+// noise.cu: keyed Philox4x32-10 normals, out [n_slices, NB, L, 3] for slices first_slice .. first_slice + n_slices - 1
+int launch_keyed_normal(unsigned long long seed, const long long* keys, int NB, int L, unsigned int draw, int first_slice, int n_slices,
+                        float* out, cudaStream_t s);
 
 // The fused update's kept-row overwrite reads the plan's inpainting buffers with `inpaint_row` = the step's
 // {sqrt(acp_prev), sqrt(1 - acp_prev)}; nullptr = no inpainting.

@@ -289,6 +289,52 @@ def knn_topk(X: torch.Tensor, lengths, K: int):
     return D, idx
 
 
+NOISE_MAX_SLICES = 2048      # slice index field of the keyed-noise counter: 11 bits above the 21 of the residue row
+NOISE_MAX_L = 1 << 21
+
+
+def _check_uint(name, v, bits):
+    if isinstance(v, bool) or not isinstance(v, numbers.Integral) or not 0 <= v < (1 << bits):
+        raise ValueError(f"{name} must be an integer in [0, 2^{bits}), got {v!r}")
+
+
+def check_keyed_normal_args(seed, L, draw, first_slice, n_slices):
+    """Scalar arguments of keyed_normal: seed in [0, 2^64), 1 <= L < 2^21, draw in [0, 2^32), slices [first_slice, first_slice +
+    n_slices) non-empty within [0, 2048).  Raises ValueError; touches no device."""
+    _check_uint("seed", seed, 64)
+    _check_uint("draw", draw, 32)
+    if isinstance(L, bool) or not isinstance(L, numbers.Integral) or not 1 <= L < NOISE_MAX_L:
+        raise ValueError(f"L must be an integer in [1, 2^21), got {L!r}")
+    for name, v in (("first_slice", first_slice), ("n_slices", n_slices)):
+        if isinstance(v, bool) or not isinstance(v, numbers.Integral):
+            raise ValueError(f"{name} must be an integer, got {v!r}")
+    if first_slice < 0 or n_slices < 1 or first_slice + n_slices > NOISE_MAX_SLICES:
+        raise ValueError(f"slices [{first_slice}, {first_slice + n_slices}) must be non-empty and lie in [0, {NOISE_MAX_SLICES})")
+
+
+def keyed_normal(seed: int, keys: torch.Tensor, L: int, draw: int, first_slice: int, n_slices: int, out: torch.Tensor = None):
+    """Keyed standard normals (cb2_keyed_normal): slices [first_slice, first_slice + n_slices) of every member as float32
+    [n_slices, NB, L, 3], written into `out` (CUDA float32 contiguous, that shape) when given.  keys int64 [NB] on the current CUDA
+    device, one 64-bit key per member.  Each value depends on (seed, key, draw, slice, row, channel) alone: a member's draws are the
+    same bit for bit in any batch, at any padded length, and a partial fill equals those slices of a full one.  Slice 0 is a
+    sampling pass's start draw and slice 1 + s the noise of respaced step s."""
+    N.require_cuda()
+    check_keyed_normal_args(seed, L, draw, first_slice, n_slices)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if not torch.is_tensor(keys) or keys.dtype != torch.int64 or keys.dim() != 1 or keys.numel() < 1 or keys.device != dev:
+        raise ValueError(f"keys must be a non-empty int64 tensor of shape [NB] on {dev}")
+    keys = keys.contiguous()
+    shape = (int(n_slices), keys.numel(), int(L), 3)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float32, device=dev)
+    elif not torch.is_tensor(out) or out.dtype != torch.float32 or tuple(out.shape) != shape or out.device != dev \
+            or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous float32 tensor of shape {shape} on {dev}")
+    N.check(N.lib().cb2_keyed_normal(int(seed), N.dptr(keys), shape[1], shape[2], int(draw), int(first_slice), int(n_slices), N.dptr(out),
+                                     N.stream_ptr()), "keyed_normal")
+    return out
+
+
 def radius_graph(X: torch.Tensor, lengths, cutoff: float = 21.0):
     """Directed radius graph of every frame on the device (cb2_radius_graph_rows / _fill): X [F,L,3] CUDA fp32, lengths [F] (None =
     all L) -> (row_ptr [F*L+1], col [E]) CUDA int32, the layout of batching.batch_csr(synthetic.radius_graph(...)): a CSR over the

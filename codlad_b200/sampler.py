@@ -20,7 +20,7 @@ import torch
 
 from . import batching, distributed, metrics, topology, weights
 from .diffusion import create_diffusion
-from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args, check_start_steps
+from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args, check_keyed_normal_args, check_start_steps, keyed_normal
 
 VAE_DATA = {"N6": "PED", "K3": "PDB", "K4": "Atlas"}
 
@@ -64,6 +64,51 @@ def residue_atom_ranges(fs: "FrameSet"):
     rows = torch.nonzero(counts > 0).squeeze(1)
     atoms = (slots.long() + fs.out_off.cpu().long()[:, None, None])[present]      # row-major: each residue's atoms in one run
     return atoms, counts[rows], rows
+
+
+MEMBER_BITS = 16            # member key = frame key * 2^16 + ensemble index
+FRAME_KEY_LIMIT = 1 << 47   # frame keys in [0, 2^47) keep every member key a non-negative int64
+
+
+def member_keys(fs: "FrameSet", frame_keys=None) -> torch.Tensor:
+    """Keys of the keyed sampling noise (engine.keyed_normal), host int64 [NB]: key_b = frame_keys[frame_of[b]] * 2^16 + e_b, where
+    e_b counts the members of b's frame that come before b in member order.  frame_keys [F] defaults to arange(F); a caller that
+    samples part of a larger job passes the frames' indices in that job, so a member gets the same noise as there.  For
+    frames_from_batch(..., num_ensemble), where b = e * F + f, key_b = f * 2^16 + e."""
+    fo = fs.frame_of.detach().cpu().long()
+    if frame_keys is None:
+        frame_keys = torch.arange(fs.F, dtype=torch.int64)
+    else:
+        frame_keys = torch.as_tensor(frame_keys).detach().cpu()
+        if frame_keys.dtype.is_floating_point or frame_keys.dtype.is_complex or frame_keys.dtype == torch.bool \
+                or tuple(frame_keys.shape) != (fs.F,):
+            raise ValueError(f"frame_keys must be an integer sequence of length {fs.F}")
+        frame_keys = frame_keys.long()
+    order = torch.sort(fo, stable=True).indices                         # members grouped by frame, member order kept within a frame
+    counts = torch.bincount(fo, minlength=fs.F)
+    ens = torch.empty_like(fo)
+    ens[order] = torch.arange(fs.NB) - (torch.cumsum(counts, 0) - counts)[fo[order]]
+    return _compose_keys(frame_keys[fo], ens)
+
+
+def unit_keys(units) -> torch.Tensor:
+    """member_keys for a list of (frame, ensemble index) units of a job: host int64 [len(units)], key = frame * 2^16 + e, the key
+    the unit gets from member_keys in a single frames_from_batch of the whole job (b = e * F + f).  ShardedBackmapper keys each
+    rank's units with it."""
+    t = torch.tensor([[int(f), int(e)] for f, e in units], dtype=torch.int64).view(-1, 2)
+    if bool((t[:, 0] < 0).any()) or bool((t[:, 1] < 0).any()):
+        raise ValueError("frame and ensemble indices of the units must be non-negative")
+    return _compose_keys(t[:, 0], t[:, 1])
+
+
+def _compose_keys(frame_keys: torch.Tensor, ens: torch.Tensor) -> torch.Tensor:
+    """frame_keys * 2^16 + ens (int64), refusing what would make two members share a key: a frame key outside [0, 2^47) or an
+    ensemble index of 2^16 or more."""
+    if bool(((frame_keys < 0) | (frame_keys >= FRAME_KEY_LIMIT)).any()):
+        raise ValueError("frame keys must lie in [0, 2^47)")
+    if ens.numel() and int(ens.max()) >= 1 << MEMBER_BITS:
+        raise ValueError(f"a frame holds {int(ens.max()) + 1} members; member keys allow at most 2^16 per frame")
+    return frame_keys * (1 << MEMBER_BITS) + ens
 
 
 @dataclass
@@ -200,6 +245,7 @@ class Backmapper:
         self.T = self.diffusion.num_timesteps
         self._plans = {}
         self._bufs = {}
+        self._keys = {}                 # id(plan) -> (host keys, the same on the device) of the plan's last seeded pass
         self._host_xyz = {}
 
     def plan_for(self, fs: FrameSet, keep_debug: bool = False) -> Plan:
@@ -209,6 +255,7 @@ class Backmapper:
             while len(self._plans) >= self.max_plans:              # a plan owns every buffer of its geometry: keep few of them
                 old = self._plans.pop(next(iter(self._plans)))
                 self._bufs.pop(id(old), None)
+                self._keys.pop(id(old), None)
                 old.close()
             plan = Plan(self.denoiser, fs.F, fs.NB, fs.L, self.precision, keep_debug)
             if self.sampler == "ddim":
@@ -228,34 +275,44 @@ class Backmapper:
         return plan
 
     def sample(self, plan: Plan, fs: FrameSet, z: torch.Tensor = None, step_noise: torch.Tensor = None,
-               use_graph: bool = True, generator: torch.Generator = None):
+               use_graph: bool = True, generator: torch.Generator = None, seed: int = None, keys: torch.Tensor = None, draw: int = 0):
         """Device-resident path: returns dict(latent, idx, ic_recon, xyz) of CUDA tensors.
-        z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted.  DDIM with eta = 0 uses no
-        step noise: `step_noise` is ignored.  Every residue is sampled anew, also after resample() on the same plan."""
+        z [NB,L,3] initial noise, step_noise [T,NB,L,3]; drawn on the device when omitted, from `generator` or, with `seed`, as
+        keyed noise (engine.keyed_normal): member b gets slices 0 (z) and 1 + s (the noise of step s) of its key keys[b] (int64 [NB],
+        default member_keys(fs)) and `draw`, the same in any batch that holds it.  seed excludes generator, z and step_noise.
+        DDIM with eta = 0 uses no step noise: `step_noise` is ignored.  Every residue is sampled anew, also after resample() on
+        the same plan."""
+        self._check_noise_args(fs, z, step_noise, generator, seed, keys, draw)
         plan.clear_inpaint()
         plan.set_start(0)
-        return self._sample(plan, fs, z, step_noise, use_graph, generator)
+        return self._sample(plan, fs, z, step_noise, use_graph, generator, None, seed, keys, draw)
 
     def resample(self, plan: Plan, fs: FrameSet, latent: torch.Tensor, keep: torch.Tensor, z: torch.Tensor = None,
-                 step_noise: torch.Tensor = None, generator: torch.Generator = None):
+                 step_noise: torch.Tensor = None, generator: torch.Generator = None, seed: int = None, keys: torch.Tensor = None,
+                 draw: int = 0):
         """Latent inpainting: keep the residues of an earlier pass where keep [NB,L] (bool) is True and sample the others
         anew, conditioned on the kept ones through the denoiser.  latent [NB,L,3] is that pass's normalised latent
         (`sample(...)["latent"]`, which may be passed as is).  Kept rows follow the forward marginal of their latent with the
-        fixed draw z and end at it exactly, so they keep their VQ index.  z and step_noise as in sample().  Returns the same
-        dict as sample()."""
+        fixed draw z and end at it exactly, so they keep their VQ index.  z, step_noise, generator, seed, keys and draw as in
+        sample().  Returns the same dict as sample()."""
+        self._check_noise_args(fs, z, step_noise, generator, seed, keys, draw)
         self._check_latent_keep(plan, fs, latent, keep)
         plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())      # copies latent before z overwrites its buffer
         plan.set_start(0)
-        return self._sample(plan, fs, z, step_noise, True, generator)
+        return self._sample(plan, fs, z, step_noise, True, generator, None, seed, keys, draw)
 
     def refine(self, plan: Plan, fs: FrameSet, latent: torch.Tensor, steps: int, keep: torch.Tensor = None, z: torch.Tensor = None,
-               step_noise: torch.Tensor = None, generator: torch.Generator = None):
+               step_noise: torch.Tensor = None, generator: torch.Generator = None, seed: int = None, keys: torch.Tensor = None,
+               draw: int = 0):
         """Partial-noise refinement (SDEdit): noise the normalised latent [NB,L,3] to the level of respaced step `steps` with the
         draw z, x = sqrt(acp[steps-1]) latent + sqrt(1 - acp[steps-1]) z, and run only the last `steps` of the T steps,
         conditioned on the frames of `fs` as uploaded now.  The strength is steps / T, with 1 <= steps <= T.  latent may be
         `sample(...)["latent"]` as it is.  keep [NB,L] (bool) keeps those residues exactly, as resample() does; None refines every
         residue.  z [NB,L,3] and step_noise [T,NB,L,3] (slices [0, steps) are read) are drawn when omitted; DDIM with eta = 0 uses
-        no step noise.  Returns the same dict as sample(); a later sample() or resample() is a full pass again."""
+        no step noise.  With `seed` the keyed slices 0 and 1 .. steps are filled, the ones a full pass would use for z and those
+        steps (generator, seed, keys and draw as in sample()).  Returns the same dict as sample(); a later sample() or resample()
+        is a full pass again."""
+        self._check_noise_args(fs, z, step_noise, generator, seed, keys, draw)
         check_start_steps(steps)
         if not 1 <= steps <= self.T:
             raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
@@ -264,7 +321,20 @@ class Backmapper:
         self._check_latent_keep(plan, fs, latent, keep)
         plan.set_inpaint(keep, latent, self.diffusion.inpaint_coef_table())
         plan.set_start(steps)
-        return self._sample(plan, fs, z, step_noise, True, generator, steps)
+        return self._sample(plan, fs, z, step_noise, True, generator, steps, seed, keys, draw)
+
+    @staticmethod
+    def _check_noise_args(fs: FrameSet, z, step_noise, generator, seed, keys, draw):
+        """seed is one source of noise, generator / z / step_noise another; keys [NB] (int64) and draw belong to seed."""
+        if seed is None:
+            if keys is not None or draw != 0:
+                raise ValueError("keys and draw select keyed noise: they need a seed")
+            return
+        if generator is not None or z is not None or step_noise is not None:
+            raise ValueError("seed draws z and the step noise itself: it excludes generator, z and step_noise")
+        check_keyed_normal_args(seed, fs.L, draw, 0, 1)
+        if keys is not None and (not torch.is_tensor(keys) or keys.dtype != torch.int64 or tuple(keys.shape) != (fs.NB,)):
+            raise ValueError(f"keys must be an int64 tensor of shape {(fs.NB,)}")
 
     @staticmethod
     def _check_latent_keep(plan: Plan, fs: FrameSet, latent, keep):
@@ -290,13 +360,14 @@ class Backmapper:
         return plan.residue_clashes(xyz, threshold, grow)
 
     def repair(self, plan: Plan, fs: FrameSet, out: dict, max_rounds: int = 3, grow: int = 0, threshold: float = 1.2,
-               generator: torch.Generator = None):
+               generator: torch.Generator = None, seed: int = None, keys: torch.Tensor = None):
         """Clash-driven repair of a backmapped sample `out` (the dict of sample() / resample()): each round flags the clashing
         residues (residue_clashes), stops when no member has a clash, and otherwise resamples the flagged residues of every
-        member with latent inpainting, fresh noise from `generator`.  Per member the new latent is accepted only when its number
-        of clashing pairs went down; otherwise the member keeps its previous latent.  The accepted latents are decoded once at the
-        end.  Kept residues keep their latent and VQ index; their coordinates can still move where the IC decoder's radius graph
-        reaches a regenerated neighbour.  A round costs one resample pass (one sampling pass plus decode).
+        member with latent inpainting, fresh noise from `generator`, or with `seed` the keyed noise of draw r + 1 in round r
+        (keys as in sample()), so a member's rounds draw what they would in any other batch.  Per member the new latent is accepted
+        only when its number of clashing pairs went down; otherwise the member keeps its previous latent.  The accepted latents are
+        decoded once at the end.  Kept residues keep their latent and VQ index; their coordinates can still move where the IC
+        decoder's radius graph reaches a regenerated neighbour.  A round costs one resample pass (one sampling pass plus decode).
         Returns the dict of sample() plus `clashes` (int32 [NB, L], the counts of the returned structure) and `clash_pairs`
         (int64 [rounds run + 1, NB], clashing pairs per member; row 0 is the input's).  The plan is left for plain sample()."""
         if not isinstance(out, dict) or not all(k in out for k in ("latent", "idx", "zq", "ic_recon", "xyz")):
@@ -304,6 +375,7 @@ class Backmapper:
         if isinstance(max_rounds, bool) or not isinstance(max_rounds, int) or max_rounds < 0:
             raise ValueError(f"max_rounds must be a non-negative integer, got {max_rounds!r}")
         check_clash_args(threshold, grow, plan.K)
+        self._check_noise_args(fs, None, None, generator, seed, keys, 0)
         shape = (fs.NB, fs.L, 3)
         latent = out["latent"]
         if not torch.is_tensor(latent) or latent.dtype != torch.float32 or tuple(latent.shape) != shape or latent.device != plan.device:
@@ -312,10 +384,10 @@ class Backmapper:
         pairs = clash_pair_totals(counts)
         rows = [pairs]
         latent = latent.clone()                  # resample() writes the plan's latent buffer, which out["latent"] may be
-        for _ in range(max_rounds):
+        for r in range(max_rounds):
             if not bool((pairs > 0).any()):
                 break
-            new = self.resample(plan, fs, latent, keep, generator=generator)
+            new = self.resample(plan, fs, latent, keep, generator=generator, seed=seed, keys=keys, draw=0 if seed is None else r + 1)
             new_counts, new_keep = self.residue_clashes(plan, fs, new["xyz"], threshold, grow)
             new_pairs = clash_pair_totals(new_counts)
             acc = repair_accept(pairs, new_pairs)
@@ -353,14 +425,16 @@ class Backmapper:
         return out.view(fs.NB, fs.L)
 
     def backmap_trajectory(self, batches, info, num_ensemble: int = 1, steps: int = None, chunks: int = 1,
-                           generator: torch.Generator = None) -> torch.Tensor:
+                           generator: torch.Generator = None, seed: int = None) -> torch.Tensor:
         """Backmap consecutive frames of one protein with warm starts.  batches: one reference-schema batch dict per frame (one
         frame each, all of the same length), info: the shared topology tuple.  The frames are split into `chunks` contiguous runs
         (trajectory_chunks) that go through one plan together, each run with `num_ensemble` members.  The first frame of every run
         is sampled from noise (sample()); every later frame refines each member's latent of the previous frame (refine(), `steps`
         of the T steps, default T // 4), so members stay coherent along a run and cost steps / T of the loop per frame.  More chunks
         put more frames into one pass and break coherence chunks - 1 times.  A run that has ended repeats its last frame, and that
-        result is dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        result is dropped.  With `seed` (instead of `generator`) member e of frame f draws keyed noise (engine.keyed_normal) with key
+        f * 2^16 + e, draw 0 when it is sampled and draw 1 when it is refined, so its noise does not depend on `chunks`; its result
+        still does, through the warm start it refines.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
         batches = list(batches)
         steps, runs = self._trajectory_args(len(batches), num_ensemble, steps, chunks)
         if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
@@ -370,7 +444,7 @@ class Backmapper:
             fs = frames_from_batch(batching.merge_batches([batches[f] for f in frames]), info, num_ensemble)
             return self.upload(fs), fs
 
-        return self._trajectory_passes(len(batches), num_ensemble, steps, runs, frame_set, generator)
+        return self._trajectory_passes(len(batches), num_ensemble, steps, runs, frame_set, generator, seed)
 
     def update_coords(self, plan: Plan, fs: FrameSet, ca_full: torch.Tensor):
         """Move a plan uploaded from `fs` (upload()) to new coordinates of the same frames, with no host work: ca_full [fs.F, fs.L+2, 3]
@@ -388,14 +462,15 @@ class Backmapper:
         plan.set_coords(self.vae, ca_full)
 
     def backmap_coords(self, ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int = 1, steps: int = None,
-                       chunks: int = 1, generator: torch.Generator = None) -> torch.Tensor:
+                       chunks: int = 1, generator: torch.Generator = None, seed: int = None) -> torch.Tensor:
         """backmap_trajectory for a trajectory given as a coordinate array: ca_full float32 [n_frames, L+2, 3], host or CUDA, the
         coordinate columns of OG_CG_nxyz of every frame (termini included); restype [L+2] integer, its residue ids
         (OG_CG_nxyz[:, 0]); info the topology tuple.  The topology tables are built on the host once; ca_full is uploaded once,
         whole, and every pass, the first included, moves the plan to its frames with update_coords, so the radius graph, X and
-        k-NN graph of every frame are built on the device and no batch dict or host graph is needed.  Same passes, arguments and
-        result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to backmap_trajectory on batches of the
-        same frames wherever the caller's graph follows the same 21 A rule (it can differ only for a pair at the cutoff)."""
+        k-NN graph of every frame are built on the device and no batch dict or host graph is needed.  Same passes, arguments (`seed`
+        included) and result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to backmap_trajectory on
+        batches of the same frames wherever the caller's graph follows the same 21 A rule (it can differ only for a pair at the
+        cutoff)."""
         if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or ca_full.dim() != 3 or ca_full.shape[2] != 3 \
                 or ca_full.shape[0] < 1 or ca_full.shape[1] < 3:
             raise ValueError("ca_full must be a float32 tensor of shape [n_frames, L+2, 3] with n_frames >= 1 and L >= 1")
@@ -417,7 +492,7 @@ class Backmapper:
             self.update_coords(plan, fs, ca_dev[starts + torch.clamp(last, max=p)])
             return plan, fs
 
-        return self._trajectory_passes(ca_full.shape[0], num_ensemble, steps, runs, frame_set, generator)
+        return self._trajectory_passes(ca_full.shape[0], num_ensemble, steps, runs, frame_set, generator, seed)
 
     def _trajectory_args(self, n_frames: int, num_ensemble, steps, chunks):
         """Checks of the trajectory methods; returns (steps, runs) with the default steps = T // 4 and runs = trajectory_chunks."""
@@ -429,26 +504,32 @@ class Backmapper:
             raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
         return steps, trajectory_chunks(n_frames, chunks)
 
-    def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator) -> torch.Tensor:
+    def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator, seed=None) -> torch.Tensor:
         """The pass loop of the trajectory methods.  Pass p puts frame start + min(p, n - 1) of every run (start, n) on one plan through
         frame_set(p, frames) -> (plan, fs); pass 0 samples, every later pass refines each member from its own latent of the pass
-        before.  Results of runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        before; with `seed` the keys are the absolute frame indices (member_keys) and the draw is 0 for pass 0, 1 after.  Results of
+        runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        if seed is not None and generator is not None:
+            raise ValueError("seed draws the noise itself: it excludes generator")
         out = None
         res = None
         for p in range(runs[0][1]):                  # runs[0] is the longest
-            plan, fs = frame_set(p, [start + min(p, n - 1) for start, n in runs])
+            frames = [start + min(p, n - 1) for start, n in runs]
+            plan, fs = frame_set(p, frames)
+            noise = {"generator": generator} if seed is None else {"seed": seed, "keys": member_keys(fs, frames), "draw": int(p > 0)}
             if p == 0:
-                res = self.sample(plan, fs, generator=generator)
+                res = self.sample(plan, fs, **noise)
                 Na = int(fs.num_atoms[0])
                 out = torch.empty(n_frames, num_ensemble, Na, 3, dtype=torch.float32, device=plan.device)
             else:
-                res = self.refine(plan, fs, res["latent"], steps, generator=generator)
+                res = self.refine(plan, fs, res["latent"], steps, **noise)
             live = [c for c, (_, n) in enumerate(runs) if p < n]
             xyz = res["xyz"].view(num_ensemble, len(runs), Na, 3)                 # members are ensemble-major: b = e * chunks + c
             out[[runs[c][0] + p for c in live]] = xyz[:, live].transpose(0, 1)
         return out.cpu()
 
-    def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator, steps: int = None):
+    def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator, steps: int = None, seed: int = None,
+                keys: torch.Tensor = None, draw: int = 0):
         dev = plan.device
         shape = (fs.NB, fs.L, 3)
         noisy = self.sampler == "ddpm" or self.eta != 0
@@ -457,25 +538,42 @@ class Backmapper:
             bufs = (torch.empty(*shape, device=dev), torch.empty(self.T, *shape, device=dev) if noisy else None)
             self._bufs[id(plan)] = bufs
         x, noise = bufs
-        if z is not None:
+        n = self.T if steps is None else steps                          # the loop reads noise slices [0, steps) only
+        if seed is not None:              # keyed: slice 0 into x, slices 1 .. n into noise[:n], in place (the graph key stays)
+            keys = self._device_keys(plan, fs, keys)
+            keyed_normal(seed, keys, fs.L, draw, 0, 1, out=x.unsqueeze(0))
+            if noise is not None:
+                keyed_normal(seed, keys, fs.L, draw, 1, n, out=noise[:n])
+        elif z is not None:
             x.copy_(z, non_blocking=True)
         else:
             torch.randn(*shape, device=dev, generator=generator, out=x)
-        if noise is not None:
+        if seed is None and noise is not None:
             if step_noise is not None:
                 noise.copy_(step_noise, non_blocking=True)
             else:
-                n = self.T if steps is None else steps                 # the loop reads slices [0, steps) only
                 torch.randn(n, *shape, device=dev, generator=generator, out=noise[:n])
         plan.sample(x, noise, use_graph)
         idx, zq, ic, xyz = plan.decode(self.vae, x, denorm=True, num_atoms_total=fs.total_atoms)
         return {"latent": x, "idx": idx, "zq": zq, "ic_recon": ic, "xyz": xyz}
 
-    def backmap_host(self, fs: FrameSet, z=None, step_noise=None, generator: torch.Generator = None):
+    def _device_keys(self, plan: Plan, fs: FrameSet, keys) -> torch.Tensor:
+        """keys (default member_keys(fs)) on the plan's device.  The last host keys of a plan stay on the device, so repeated passes
+        with the same members make no copy (a copy from pageable memory would synchronise the stream)."""
+        keys = member_keys(fs) if keys is None else keys
+        if keys.is_cuda:
+            return keys.to(plan.device).contiguous()
+        cached = self._keys.get(id(plan))
+        if cached is None or not torch.equal(cached[0], keys):
+            cached = self._keys[id(plan)] = (keys.clone(), keys.to(plan.device).contiguous())
+        return cached[1]
+
+    def backmap_host(self, fs: FrameSet, z=None, step_noise=None, generator: torch.Generator = None, seed: int = None,
+                     keys: torch.Tensor = None):
         """End-to-end call with HOST inputs and HOST coordinates out (what bench.py's e2e times):
-        H2D of the frame set, per-frame precompute, T-step sampling, decode, D2H of [sum Na, 3]."""
+        H2D of the frame set, per-frame precompute, T-step sampling, decode, D2H of [sum Na, 3].  Noise as in sample()."""
         plan = self.upload(fs)
-        out = self.sample(plan, fs, z, step_noise, generator=generator)
+        out = self.sample(plan, fs, z, step_noise, generator=generator, seed=seed, keys=keys)
         host = self._host_xyz.get(fs.total_atoms)
         if host is None:
             host = self._host_xyz[fs.total_atoms] = torch.empty(fs.total_atoms, 3, dtype=torch.float32).pin_memory()
@@ -545,8 +643,10 @@ class ShardedBackmapper:
             out.append((frames, [frames.index(f) for f, _ in members], members))
         return out
 
-    def backmap_local(self, batches, infos, units, lengths, generator=None):
-        """Back-map this rank's units: {(frame, member): host tensor [Na, 3]}."""
+    def backmap_local(self, batches, infos, units, lengths, generator=None, seed=None):
+        """Back-map this rank's units: {(frame, member): host tensor [Na, 3]}.  With `seed` (instead of `generator`) unit (f, e) draws
+        keyed noise with key f * 2^16 + e (unit_keys), f its index in the whole job: what frames_from_batch of the whole job with
+        member_keys gives it on one GPU, so its noise does not depend on the world size or on the group it lands in."""
         res = {}
         for frames, frame_of, members in self.local_groups(units, lengths):
             # the padded / CSR form of a group is input-format conversion: done once per group of frames (keyed on the very batch
@@ -559,20 +659,26 @@ class ShardedBackmapper:
                     self._fs_cache.pop(next(iter(self._fs_cache)))
                 self._fs_cache[key] = fs
                 fs._keep = [batches[f] for f in frames]          # the ids in the key stay valid while the entry lives
-            host = self.bm.backmap_host(fs, generator=generator)
+            keys = None if seed is None else unit_keys(members)
+            host = self.bm.backmap_host(fs, generator=generator, seed=seed, keys=keys)
             for b, fe in enumerate(members):
                 o, na = int(fs.out_off[b]), int(fs.num_atoms[frame_of[b]])
                 res[fe] = host[o:o + na].clone()
         return res
 
-    def backmap(self, batches, infos, num_ensemble: int, generator=None, _compute=None):
+    def backmap(self, batches, infos, num_ensemble: int, generator=None, _compute=None, seed=None):
         """batches: one reference-schema batch dict per frame (CG_collate of a single frame), infos: its `info` tuple.
-        Returns on rank 0 {(frame, member): [Na, 3]} for EVERY unit of the job, on the other ranks None."""
+        Returns on rank 0 {(frame, member): [Na, 3]} for EVERY unit of the job, on the other ranks None.  With `seed` every unit
+        gets the same noise on any number of GPUs (backmap_local).  Its result can still depend on the number of GPUs: the model
+        depends on the padded length of the plan a frame is sampled in, and group_by_length groups a rank's frames differently
+        for different shares of the job."""
         import torch.distributed as dist
         lengths = [int(b["num_CGs"].sum()) for b in batches]
         n_atoms = [int(i[0].numel()) for i in infos]
         parts = self.plan(lengths, num_ensemble)
-        mine = (_compute or self.backmap_local)(batches, infos, parts[self.rank], lengths, generator) if parts[self.rank] else {}
+        noise = {} if seed is None else {"seed": seed}                  # a compute hook that takes no seed refuses one loudly
+        compute = _compute or self.backmap_local
+        mine = compute(batches, infos, parts[self.rank], lengths, generator, **noise) if parts[self.rank] else {}
         if self.world == 1 or not (dist.is_available() and dist.is_initialized()):
             return mine
         flat = lambda units, res: torch.cat([res[u] for u in units], 0) if units else torch.zeros(0, 3)

@@ -14,6 +14,8 @@
 #ifndef CODLAD_B200_H
 #define CODLAD_B200_H
 
+#include <stdint.h>
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -24,7 +26,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 6
+#define CB2_ABI_VERSION 7
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -193,6 +195,18 @@ CB2_API int cb2_knn_topk(const float* X, const int* lengths, int F, int L, int K
 CB2_API int cb2_radius_graph_rows(const float* X, const int* lengths, int F, int L, float cutoff, int* row_ptr, void* stream);
 CB2_API int cb2_radius_graph_fill(const float* X, const int* lengths, int F, int L, float cutoff, const int* row_ptr, int* col,
                           void* stream);
+
+/* Replaces: the torch.randn draws of the start latent and the per-step noise (gaussian_diffusion.py:440,540 randn / randn_like) when
+ * a sample has to be reproducible per member.  Not in the reference.  out [n_slices, NB, L, 3] fp32 gets slices first_slice ..
+ * first_slice + n_slices - 1 of member b = keys[b] (int64 [NB], any 64-bit value); slice 0 is the start draw, slice 1 + s the noise
+ * of respaced step s.  Philox4x32-10 keyed by seed, counter (key lo, key hi, draw, (slice << 21) | i) for row i, padded rows
+ * included; the four words give the three channels by Box-Muller twice, u = ((w >> 8) + 0.5) 2^-24 in fp32, which lies in (0, 1]
+ * (never 0; the largest word rounds to 1), (n0, n1) = sqrt(-2 ln u0) (cospi(2 u1), sinpi(2 u1)), n2 = sqrt(-2 ln u2) cospi(2 u3),
+ * with logf / sqrtf / sincospif.  A value depends on (seed, key, draw,
+ * slice, i, channel) alone, so it is the same bit for bit whatever NB, L, the member's position or the slice range of the call.
+ * Refuses NULL pointers, NB < 1, L < 1, L >= 2^21, first_slice < 0, n_slices < 1 and first_slice + n_slices > 2048.  One launch. */
+CB2_API int cb2_keyed_normal(uint64_t seed, const int64_t* keys, int NB, int L, uint32_t draw, int first_slice, int n_slices, float* out,
+                     void* stream);
 
 /* Replaces: VectorQuantize.forward eval (vae_model.py:835) for N = NB*L rows with per-frame lengths. */
 CB2_API int cb2_vq_lookup(const cb2_vae* v, const float* x, int NB, int L, const int* lengths, const int* frame_of,
