@@ -51,6 +51,32 @@ def trajectory_chunks(n_frames: int, chunks: int):
     return runs
 
 
+def trajectory_args(T: int, n_frames: int, num_ensemble, steps, chunks):
+    """Checks of the trajectory methods for a T-step schedule; returns (steps, runs) with the default steps = T // 4 and
+    runs = trajectory_chunks(n_frames, chunks)."""
+    if isinstance(num_ensemble, bool) or not isinstance(num_ensemble, numbers.Integral) or num_ensemble < 1:
+        raise ValueError(f"num_ensemble must be a positive integer, got {num_ensemble!r}")
+    steps = max(1, T // 4) if steps is None else steps
+    check_start_steps(steps)
+    if not 1 <= steps <= T:
+        raise ValueError(f"steps must be in [1, {T}], got {steps}")
+    return steps, trajectory_chunks(n_frames, chunks)
+
+
+def check_coords_args(ca_full, restype):
+    """The input checks of Backmapper.backmap_coords: ca_full float32 [n_frames, L+2, 3] (n_frames, L >= 1) on the host or the
+    current CUDA device, restype integer [L+2]."""
+    if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or ca_full.dim() != 3 or ca_full.shape[2] != 3 \
+            or ca_full.shape[0] < 1 or ca_full.shape[1] < 3:
+        raise ValueError("ca_full must be a float32 tensor of shape [n_frames, L+2, 3] with n_frames >= 1 and L >= 1")
+    if ca_full.device.type not in ("cpu", "cuda") or (ca_full.is_cuda and ca_full.device.index not in (None, torch.cuda.current_device())):
+        raise ValueError("ca_full must be a host tensor or on the current CUDA device")
+    L = ca_full.shape[1] - 2
+    if not torch.is_tensor(restype) or restype.dtype.is_floating_point or restype.dtype.is_complex or restype.dtype == torch.bool \
+            or tuple(restype.shape) != (L + 2,):
+        raise ValueError(f"restype must be an integer tensor of shape {(L + 2,)}")
+
+
 def residue_atom_ranges(fs: "FrameSet"):
     """The atoms of every real residue of every member of `fs`, gathered through slot_atom into contiguous ranges.  Returns
     (atoms int64 [A], counts int64 [R], rows int64 [R]): residue r = row rows[r] of the flattened [NB, L] grid owns
@@ -436,7 +462,7 @@ class Backmapper:
         f * 2^16 + e, draw 0 when it is sampled and draw 1 when it is refined, so its noise does not depend on `chunks`; its result
         still does, through the warm start it refines.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
         batches = list(batches)
-        steps, runs = self._trajectory_args(len(batches), num_ensemble, steps, chunks)
+        steps, runs = trajectory_args(self.T, len(batches), num_ensemble, steps, chunks)
         if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
             raise ValueError("backmap_trajectory: every batch must hold one frame, all of the same length")
 
@@ -471,52 +497,48 @@ class Backmapper:
         included) and result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to backmap_trajectory on
         batches of the same frames wherever the caller's graph follows the same 21 A rule (it can differ only for a pair at the
         cutoff)."""
-        if not torch.is_tensor(ca_full) or ca_full.dtype != torch.float32 or ca_full.dim() != 3 or ca_full.shape[2] != 3 \
-                or ca_full.shape[0] < 1 or ca_full.shape[1] < 3:
-            raise ValueError("ca_full must be a float32 tensor of shape [n_frames, L+2, 3] with n_frames >= 1 and L >= 1")
-        if ca_full.device.type not in ("cpu", "cuda") or (ca_full.is_cuda and ca_full.device.index not in (None, torch.cuda.current_device())):
-            raise ValueError("ca_full must be a host tensor or on the current CUDA device")
-        L = ca_full.shape[1] - 2
-        if not torch.is_tensor(restype) or restype.dtype.is_floating_point or restype.dtype.is_complex or restype.dtype == torch.bool \
-                or tuple(restype.shape) != (L + 2,):
-            raise ValueError(f"restype must be an integer tensor of shape {(L + 2,)}")
-        steps, runs = self._trajectory_args(ca_full.shape[0], num_ensemble, steps, chunks)
+        check_coords_args(ca_full, restype)
+        steps, runs = trajectory_args(self.T, ca_full.shape[0], num_ensemble, steps, chunks)
+        return self._coords_passes(ca_full, restype, info, num_ensemble, steps, runs, generator, seed)
+
+    def _coords_passes(self, ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int, steps: int, runs, generator,
+                       seed=None, key_offset: int = 0) -> torch.Tensor:
+        """The body of backmap_coords for any subset of a trajectory's runs (start, n) (trajectory_chunks order): one plan holds them
+        all, only their frames are uploaded, and frame f draws keyed noise with frame key key_offset + f.  Returns host float32
+        [sum n, num_ensemble, Na, 3], the frames of the runs in order."""
         fs = frames_from_coords(ca_full[[start for start, _ in runs]], restype, info, num_ensemble)
         dev = torch.device("cuda", torch.cuda.current_device())
-        ca_dev = ca_full.to(dev).contiguous()
-        starts = torch.tensor([start for start, _ in runs], device=dev)
+        rows = torch.cat([torch.arange(start, start + n) for start, n in runs])
+        ca_dev = ca_full[rows.to(ca_full.device)].to(dev)
+        first = torch.tensor([0] + [n for _, n in runs[:-1]]).cumsum(0).to(dev)      # each run's first row of ca_dev
         last = torch.tensor([n - 1 for _, n in runs], device=dev)
 
-        def frame_set(p, frames):                   # frames = starts + min(p, last), gathered on the device
+        def frame_set(p, frames):                   # rows first + min(p, last) of ca_dev, gathered on the device
             plan = self.upload(fs) if p == 0 else self.plan_for(fs)
-            self.update_coords(plan, fs, ca_dev[starts + torch.clamp(last, max=p)])
+            self.update_coords(plan, fs, ca_dev[first + torch.clamp(last, max=p)])
             return plan, fs
 
-        return self._trajectory_passes(ca_full.shape[0], num_ensemble, steps, runs, frame_set, generator, seed)
+        return self._trajectory_passes(rows.numel(), num_ensemble, steps, runs, frame_set, generator, seed, key_offset)
 
-    def _trajectory_args(self, n_frames: int, num_ensemble, steps, chunks):
-        """Checks of the trajectory methods; returns (steps, runs) with the default steps = T // 4 and runs = trajectory_chunks."""
-        if isinstance(num_ensemble, bool) or not isinstance(num_ensemble, numbers.Integral) or num_ensemble < 1:
-            raise ValueError(f"num_ensemble must be a positive integer, got {num_ensemble!r}")
-        steps = max(1, self.T // 4) if steps is None else steps
-        check_start_steps(steps)
-        if not 1 <= steps <= self.T:
-            raise ValueError(f"steps must be in [1, {self.T}], got {steps}")
-        return steps, trajectory_chunks(n_frames, chunks)
-
-    def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator, seed=None) -> torch.Tensor:
+    def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator, seed=None,
+                           key_offset: int = 0) -> torch.Tensor:
         """The pass loop of the trajectory methods.  Pass p puts frame start + min(p, n - 1) of every run (start, n) on one plan through
         frame_set(p, frames) -> (plan, fs); pass 0 samples, every later pass refines each member from its own latent of the pass
-        before; with `seed` the keys are the absolute frame indices (member_keys) and the draw is 0 for pass 0, 1 after.  Results of
-        runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        before; with `seed` the frame keys are key_offset + the absolute frame indices (member_keys) and the draw is 0 for pass 0, 1
+        after.  Results of runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3] with n_frames the
+        frames of all runs, run after run: the whole trajectory when `runs` are all of its runs."""
         if seed is not None and generator is not None:
             raise ValueError("seed draws the noise itself: it excludes generator")
+        if n_frames != sum(n for _, n in runs):
+            raise ValueError(f"the runs hold {sum(n for _, n in runs)} frames, not {n_frames}")
+        first = [sum(n for _, n in runs[:c]) for c in range(len(runs))]         # each run's first output row
         out = None
         res = None
-        for p in range(runs[0][1]):                  # runs[0] is the longest
+        for p in range(max(n for _, n in runs)):
             frames = [start + min(p, n - 1) for start, n in runs]
             plan, fs = frame_set(p, frames)
-            noise = {"generator": generator} if seed is None else {"seed": seed, "keys": member_keys(fs, frames), "draw": int(p > 0)}
+            noise = {"generator": generator} if seed is None else \
+                {"seed": seed, "keys": member_keys(fs, [key_offset + f for f in frames]), "draw": int(p > 0)}
             if p == 0:
                 res = self.sample(plan, fs, **noise)
                 Na = int(fs.num_atoms[0])
@@ -525,7 +547,7 @@ class Backmapper:
                 res = self.refine(plan, fs, res["latent"], steps, **noise)
             live = [c for c, (_, n) in enumerate(runs) if p < n]
             xyz = res["xyz"].view(num_ensemble, len(runs), Na, 3)                 # members are ensemble-major: b = e * chunks + c
-            out[[runs[c][0] + p for c in live]] = xyz[:, live].transpose(0, 1)
+            out[[first[c] + p for c in live]] = xyz[:, live].transpose(0, 1)
         return out.cpu()
 
     def _sample(self, plan: Plan, fs: FrameSet, z, step_noise, use_graph: bool, generator, steps: int = None, seed: int = None,
@@ -597,6 +619,38 @@ def partition_units(lengths, num_ensemble: int, world: int, k_neighbors: int = 6
     units = [(f, e) for f in range(F) for e in range(num_ensemble)]
     parts = distributed.shard_by_cost([cost[f] for f, _ in units], world)
     return [[units[i] for i in p] for p in parts]
+
+
+def partition_trajectory_units(n_frames, lengths, num_ensemble: int, steps: int, T: int, chunks: int, world: int,
+                               k_neighbors: int = 64):
+    """Units of a trajectory job = (trajectory t, run c).  Trajectory t (n_frames[t] frames of lengths[t] residues) is split into
+    runs = trajectory_chunks(n_frames[t], min(chunks, n_frames[t])), which depend on the job alone, never on `world`.  A run of n
+    frames costs L * min(K, L) * num_ensemble * (T + (n - 1) * steps): one full pass, then n - 1 refinements of `steps` steps.  The
+    units are dealt out longest-processing-time first (distributed.shard_by_cost).  Returns (runs, parts): runs[t] the [(first
+    frame, length)] of trajectory t, parts[r] the (t, c) units of rank r in ascending order (empty when there are fewer units than
+    ranks)."""
+    if isinstance(chunks, bool) or not isinstance(chunks, numbers.Integral) or chunks < 1:
+        raise ValueError(f"chunks must be a positive integer, got {chunks!r}")
+    if len(n_frames) != len(lengths):
+        raise ValueError(f"{len(n_frames)} frame counts for {len(lengths)} lengths")
+    runs = [trajectory_chunks(int(n), min(int(chunks), int(n))) for n in n_frames]
+    units = [(t, c) for t in range(len(runs)) for c in range(len(runs[t]))]
+    cost = [float(lengths[t]) * min(int(k_neighbors), int(lengths[t])) * num_ensemble * (T + (runs[t][c][1] - 1) * steps)
+            for t, c in units]
+    return runs, [[units[i] for i in part] for part in distributed.shard_by_cost(cost, world)]
+
+
+def trajectory_key_offsets(n_frames):
+    """Frame-key offsets of a trajectory job: offset_t = the frames of trajectories 0 .. t-1, so frame f of trajectory t has the
+    frame key offset_t + f, its index in the whole job.  Refuses a job whose keys would reach 2^47 (member_keys)."""
+    offsets, total = [], 0
+    for n in n_frames:
+        offsets.append(total)
+        total += int(n)
+    if total > FRAME_KEY_LIMIT:
+        raise ValueError(f"the job holds {total} frames in {len(offsets)} trajectories: its frame keys (frame index in the job) "
+                         f"must lie in [0, 2^47)")
+    return offsets
 
 
 def group_by_length(frames, lengths, max_frames: int = 32, max_pad: float = 0.12):
@@ -698,4 +752,87 @@ class ShardedBackmapper:
             for f, e in parts[r]:
                 out[(f, e)] = buf[o:o + n_atoms[f]]
                 o += n_atoms[f]
+        return out
+
+    def backmap_coords_local(self, trajectories, units, runs, offsets, num_ensemble: int, steps: int, generator=None, seed=None):
+        """Back-map this rank's (trajectory, run) units of a trajectory job: {(t, c): host float32 [n_run, num_ensemble, Na_t, 3]}.
+        The local runs of one trajectory share one plan, as `chunks` runs do in Backmapper.backmap_coords, and only their frames are
+        uploaded.  With `seed` frame f of trajectory t draws with frame key offsets[t] + f, its index in the whole job."""
+        by_traj = {}
+        for t, c in units:
+            by_traj.setdefault(t, []).append(c)
+        res = {}
+        for t, cs in by_traj.items():
+            ca_full, restype, info = trajectories[t]
+            xyz = self.bm._coords_passes(ca_full, restype, info, num_ensemble, steps, [runs[t][c] for c in cs], generator, seed,
+                                         offsets[t])
+            row = 0
+            for c in cs:
+                n = runs[t][c][1]
+                res[(t, c)] = xyz[row:row + n]
+                row += n
+        return res
+
+    def backmap_coords(self, trajectories, num_ensemble: int = 1, steps: int = None, chunks: int = 1, generator=None, seed=None,
+                       _compute=None):
+        """Backmapper.backmap_coords for a job of trajectories over the ranks.  trajectories: a list of (ca_full [n_t, L_t+2, 3],
+        restype [L_t+2], info_t), each what backmap_coords takes; num_ensemble, steps (default T // 4) and chunks apply to every
+        trajectory.  Trajectory t is split into min(chunks, n_t) runs, the same on any number of GPUs, and the (t, run) units are
+        dealt out by cost (partition_trajectory_units); a rank backmaps its runs of one trajectory in one plan with warm starts.
+        Returns on rank 0 a list of host float32 [n_t, num_ensemble, Na_t, 3], one per trajectory in input order; the other ranks send
+        their runs to rank 0 one unit at a time and return None.  With no process group (or world 1) a rank returns that list with
+        its own runs filled in and the others NaN: the whole result for world 1.
+        With `seed`, frame f of trajectory t draws keyed noise with frame key (frames of trajectories before t) + f, so a
+        one-trajectory job draws what Backmapper.backmap_coords(seed=) draws.  A trajectory is never padded and its runs do not
+        depend on the world size, so the result does not either: bit for bit in the fp32 tier, within the f16 tier's tolerance (its
+        MMA tiles sum a row's neighbours in a layout that depends on the row's place in the plan).  With `generator` every rank draws
+        from its own generator, and the result depends on the partition."""
+        import torch.distributed as dist
+        trajectories = list(trajectories)
+        if not trajectories:
+            raise ValueError("backmap_coords: the job holds no trajectory")
+        if seed is not None and generator is not None:
+            raise ValueError("seed draws the noise itself: it excludes generator")
+        if isinstance(chunks, bool) or not isinstance(chunks, numbers.Integral) or chunks < 1:
+            raise ValueError(f"chunks must be a positive integer, got {chunks!r}")
+        for t, traj in enumerate(trajectories):
+            try:
+                if not isinstance(traj, (tuple, list)) or len(traj) != 3:
+                    raise ValueError("it must be a tuple (ca_full, restype, info)")
+                check_coords_args(traj[0], traj[1])
+                steps_t, _ = trajectory_args(self.bm.T, traj[0].shape[0], num_ensemble, steps, min(chunks, traj[0].shape[0]))
+            except ValueError as e:
+                raise ValueError(f"backmap_coords: trajectory {t}: {e}") from None
+        steps = steps_t
+        n_frames = [int(ca.shape[0]) for ca, _, _ in trajectories]
+        offsets = trajectory_key_offsets(n_frames)
+        runs, parts = partition_trajectory_units(n_frames, [int(ca.shape[1]) - 2 for ca, _, _ in trajectories], num_ensemble, steps,
+                                                 self.bm.T, chunks, self.world, self.bm.k_neighbors)
+        noise = {} if seed is None else {"seed": seed}
+        compute = _compute or self.backmap_coords_local
+        mine = compute(trajectories, parts[self.rank], runs, offsets, num_ensemble, steps, generator, **noise) if parts[self.rank] else {}
+        gather = self.world > 1 and dist.is_available() and dist.is_initialized()
+        nccl = gather and dist.get_backend() == "nccl"
+        if gather and self.rank != 0:
+            for u in parts[self.rank]:                               # partition order, as rank 0 receives them
+                dist.send(mine[u].cuda() if nccl else mine[u].contiguous(), dst=0)
+            return None
+        out = [torch.full((n, num_ensemble, int(info[0].numel()), 3), math.nan) for n, (_, _, info) in zip(n_frames, trajectories)]
+
+        def block(t, c):                                             # the rows of run c in trajectory t's output
+            start, n = runs[t][c]
+            return out[t][start:start + n]
+
+        for u in parts[self.rank]:
+            block(*u).copy_(mine[u])
+        if gather:
+            for r in range(1, self.world):
+                for u in parts[r]:
+                    dst = block(*u)
+                    if nccl:
+                        buf = torch.empty(dst.shape, device="cuda")
+                        dist.recv(buf, src=r)
+                        dst.copy_(buf)
+                    else:
+                        dist.recv(dst, src=r)
         return out
