@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CB2_LIB") or os.path.join(_HERE, "libcodlad_b200.so")      # CB2_LIB: experiment builds
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 PRECISION = {"fp32": 0, "f32": 0, "f16": 1, "fp16": 1}
 
@@ -46,6 +46,7 @@ SIGNATURES = {
     "cb2_plan_set_coords": (_I, [_P, _P, _P, _P]),
     "cb2_plan_decode": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "cb2_plan_residue_clashes": (_I, [_P, _P, C.c_float, _I, _P, _P, _P]),
+    "cb2_plan_relax": (_I, [_P, _P, _P, C.c_float, _I, _P, _P, _P]),
     "cb2_plan_buffer": (_I, [_P, C.c_char_p, _P, _LL, _P]),
     "cb2_plan_run_edge_kernel": (_I, [_P, _I, _I, _P]),
     "cb2_plan_run_stage": (_I, [_P, _P, _I, _I, _P, _P]),

@@ -111,7 +111,8 @@ struct cb2_plan {
     float *edge_w = nullptr, *S40 = nullptr, *phi = nullptr, *ic = nullptr, *zq = nullptr;
     int* vq_idx = nullptr;
     float *xa = nullptr, *xb = nullptr;     // ping-pong latents of the sampling loop
-    float4* clash_bounds = nullptr;         // [NB*L] residue centre + radius of cb2_plan_residue_clashes
+    float4* clash_bounds = nullptr;         // [NB*L] residue centre + radius of cb2_plan_residue_clashes (and cb2_plan_relax)
+    RelaxBufs relax{};                      // cb2_plan_relax; sized by the plan's geometry, so allocated once, on first use
     int keep_debug = 0;
     bool frames_ready = false, topo_ready = false;
 };
@@ -834,6 +835,37 @@ int cb2_plan_residue_clashes(cb2_plan* h, const float* xyz, float threshold, int
     return 0;
 }
 
+int cb2_plan_relax(cb2_plan* h, const float* xyz_in, float* xyz_out, float threshold, int iterations, float* max_shift,
+                   float* max_restraint_dev, void* stream) {
+    if (!h || !xyz_in || !xyz_out) { set_error("relax: null argument"); return 1; }
+    if (!h->topo_ready) { set_error("relax: cb2_plan_set_topology has not been called"); return 1; }
+    Plan& p = h->p;
+    if (!(threshold > 0.0f && threshold <= 2.0f)) { set_error("relax: threshold must lie in (0, 2] A"); return 1; }
+    if (iterations < 0 || iterations > 100000) { set_error("relax: iterations=%d outside [0, 100000]", iterations); return 1; }
+    const size_t S = (size_t)p.NB * p.L * 14;
+    if (S * 16 >= (size_t)1 << 31) { set_error("relax: NB*L=%lld is too large for the restraint lists", (long long)p.NB * p.L); return 1; }
+    RelaxBufs& rb = h->relax;
+    if (!rb.x0) {
+        RelaxBufs nb{};
+        int e = 0;
+        e |= dev_alloc(p.allocs, &nb.x0, S * 3);
+        e |= dev_alloc(p.allocs, &nb.xa, S * 3);
+        e |= dev_alloc(p.allocs, &nb.xb, S * 3);
+        e |= dev_alloc(p.allocs, &nb.partner, S * 16);
+        e |= dev_alloc(p.allocs, &nb.d0, S * 16);
+        e |= dev_alloc(p.allocs, &nb.cand, (size_t)p.NB * p.L * ((p.L + 31) / 32));
+        e |= dev_alloc(p.allocs, &nb.grid_slot, (size_t)p.F * p.L * 14);
+        e |= dev_alloc(p.allocs, &nb.grid_off, p.NB);
+        e |= dev_alloc(p.allocs, &nb.nrep, S);
+        if (!h->clash_bounds) e |= dev_alloc(p.allocs, &h->clash_bounds, (size_t)p.NB * p.L);
+        if (e) return e;    // the plan keeps none of them (those that were allocated are freed with it)
+        nb.bounds = h->clash_bounds;
+        rb = nb;
+    }
+    return launch_relax(xyz_in, xyz_out, h->slot_atom, h->out_off, p.lengths, p.frame_of, p.F, p.NB, p.L, threshold, iterations,
+                        max_shift, max_restraint_dev, rb, (cudaStream_t)stream, &p.launches);
+}
+
 int cb2_plan_buffer(cb2_plan* h, const char* name, void* dst, long long dst_bytes, void* stream) {
     if (!h || !name || !dst) { set_error("plan_buffer: null argument"); return 1; }
     void* src = nullptr;
@@ -855,6 +887,9 @@ int cb2_plan_buffer(cb2_plan* h, const char* name, void* dst, long long dst_byte
         if (!p.tc_trace) { unsigned long long* t = nullptr; if (dev_alloc(p.allocs, &t, 6144)) return 1; cudaMemsetAsync(t, 0, 49152, (cudaStream_t)stream); p.tc_trace = t; }
         *ptr = p.tc_trace; *bytes = 49152;
     }
+    else if (n == "relax_partner") { *ptr = h->relax.partner; *bytes = N * 14 * 16 * 4; }
+    else if (n == "relax_d0") { *ptr = h->relax.d0; *bytes = N * 14 * 16 * 4; }
+    else if (n == "relax_nrep") { *ptr = h->relax.nrep; *bytes = N * 14 * 4; }
     else if (n == "mod") { *ptr = p.mod; *bytes = (size_t)p.mod_capacity * CB2_MOD_TOTAL * 4; }
     else { set_error("plan_buffer: unknown buffer '%s'", name); return 1; }
     if (!src || dst_bytes > size) { set_error("plan_buffer: '%s' holds %lld bytes, %lld requested", name, size, dst_bytes); return 1; }

@@ -136,13 +136,21 @@ __global__ void __launch_bounds__(128) clash_keep_kernel(const int* __restrict__
 
 }  // namespace
 
+int launch_residue_bounds(const float* xyz, const int* slot_atom, const long long* out_off, const int* lengths, const int* frame_of,
+                          int NB, int L, float4* bounds, cudaStream_t s) {
+    const int N = NB * L;
+    if (N <= 0) return 0;
+    residue_bounds_kernel<<<(N + 127) / 128, 128, 0, s>>>(xyz, slot_atom, out_off, lengths, frame_of, NB, L, bounds);
+    CB2_LAUNCH_CHECK();
+    return 0;
+}
+
 int launch_residue_clashes(const float* xyz, const int* slot_atom, const long long* out_off, const int* lengths, const int* frame_of,
                            const int* nbr_idx, int NB, int L, int K, float threshold, int grow, float4* bounds, int* counts,
                            unsigned char* keep, cudaStream_t s) {
     const int N = NB * L;
     if (N <= 0) return 0;
-    residue_bounds_kernel<<<(N + 127) / 128, 128, 0, s>>>(xyz, slot_atom, out_off, lengths, frame_of, NB, L, bounds);
-    CB2_LAUNCH_CHECK();
+    if (int e = launch_residue_bounds(xyz, slot_atom, out_off, lengths, frame_of, NB, L, bounds, s)) return e;
     residue_clash_kernel<<<(N + CL_WARPS - 1) / CL_WARPS, CL_WARPS * 32, 0, s>>>(xyz, slot_atom, out_off, lengths, frame_of, bounds, NB, L,
                                                                                threshold, counts);
     CB2_LAUNCH_CHECK();

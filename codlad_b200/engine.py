@@ -32,6 +32,20 @@ def check_clash_args(threshold, grow, K: int):
         raise ValueError(f"grow must be an integer in [0, {K}), got {grow!r}")
 
 
+RELAX_MAX_THRESHOLD = 2.0      # A: above it the repulsion distance reaches the restrained 1-3 geometry of the peptide
+RELAX_MAX_ITERATIONS = 100_000
+
+
+def check_relax_args(threshold, iterations):
+    """Arguments of the clash relaxation: threshold (Angstrom) in (0, 2.0] and an integer number of iterations in [0, 10^5].
+    Above 2 A the repulsion distance, threshold + 0.2 A, would reach the restrained 1-3 distances of the peptide (about
+    2.25-2.45 A), which the relaxation must leave as decoded.  Raises ValueError; touches no device."""
+    if isinstance(threshold, bool) or not isinstance(threshold, numbers.Real) or not 0 < threshold <= RELAX_MAX_THRESHOLD:
+        raise ValueError(f"threshold must lie in (0, {RELAX_MAX_THRESHOLD}] Angstrom, got {threshold!r}")
+    if isinstance(iterations, bool) or not isinstance(iterations, numbers.Integral) or not 0 <= iterations <= RELAX_MAX_ITERATIONS:
+        raise ValueError(f"iterations must be an integer in [0, {RELAX_MAX_ITERATIONS}], got {iterations!r}")
+
+
 def check_start_steps(steps):
     """Argument of Plan.set_start: a non-negative integer (0 = the whole schedule).  Raises ValueError; touches no device."""
     if isinstance(steps, bool) or not isinstance(steps, numbers.Integral) or steps < 0:
@@ -258,6 +272,23 @@ class Plan:
                                                  N.dptr(keep), N.stream_ptr()), "residue_clashes")
         return counts, keep.view(torch.bool)
 
+    def relax(self, xyz, threshold: float = 1.2, iterations: int = 50):
+        """Restrained clash relaxation of a decoded sample (cb2_plan_relax; needs set_topology).  xyz [total atoms, 3] CUDA fp32 as
+        decode() writes it; it is not modified.  Returns (xyz_out, max_shift [NB], max_restraint_dev [NB]): the relaxed copy (C-alphas,
+        padded and absent rows as given), and per member the largest distance an atom moved and the largest deviation of a restrained
+        distance from its input value.  See Backmapper.relax for the objective."""
+        if not torch.is_tensor(xyz) or xyz.dtype != torch.float32 or xyz.dim() != 2 or xyz.shape[1] != 3:
+            raise ValueError("xyz must be a float32 tensor of shape [total atoms, 3]")
+        if xyz.device != self.device:
+            raise ValueError(f"xyz must be on {self.device}")
+        check_relax_args(threshold, iterations)
+        out = xyz.contiguous().clone()
+        shift = torch.empty(self.NB, device=self.device, dtype=torch.float32)
+        dev = torch.empty(self.NB, device=self.device, dtype=torch.float32)
+        N.check(N.lib().cb2_plan_relax(self.handle, N.dptr(out), N.dptr(out), C.c_float(threshold), int(iterations), N.dptr(shift),
+                                       N.dptr(dev), N.stream_ptr()), "relax")
+        return out, shift, dev
+
     # -- debug -------------------------------------------------------------------------------------
     def buffer(self, name: str) -> torch.Tensor:
         """Copy of a plan-owned buffer (parity tests)."""
@@ -268,6 +299,8 @@ class Plan:
             "hE": (edge_dtype, (self.NB, self.L, self.K, 128)), "hV": (torch.float32, (self.NB, self.L, 128)),
             "S": (torch.float32, (self.NB, self.L, 128)), "out6": (torch.float32, (self.NB, self.L, 6)),
             "tc_trace": (torch.int64, (6144,)),
+            "relax_partner": (torch.int32, (self.NB, self.L, 14, 16)), "relax_d0": (torch.float32, (self.NB, self.L, 14, 16)),
+            "relax_nrep": (torch.int32, (self.NB, self.L, 14)),
         }[name]
         out = torch.empty(spec[1], device=self.device, dtype=spec[0])
         N.check(N.lib().cb2_plan_buffer(self.handle, name.encode(), N.dptr(out), out.numel() * out.element_size(), N.stream_ptr()),

@@ -20,7 +20,8 @@ import torch
 
 from . import batching, distributed, metrics, topology, weights
 from .diffusion import create_diffusion
-from .engine import DenoiserEngine, Plan, VaeEngine, check_clash_args, check_keyed_normal_args, check_start_steps, keyed_normal
+from .engine import (DenoiserEngine, Plan, VaeEngine, check_clash_args, check_keyed_normal_args, check_relax_args, check_start_steps,
+                     keyed_normal)
 
 VAE_DATA = {"N6": "PED", "K3": "PDB", "K4": "Atlas"}
 
@@ -61,6 +62,21 @@ def trajectory_args(T: int, n_frames: int, num_ensemble, steps, chunks):
     if not 1 <= steps <= T:
         raise ValueError(f"steps must be in [1, {T}], got {steps}")
     return steps, trajectory_chunks(n_frames, chunks)
+
+
+RELAX_ITERATIONS = 50       # default iterations of Backmapper.relax: planted 0.4 A overlaps are pushed past the threshold in them
+
+
+def relax_option(relax):
+    """The `relax=` option of the trajectory methods: None (no relaxation) or a dict with the keys `iterations` and `threshold` of
+    Backmapper.relax, both optional.  Returns the full keyword dict (or None); raises ValueError; touches no device."""
+    if relax is None:
+        return None
+    if not isinstance(relax, dict) or not set(relax) <= {"iterations", "threshold"}:
+        raise ValueError(f"relax must be None or a dict with the keys 'iterations' and 'threshold', got {relax!r}")
+    opts = {"iterations": RELAX_ITERATIONS, "threshold": 1.2, **relax}
+    check_relax_args(opts["threshold"], opts["iterations"])
+    return opts
 
 
 def check_coords_args(ca_full, restype):
@@ -432,6 +448,32 @@ class Backmapper:
         res["clash_pairs"] = torch.stack(rows, 0)
         return res
 
+    def relax(self, plan: Plan, fs: FrameSet, out: dict, iterations: int = RELAX_ITERATIONS, threshold: float = 1.2):
+        """Restrained clash relaxation of a backmapped sample `out` (the dict of sample() / resample() / refine() / repair()), on the
+        device (cb2_plan_relax): pushes atoms of different residues that are closer than `threshold` apart while holding the decoded
+        bonded geometry and the C-alpha trace.  Per member: the C-alphas never move; every intra-residue pair within 3 A at the input
+        (bonds, angles, ring closures) and the peptide pairs C(i)-N(i+1), CA(i)-N(i+1), O(i)-N(i+1), C(i)-CA(i+1) are restrained to
+        their input distance d0; every other pair of two residues closer than c = threshold + 0.2 A is repelled.  It minimises
+        E = sum 1.0 (d - d0)^2 + sum 10.0 (c - d)^2 with `iterations` capped steepest-descent steps (0.05 A^2 per unit force, at most
+        0.1 A per atom and step), a fixed amount of work with no early exit.  Deterministic, and a member's result does not depend on
+        its batch; a member with no pair closer than c comes back bit for bit.  Intra-residue overlaps are left as decoded.
+        threshold must lie in (0, 2.0] A: above that the repulsion distance would reach the restrained 1-3 distances of the peptide
+        (about 2.25-2.45 A).  0 <= iterations <= 10^5.
+        Returns dict(out) with `xyz` replaced by the relaxed coordinates; `latent`, `idx` and `zq` are unchanged, so refine() and
+        repair() can continue from them, and `ic_recon` still describes the unrelaxed decode.  Adds `clash_pairs` (int64 [2, NB]: pairs
+        under `threshold` per member before and after, residue_clashes), `clashes` (int32 [NB, L], the counts after), `max_shift`
+        (float32 [NB], the largest distance an atom moved) and `max_restraint_dev` (float32 [NB], the largest |d - d0|)."""
+        if not isinstance(out, dict) or not all(k in out for k in ("latent", "idx", "zq", "ic_recon", "xyz")):
+            raise ValueError("out must be the dict returned by sample(), resample(), refine() or repair()")
+        check_relax_args(threshold, iterations)
+        before, _ = self.residue_clashes(plan, fs, out["xyz"], threshold)
+        xyz, shift, dev = plan.relax(out["xyz"], threshold, iterations)
+        after, _ = self.residue_clashes(plan, fs, xyz, threshold)
+        res = dict(out)
+        res.update(xyz=xyz, clashes=after, clash_pairs=torch.stack((clash_pair_totals(before), clash_pair_totals(after)), 0),
+                   max_shift=shift, max_restraint_dev=dev)
+        return res
+
     def residue_motion(self, fs: FrameSet, xyz_a: torch.Tensor, xyz_b: torch.Tensor) -> torch.Tensor:
         """Per-residue RMSD between two decoded structures of the same frame set (xyz [fs.total_atoms, 3] CUDA float32, as
         sample() returns them), each residue's atoms superposed on their own (cb2_superposed_rmsd over the residue_atom_ranges).
@@ -451,7 +493,7 @@ class Backmapper:
         return out.view(fs.NB, fs.L)
 
     def backmap_trajectory(self, batches, info, num_ensemble: int = 1, steps: int = None, chunks: int = 1,
-                           generator: torch.Generator = None, seed: int = None) -> torch.Tensor:
+                           generator: torch.Generator = None, seed: int = None, relax: dict = None) -> torch.Tensor:
         """Backmap consecutive frames of one protein with warm starts.  batches: one reference-schema batch dict per frame (one
         frame each, all of the same length), info: the shared topology tuple.  The frames are split into `chunks` contiguous runs
         (trajectory_chunks) that go through one plan together, each run with `num_ensemble` members.  The first frame of every run
@@ -460,9 +502,12 @@ class Backmapper:
         put more frames into one pass and break coherence chunks - 1 times.  A run that has ended repeats its last frame, and that
         result is dropped.  With `seed` (instead of `generator`) member e of frame f draws keyed noise (engine.keyed_normal) with key
         f * 2^16 + e, draw 0 when it is sampled and draw 1 when it is refined, so its noise does not depend on `chunks`; its result
-        still does, through the warm start it refines.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
+        still does, through the warm start it refines.  relax = dict(iterations=..., threshold=...) (either may be left out) relaxes
+        every frame's coordinates with relax() before they are stored; the warm starts keep the unrelaxed latents, so relaxing changes
+        no frame's sampling.  Returns host float32 [n_frames, num_ensemble, Na, 3]."""
         batches = list(batches)
         steps, runs = trajectory_args(self.T, len(batches), num_ensemble, steps, chunks)
+        relax = relax_option(relax)
         if any(b["num_CGs"].numel() != 1 for b in batches) or len({int(b["num_CGs"].sum()) for b in batches}) != 1:
             raise ValueError("backmap_trajectory: every batch must hold one frame, all of the same length")
 
@@ -470,7 +515,7 @@ class Backmapper:
             fs = frames_from_batch(batching.merge_batches([batches[f] for f in frames]), info, num_ensemble)
             return self.upload(fs), fs
 
-        return self._trajectory_passes(len(batches), num_ensemble, steps, runs, frame_set, generator, seed)
+        return self._trajectory_passes(len(batches), num_ensemble, steps, runs, frame_set, generator, seed, relax=relax)
 
     def update_coords(self, plan: Plan, fs: FrameSet, ca_full: torch.Tensor):
         """Move a plan uploaded from `fs` (upload()) to new coordinates of the same frames, with no host work: ca_full [fs.F, fs.L+2, 3]
@@ -488,23 +533,25 @@ class Backmapper:
         plan.set_coords(self.vae, ca_full)
 
     def backmap_coords(self, ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int = 1, steps: int = None,
-                       chunks: int = 1, generator: torch.Generator = None, seed: int = None) -> torch.Tensor:
+                       chunks: int = 1, generator: torch.Generator = None, seed: int = None, relax: dict = None) -> torch.Tensor:
         """backmap_trajectory for a trajectory given as a coordinate array: ca_full float32 [n_frames, L+2, 3], host or CUDA, the
         coordinate columns of OG_CG_nxyz of every frame (termini included); restype [L+2] integer, its residue ids
         (OG_CG_nxyz[:, 0]); info the topology tuple.  The topology tables are built on the host once; ca_full is uploaded once,
         whole, and every pass, the first included, moves the plan to its frames with update_coords, so the radius graph, X and
         k-NN graph of every frame are built on the device and no batch dict or host graph is needed.  Same passes, arguments (`seed`
-        included) and result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to backmap_trajectory on
-        batches of the same frames wherever the caller's graph follows the same 21 A rule (it can differ only for a pair at the
-        cutoff)."""
+        included, and `relax`) and result as backmap_trajectory: host float32 [n_frames, num_ensemble, Na, 3], equal to
+        backmap_trajectory on batches of the same frames wherever the caller's graph follows the same 21 A rule (it can differ only
+        for a pair at the cutoff)."""
         check_coords_args(ca_full, restype)
         steps, runs = trajectory_args(self.T, ca_full.shape[0], num_ensemble, steps, chunks)
-        return self._coords_passes(ca_full, restype, info, num_ensemble, steps, runs, generator, seed)
+        relax = relax_option(relax)
+        return self._coords_passes(ca_full, restype, info, num_ensemble, steps, runs, generator, seed, relax=relax)
 
     def _coords_passes(self, ca_full: torch.Tensor, restype: torch.Tensor, info, num_ensemble: int, steps: int, runs, generator,
-                       seed=None, key_offset: int = 0) -> torch.Tensor:
+                       seed=None, key_offset: int = 0, relax: dict = None) -> torch.Tensor:
         """The body of backmap_coords for any subset of a trajectory's runs (start, n) (trajectory_chunks order): one plan holds them
-        all, only their frames are uploaded, and frame f draws keyed noise with frame key key_offset + f.  Returns host float32
+        all, only their frames are uploaded, and frame f draws keyed noise with frame key key_offset + f; relax as relax_option
+        returns it.  Returns host float32
         [sum n, num_ensemble, Na, 3], the frames of the runs in order."""
         fs = frames_from_coords(ca_full[[start for start, _ in runs]], restype, info, num_ensemble)
         dev = torch.device("cuda", torch.cuda.current_device())
@@ -518,14 +565,15 @@ class Backmapper:
             self.update_coords(plan, fs, ca_dev[first + torch.clamp(last, max=p)])
             return plan, fs
 
-        return self._trajectory_passes(rows.numel(), num_ensemble, steps, runs, frame_set, generator, seed, key_offset)
+        return self._trajectory_passes(rows.numel(), num_ensemble, steps, runs, frame_set, generator, seed, key_offset, relax)
 
     def _trajectory_passes(self, n_frames: int, num_ensemble: int, steps: int, runs, frame_set, generator, seed=None,
-                           key_offset: int = 0) -> torch.Tensor:
+                           key_offset: int = 0, relax: dict = None) -> torch.Tensor:
         """The pass loop of the trajectory methods.  Pass p puts frame start + min(p, n - 1) of every run (start, n) on one plan through
         frame_set(p, frames) -> (plan, fs); pass 0 samples, every later pass refines each member from its own latent of the pass
         before; with `seed` the frame keys are key_offset + the absolute frame indices (member_keys) and the draw is 0 for pass 0, 1
-        after.  Results of runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3] with n_frames the
+        after.  With `relax` (relax_option's dict) each pass's coordinates are relaxed (Plan.relax) before they are stored; the next
+        pass refines the unrelaxed latent.  Results of runs that have ended are dropped.  Returns host float32 [n_frames, num_ensemble, Na, 3] with n_frames the
         frames of all runs, run after run: the whole trajectory when `runs` are all of its runs."""
         if seed is not None and generator is not None:
             raise ValueError("seed draws the noise itself: it excludes generator")
@@ -546,7 +594,8 @@ class Backmapper:
             else:
                 res = self.refine(plan, fs, res["latent"], steps, **noise)
             live = [c for c, (_, n) in enumerate(runs) if p < n]
-            xyz = res["xyz"].view(num_ensemble, len(runs), Na, 3)                 # members are ensemble-major: b = e * chunks + c
+            xyz = res["xyz"] if relax is None else plan.relax(res["xyz"], relax["threshold"], relax["iterations"])[0]
+            xyz = xyz.view(num_ensemble, len(runs), Na, 3)                        # members are ensemble-major: b = e * chunks + c
             out[[first[c] + p for c in live]] = xyz[:, live].transpose(0, 1)
         return out.cpu()
 
@@ -754,10 +803,12 @@ class ShardedBackmapper:
                 o += n_atoms[f]
         return out
 
-    def backmap_coords_local(self, trajectories, units, runs, offsets, num_ensemble: int, steps: int, generator=None, seed=None):
+    def backmap_coords_local(self, trajectories, units, runs, offsets, num_ensemble: int, steps: int, generator=None, seed=None,
+                             relax=None):
         """Back-map this rank's (trajectory, run) units of a trajectory job: {(t, c): host float32 [n_run, num_ensemble, Na_t, 3]}.
         The local runs of one trajectory share one plan, as `chunks` runs do in Backmapper.backmap_coords, and only their frames are
-        uploaded.  With `seed` frame f of trajectory t draws with frame key offsets[t] + f, its index in the whole job."""
+        uploaded.  With `seed` frame f of trajectory t draws with frame key offsets[t] + f, its index in the whole job.  relax as
+        relax_option returns it."""
         by_traj = {}
         for t, c in units:
             by_traj.setdefault(t, []).append(c)
@@ -765,7 +816,7 @@ class ShardedBackmapper:
         for t, cs in by_traj.items():
             ca_full, restype, info = trajectories[t]
             xyz = self.bm._coords_passes(ca_full, restype, info, num_ensemble, steps, [runs[t][c] for c in cs], generator, seed,
-                                         offsets[t])
+                                         offsets[t], relax)
             row = 0
             for c in cs:
                 n = runs[t][c][1]
@@ -774,7 +825,7 @@ class ShardedBackmapper:
         return res
 
     def backmap_coords(self, trajectories, num_ensemble: int = 1, steps: int = None, chunks: int = 1, generator=None, seed=None,
-                       _compute=None):
+                       _compute=None, relax=None):
         """Backmapper.backmap_coords for a job of trajectories over the ranks.  trajectories: a list of (ca_full [n_t, L_t+2, 3],
         restype [L_t+2], info_t), each what backmap_coords takes; num_ensemble, steps (default T // 4) and chunks apply to every
         trajectory.  Trajectory t is split into min(chunks, n_t) runs, the same on any number of GPUs, and the (t, run) units are
@@ -786,9 +837,11 @@ class ShardedBackmapper:
         one-trajectory job draws what Backmapper.backmap_coords(seed=) draws.  A trajectory is never padded and its runs do not
         depend on the world size, so the result does not either: bit for bit in the fp32 tier, within the f16 tier's tolerance (its
         MMA tiles sum a row's neighbours in a layout that depends on the row's place in the plan).  With `generator` every rank draws
-        from its own generator, and the result depends on the partition."""
+        from its own generator, and the result depends on the partition.  relax as in Backmapper.backmap_coords: relaxation is per
+        member and deterministic, so it keeps the result independent of the world size."""
         import torch.distributed as dist
         trajectories = list(trajectories)
+        relax = relax_option(relax)
         if not trajectories:
             raise ValueError("backmap_coords: the job holds no trajectory")
         if seed is not None and generator is not None:
@@ -809,6 +862,8 @@ class ShardedBackmapper:
         runs, parts = partition_trajectory_units(n_frames, [int(ca.shape[1]) - 2 for ca, _, _ in trajectories], num_ensemble, steps,
                                                  self.bm.T, chunks, self.world, self.bm.k_neighbors)
         noise = {} if seed is None else {"seed": seed}
+        if relax is not None:
+            noise["relax"] = relax
         compute = _compute or self.backmap_coords_local
         mine = compute(trajectories, parts[self.rank], runs, offsets, num_ensemble, steps, generator, **noise) if parts[self.rank] else {}
         gather = self.world > 1 and dist.is_available() and dist.is_initialized()

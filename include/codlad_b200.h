@@ -26,7 +26,7 @@ extern "C" {
 #define CB2_API
 #endif
 
-#define CB2_ABI_VERSION 7
+#define CB2_ABI_VERSION 8
 #define CB2_PRECISION_F32 0   /* fp32 SIMT tier: tracks the fp32 reference to ~1e-6 */
 #define CB2_PRECISION_F16 1   /* tcgen05 tier: fp16 operands / edge state, fp32 accumulation in TMEM */
 #define CB2_MOD_WIDTH 6016    /* adaLN table row: 3*1152 (enc) + 3*768 (dec) + 256 (final) */
@@ -164,7 +164,25 @@ CB2_API int cb2_plan_decode(cb2_plan* p, const cb2_vae* v, const float* latent, 
 CB2_API int cb2_plan_residue_clashes(cb2_plan* p, const float* xyz, float threshold, int grow, int* counts, unsigned char* keep,
                              void* stream);
 
-/* Debug / parity access to plan-owned buffers: "nbr_idx" "nbr_dist" "E" "hE0" "hE" "hV" "S" "out6" "mod".
+/* Not in the reference (it has no refinement after ic_to_xyz): restrained clash relaxation of a decoded sample, the short
+ * minimisation backmapping pipelines finish with.  xyz_in / xyz_out [sum Na,3] as cb2_plan_decode writes them (slot_atom / out_offset
+ * of cb2_plan_set_topology, which must have been called); xyz_in == xyz_out is allowed.  Per member, over the present atoms of real
+ * residues: the C-alphas (slot 3) never move; restraints, built once per call, hold every intra-residue pair within 3 A at the input
+ * and the peptide pairs C(i)-N(i+1), CA(i)-N(i+1), O(i)-N(i+1), C(i)-CA(i+1) at their input distance d0; repulsion acts on every
+ * pair of two residues that is not such a peptide pair and has d < c = threshold + 0.2 A, d as cb2_plan_residue_clashes forms it.
+ * E = sum 1.0 (d - d0)^2 + sum 10.0 (c - d)^2 (A^-2); `iterations` Jacobi steps x += 0.05 F, each atom's step capped at 0.1 A;
+ * pairs with a non-finite atom are skipped and non-finite atoms stay.  No early exit and no host synchronisation; deterministic,
+ * and a member's result does not depend on the other members or the padded length.  A member with no pair closer than c is
+ * returned bit for bit.  Only the rows of present atoms of real residues are written.  max_shift / max_restraint_dev [NB] fp32 or
+ * NULL: per member, the largest distance an atom moved and the largest |d - d0| over its restraints.  Refuses a threshold outside
+ * (0, 2] A (above 2 A the repulsion distance reaches the restrained 1-3 geometry of the peptide, about 2.25-2.45 A) and iterations
+ * outside [0, 100000]; iterations = 0 copies the input.  Launches 3 + iterations + 2 ceil(iterations / 5) kernels. */
+CB2_API int cb2_plan_relax(cb2_plan* p, const float* xyz_in, float* xyz_out, float threshold, int iterations, float* max_shift,
+                   float* max_restraint_dev, void* stream);
+
+/* Debug / parity access to plan-owned buffers: "nbr_idx" "nbr_dist" "E" "hE0" "hE" "hV" "S" "out6" "mod", and after
+ * cb2_plan_relax "relax_partner" / "relax_d0" ([NB,L,14,16] restraint lists: member-local slot index j*14+u, -1 past the end, and
+ * d0) and "relax_nrep" ([NB,L,14] int32: repulsive pairs each moving atom evaluated in the last iteration).
  * Copies the first dst_bytes of the buffer into the caller's device memory (error if it is smaller). */
 CB2_API int cb2_plan_buffer(cb2_plan* p, const char* name, void* dst, long long dst_bytes, void* stream);
 
